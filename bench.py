@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the AlphaQuoridorGNN hot path on B200 (contract: see the task statement / DESIGN.md section 7).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one batched leaf evaluation (BaseNetwork.predict semantics for B states: legal-move mask + graph build +
 GNN forward + restriction to legal actions) over one batch of B = 16,384 synthetic legal positions per GPU --
@@ -39,6 +39,24 @@ BYTES_PER_BOARD_HEADS = 128 * 4 + 209 * 4 + 4 + 32
 # named here (a profiler cannot run inside the timed bench; the capture is of the same command line)
 NCU_TRAFFIC = {("gcn_forward_kernel", 1, 16384): (632064, "profiles/r1_v3_kernels_ncu.csv: gcn_forward_tc2_kernel, dram read 0.632 MB + write 0 "
                                                   "(the 8 MB of pooled output is still in L2 when the kernel ends)")}
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes the result arrays of one leaf-evaluation step as <out_dir>/<name>.npy: float32, and float64 for the 32-bit legal-mask
+    words, so every value is stored exactly.  When the boards do not fit in DUMP_MAX_BYTES, a fixed seeded sample of them is written;
+    board_index.npy names the boards written, so two builds run with the same arguments compare output for output."""
+    host = {k: v.cpu().numpy() for k, v in outputs.items()}
+    host["mask"] = host["mask"].view(np.uint32).astype(np.float64)
+    host = {k: v if v.dtype == np.float64 else v.astype(np.float32) for k, v in host.items()}
+    B = len(host["priors"])
+    per_board = sum(v[:1].nbytes for v in host.values()) + 8                  # + the board's index
+    n = min(B, (DUMP_MAX_BYTES - 4096) // per_board)                          # 4 KB for the .npy headers
+    idx = np.arange(B) if n == B else np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "board_index.npy"), idx.astype(np.float64))
+    for k, v in host.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v[idx])
 
 
 def peaks():
@@ -437,6 +455,8 @@ def run_ours(args, rank, world, local_rank):
     sampler.start()
     ms_step, gpu_launches = timed(step, K, Wm)
     value_main = world * B / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:   # the buffers still hold the last timed step; the kernel timings below overwrite them
+        dump_outputs(args.dump_outputs, {"priors": priors, "value": value, "mask": mask, "pawn": pawn})
 
     # ---- per-kernel durations (same inputs, same stream) for the roofline ------------------------
     def k_legal(i):
@@ -733,7 +753,12 @@ def main():
     ap.add_argument("--mcts-sims", type=int, default=200)
     ap.add_argument("--skip-extra", action="store_true")
     ap.add_argument("--skip-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them returned (priors, value, mask, pawn of rank 0's batch) "
+                         "as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference has none")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
