@@ -86,117 +86,38 @@ __global__ void unpack_states_kernel(const AqState *__restrict__ states, int64_t
 }
 
 // ------------------------------------------------------------------------------------------
-// K1 legal_mask: kLanes lanes per state (32 / kLanes states per warp), kLanes in {2, 8, 32} chosen by batch size:
-//   the per-state work is a variable number of flood fills (0 .. ~60), so small batches are bound by the slowest
-//   states of a nearly empty machine and want many lanes per state, while large batches want many states per warp.
-//   every lane: open-direction bitboards, can_place + gate for all 128 candidates (bit-parallel);
-//   sub-lanes 0/1: one witness path for the mover / the opponent on the board WITHOUT a candidate,
-//   as the sets of slots that would cut it (find_path_cuts);
-//   a gated candidate needs a real search only for the player whose witness it cuts: those
-//   (candidate, player) tasks are compacted into a per-state list and dealt round-robin to the
-//   state's lanes; each lane runs its flood fills in registers.
+// K1 legal_mask.  Three forms, all running the per-state steps of legal_steps.cuh: prepare (open-direction boards, can_place + gate of
+// all 128 candidates, the witness paths of mover and opponent, and the (candidate, player) searches still needed as task sets), the
+// searches, and the mask and pawn words.  They differ only in where a state's tasks go:
+//   legal_mask_kernel<kLanes>  (one kernel; aq_legal_mask, and aq_legal_mask_ws up to 4,096 states): to the state's own kLanes lanes
+//                          (32 / kLanes states per warp, kLanes in {2, 8, 32} by batch size), dealt round-robin by rank; each lane
+//                          runs its flood fills in registers.  The per-state work is a variable number of flood fills (0 .. ~60), so
+//                          small batches are bound by the slowest states of a nearly empty machine and want many lanes per state, while
+//                          large batches want many states per warp.
+//   legal_prepare_kernel + legal_search_kernel  (two-phase, below): to a global task list;
+//   the legal warpgroup of the fused leaf-evaluation trunk (gnn_tc2.cu): to a task list in shared memory.
 // ------------------------------------------------------------------------------------------
 constexpr int kLegalWarps = 4;
 
-template <int kLanesPerState>
+template <int kLanes>
 __global__ void __launch_bounds__(kLegalWarps * 32)
-legal_mask_kernel(const AqState *__restrict__ states, int64_t B, uint32_t *__restrict__ mask,
-                  uint8_t *__restrict__ pawn) {
-    constexpr int kStatesPerWarp = 32 / kLanesPerState;
-    __shared__ uint8_t task[kLegalWarps * kStatesPerWarp][256];
+legal_mask_kernel(const AqState *__restrict__ states, int64_t B, uint32_t *__restrict__ mask, uint8_t *__restrict__ pawn) {
     aq_pdl_trigger();  // a kernel launched programmatically behind this one (the GNN trunk of a leaf evaluation) may start as SMs free up
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int sub = lane & (kLanesPerState - 1), grp = lane / kLanesPerState;
-    const unsigned gmask = kLanesPerState == 32 ? 0xffffffffu : ((1u << (kLanesPerState & 31)) - 1u) << (grp * kLanesPerState);
-    const int64_t b = ((int64_t)blockIdx.x * kLegalWarps + warp) * kStatesPerWarp + grp;
-    if (b >= B) return;  // the whole lane group of a state leaves together
-    uint8_t *tl = task[warp * kStatesPerWarp + grp];
-    const AqState s = load_state(states + b);
-    const Open base = open_from_walls(s.hwalls, s.vwalls);
-    const int me = s.ppos, en = 80 - (int)s.epos;  // enemy square in the mover's frame, game_logic.py:136
-
-    u64 legalH = 0, legalV = 0;
-    if (s.pwalls > 0) {  // game_logic.py:113
-        const WallSets ws = wall_sets(s.hwalls, s.vwalls);
-        legalH = ws.freeH;
-        legalV = ws.freeV;
-        if (ws.needH | ws.needV) {
-            // witness paths: mover (start me, obstacle en, goal row 0) on sub-lane 0, opponent in the
-            // un-rotated frame (start en, obstacle me, goal row 8) on sub-lane 1  (game_logic.py:332-348)
-            PathCuts pc;
-            pc.cutH = 0; pc.cutV = 0; pc.exists = 0;
-            if (sub < 2) pc = find_path_cuts(base, sub == 0 ? me : en, sub == 0 ? en : me, sub == 0 ? goal_row0() : goal_row8());
-            __syncwarp(gmask);
-            u64 set[4];  // tasks: [mover H, mover V, opponent H, opponent V]
-#pragma unroll
-            for (int p = 0; p < 2; ++p) {
-                const int ex = __shfl_sync(gmask, pc.exists, p, kLanesPerState);
-                const u64 ch = ((u64)__shfl_sync(gmask, (unsigned)(pc.cutH >> 32), p, kLanesPerState) << 32) |
-                               __shfl_sync(gmask, (unsigned)pc.cutH, p, kLanesPerState);
-                const u64 cv = ((u64)__shfl_sync(gmask, (unsigned)(pc.cutV >> 32), p, kLanesPerState) << 32) |
-                               __shfl_sync(gmask, (unsigned)pc.cutV, p, kLanesPerState);
-                set[2 * p + 0] = ws.needH & (ex ? ch : ~0ull);
-                set[2 * p + 1] = ws.needV & (ex ? cv : ~0ull);
-            }
-            int offs[5];
-            offs[0] = 0;
-#pragma unroll
-            for (int q = 0; q < 4; ++q) offs[q + 1] = offs[q] + __popcll(set[q]);
-            const int total = offs[4];
-            // every lane walks the (few) set bits and writes those whose rank is its own modulo the lane count; a loop over all
-            // 64 slots per set cost 128 iterations per lane at two lanes per state
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                u64 mm = set[q];
-                for (int r = 0; mm; ++r, mm &= mm - 1)
-                    if ((r & (kLanesPerState - 1)) == sub) tl[offs[q] + r] = (uint8_t)((__ffsll((long long)mm) - 1) | (q << 6));
-            }
-            __syncwarp(gmask);
-            u64 failH = 0, failV = 0;
-            for (int j = sub; j < total; j += kLanesPerState) {
-                const int code = tl[j];
-                const int slot = code & 63, orient = ((code >> 6) & 1) + 1, opp = code >> 7;
-                Open o = base;
-                add_wall(o, orient, slot);
-                const bool ok = opp ? reaches(o, en, me, goal_row8()) : reaches(o, me, en, goal_row0());
-                if (!ok) {
-                    if (orient == 1) failH |= 1ull << slot; else failV |= 1ull << slot;
-                }
-            }
-            __syncwarp(gmask);
-            const unsigned a0 = __reduce_or_sync(gmask, (unsigned)failH), a1 = __reduce_or_sync(gmask, (unsigned)(failH >> 32));
-            const unsigned c0 = __reduce_or_sync(gmask, (unsigned)failV), c1 = __reduce_or_sync(gmask, (unsigned)(failV >> 32));
-            legalH |= ws.needH & ~(((u64)a1 << 32) | a0);
-            legalV |= ws.needV & ~(((u64)c1 << 32) | c0);
-        }
-    }
-    if (sub == 0) {
-        uint8_t pm[8] = {0, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0, 0};
-        const int n = pawn_moves(base, me, en, pm + 1);
-        pm[0] = (uint8_t)n;
-        u128 lo = 0;
-        for (int k = 0; k < n; ++k) lo |= (u128)1 << pm[1 + k];
-        lo |= (u128)legalH << 81;                                  // H wall actions 81..144
-        const u128 hi = (u128)(legalH >> 47) | ((u128)legalV << 17);  // V wall actions 145..208
-        uint4 *m = reinterpret_cast<uint4 *>(mask + 8 * b);
-        uint4 w;
-        w.x = (unsigned)lo; w.y = (unsigned)(lo >> 32); w.z = (unsigned)(lo >> 64); w.w = (unsigned)(lo >> 96);
-        m[0] = w;
-        w.x = (unsigned)hi; w.y = (unsigned)(hi >> 32); w.z = (unsigned)(hi >> 64); w.w = (unsigned)(hi >> 96);
-        m[1] = w;
-        uint2 p;
-        p.x = pm[0] | (pm[1] << 8) | (pm[2] << 16) | ((unsigned)pm[3] << 24);
-        p.y = pm[4] | (pm[5] << 8);
-        *reinterpret_cast<uint2 *>(pawn + 8 * b) = p;
-    }
+    const int64_t b0 = ((int64_t)blockIdx.x * kLegalWarps + warp) * (32 / kLanes) + lane / kLanes;
+    const bool valid = b0 < B;
+    const int64_t b = valid ? b0 : B - 1;  // out-of-range lanes shadow the last state and write nothing
+    LegalPrep p;
+    legal_prepare_state<kLanes>(load_state(states + b), lane, p);
+    u64 legalH, legalV;
+    legal_search_in_place<kLanes, true>(p, lane, legalH, legalV);
+    if ((lane & (kLanes - 1)) == 0 && valid) legal_store(p, legalH, legalV, mask + 8 * b, pawn + 8 * b);
 }
 
 // ------------------------------------------------------------------------------------------
 // K1, two-phase form (the default above 4,096 states): the searches of ALL states go through one flat task list.
-//   legal_prepare_kernel : two lanes per state; everything of legal_mask_kernel up to the witness paths (lane 0: the mover's,
-//                          lane 1: the opponent's), then the (candidate, player) searches that are still needed are appended to a
-//                          global task list (one warp-aggregated atomicAdd) and the mask is written OPTIMISTICALLY (every gated
-//                          candidate legal);
+//   legal_prepare_kernel : two lanes per state; the prepare step, then the state's tasks are appended to a global task list (one
+//                          warp-aggregated atomicAdd) and the mask is written OPTIMISTICALLY (every gated candidate legal);
 //   legal_search_kernel  : persistent warps of 32 search state machines fed from the global list through a cursor: a lane whose
 //                          flood fill has finished (goal reached, or nothing new: clear the candidate's mask bit) takes the next
 //                          task while the others continue.  Fills that fail explore their whole region and take several times
@@ -206,8 +127,8 @@ legal_mask_kernel(const AqState *__restrict__ states, int64_t B, uint32_t *__res
 //                          fill and read-back as stages -- were built and measured: 13 instead of 11 active lanes per instruction, no
 //                          gain in time, because lanes in different stages split every round; dropped.)
 // The per-state number of searches is 0 .. ~60 with a mean of 2-4, so the one-kernel form spends most of its lanes waiting for the
-// slowest state of their warp.  A state whose tasks do not fit the list (capacity 8 per state on average) runs them itself, as
-// legal_mask_kernel does -- results never depend on the capacity.
+// slowest state of their warp.  A state whose tasks do not fit the list (capacity 8 per state on average) runs them itself
+// (legal_search_in_place) -- results never depend on the capacity.
 // task word: state index << 8 | slot | (orient - 1) << 6 | opponent << 7;  kNullTask = hole left by an overflow.
 // workspace: [0] number of tasks, [1] the search kernel's cursor, tasks from byte 256.
 // ------------------------------------------------------------------------------------------
@@ -227,7 +148,7 @@ legal_prepare_kernel(const AqState *__restrict__ states, int64_t B, uint32_t *__
     const bool valid = b0 < B;
     const int64_t b = valid ? b0 : B - 1;  // out-of-range lanes shadow the last state and write nothing
     LegalPrep p;
-    legal_prepare_state(load_state(states + b), lane, p);
+    legal_prepare_state<2>(load_state(states + b), lane, p);
     const int total = valid ? p.offs[4] : 0;
     const unsigned start = legal_reserve(total, lane, counter);  // list space for the whole warp with one atomic
     const bool fits = (u64)start + (unsigned)total <= cap;
@@ -235,13 +156,13 @@ legal_prepare_kernel(const AqState *__restrict__ states, int64_t B, uint32_t *__
     if (!total || fits) {
         // optimistic: every gated candidate legal (those whose witnesses survive need no search at all);
         // legal_search_kernel clears the bits of the candidates whose search fails
-        if (total) legal_emit_tasks(p, sub, [&](int i, uint32_t code) { tasks[start + i] = ((uint32_t)b << 8) | code; });
-        legalH = p.legalH | p.needH;
-        legalV = p.legalV | p.needV;
+        if (total) legal_for_tasks<2>(p, sub, [&](int i, uint32_t code) { tasks[start + i] = ((uint32_t)b << 8) | code; });
+        legalH = p.legalH;
+        legalV = p.legalV;
     } else {
         // the list is full: mark what is left of it as holes and run this state's searches here
         for (unsigned t = start + sub; t < cap; t += 2) tasks[t] = kNullTask;
-        legal_search_in_place(p, lane, legalH, legalV);
+        legal_search_in_place<2, false>(p, lane, legalH, legalV);
     }
     if (sub == 0 && valid) legal_store(p, legalH, legalV, mask + 8 * b, pawn + 8 * b);
 }

@@ -180,17 +180,17 @@ __device__ __forceinline__ void legal_warpgroup(const AqState *__restrict__ stat
         const bool valid = b0 < B;
         const int64_t b = valid ? b0 : board(i0);  // out-of-range lanes shadow the round's first state and write nothing
         LegalPrep p;
-        legal_prepare_state(load_state(states + b), lane, p);
+        legal_prepare_state<2>(load_state(states + b), lane, p);
         const int total = valid ? p.offs[4] : 0;
         const unsigned start = legal_reserve(total, lane, &L.count[par][0]);
         u64 legalH, legalV;
         if (!total || start + (unsigned)total <= (unsigned)kLegalCap) {
-            if (total) legal_emit_tasks(p, sub, [&](int k, uint32_t code) { L.task[start + k] = (unsigned short)((j << 8) | code); });
-            legalH = p.legalH | p.needH;
-            legalV = p.legalV | p.needV;
+            if (total) legal_for_tasks<2>(p, sub, [&](int k, uint32_t code) { L.task[start + k] = (unsigned short)((j << 8) | code); });
+            legalH = p.legalH;
+            legalV = p.legalV;
         } else {  // the list is full: mark what is left of it as holes and run this state's searches here
             for (unsigned t = start + sub; t < (unsigned)kLegalCap; t += 2) L.task[t] = kNullTask16;
-            legal_search_in_place(p, lane, legalH, legalV);
+            legal_search_in_place<2, false>(p, lane, legalH, legalV);
 #if TC2_OVERFLOW_COUNT
             if (sub == 0) atomicAdd(&g_tc2_overflow, 1ull);
 #endif

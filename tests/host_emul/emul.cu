@@ -1,9 +1,10 @@
-// Host-side emulation of the legal-mask kernel's per-state algorithm, compiled from the SAME
-// device header (aq_common.cuh is __host__ __device__).  Test-only: lets the CPU suite check the
-// bitboard restatement (flood fill with pawn rules, bit-parallel gate) against the golden
-// fixtures before any GPU time is spent.  The warp-level plumbing of the real kernel
-// (compaction, OR-reduction) is covered by the -m gpu tests.
-#include "../../alphaquoridorgnn_b200/csrc/aq_common.cuh"
+// Host build of the legal mask's per-state steps: the same device headers (aq_common.cuh and legal_steps.cuh are
+// __host__ __device__ where it matters) compiled for the host.  Test-only: lets the CPU suite check the bitboard
+// algorithm (flood fill with pawn rules, bit-parallel gate, witness paths and their task sets, the mask and pawn
+// packing) against the golden fixtures before any GPU time is spent.  The warp-level plumbing of the kernels (the
+// deal of the tasks to lanes, the task lists, the reductions) is covered by the -m gpu tests.
+#include <cstring>
+#include "../../alphaquoridorgnn_b200/csrc/legal_steps.cuh"
 using namespace aq;
 
 extern "C" void emul_pack(const uint8_t *rows, const int16_t *plies, long long B, AqState *out) {
@@ -20,45 +21,29 @@ extern "C" void emul_pack(const uint8_t *rows, const int16_t *plies, long long B
     }
 }
 
+// The kernels' steps one after another: wall sets, the two witness paths, the task sets, one search per task (a failed
+// search clears its candidate), the packing.
 extern "C" void emul_legal_mask(const AqState *states, long long B, uint32_t *mask, uint8_t *pawn) {
     for (long long b = 0; b < B; ++b) {
         const AqState s = states[b];
         const Open base = open_from_walls(s.hwalls, s.vwalls);
         const int me = s.ppos, en = 80 - (int)s.epos;
-        u64 legalH = 0, legalV = 0;
-        if (s.pwalls > 0) {
-            const WallSets ws = wall_sets(s.hwalls, s.vwalls);
-            legalH = ws.freeH;
-            legalV = ws.freeV;
-            // same decision structure as legal_mask_kernel: witness paths first, a real search only for the
-            // player whose witness the candidate cuts
-            const PathCuts pm_ = find_path_cuts(base, me, en, goal_row0());
-            const PathCuts pe_ = find_path_cuts(base, en, me, goal_row8());
+        WallSets ws{};
+        if (s.pwalls > 0) ws = wall_sets(s.hwalls, s.vwalls);
+        const PathCuts pc[2] = {find_path_cuts(base, me, en, goal_row0()), find_path_cuts(base, en, me, goal_row8())};
+        u64 set[4];
+        legal_task_sets(ws, pc, set);
+        u64 legal[2] = {ws.freeH | ws.needH, ws.freeV | ws.needV};
+        for (int q = 0; q < 4; ++q)
             for (int slot = 0; slot < 64; ++slot)
-                for (int orient = 1; orient <= 2; ++orient) {
-                    const u64 need = orient == 1 ? ws.needH : ws.needV;
-                    if (!((need >> slot) & 1)) continue;
-                    const u64 cm = orient == 1 ? pm_.cutH : pm_.cutV, ce = orient == 1 ? pe_.cutH : pe_.cutV;
+                if ((set[q] >> slot) & 1) {
                     Open o = base;
-                    add_wall(o, orient, slot);
-                    bool ok = true;
-                    if (!pm_.exists || ((cm >> slot) & 1)) ok = ok && reaches(o, me, en, goal_row0());
-                    if (!pe_.exists || ((ce >> slot) & 1)) ok = ok && reaches(o, en, me, goal_row8());
-                    if (ok) {
-                        if (orient == 1) legalH |= 1ull << slot; else legalV |= 1ull << slot;
-                    }
+                    add_wall(o, (q & 1) + 1, slot);
+                    if (!(q >> 1 ? reaches(o, en, me, goal_row8()) : reaches(o, me, en, goal_row0()))) legal[q & 1] &= ~(1ull << slot);
                 }
-        }
-        uint8_t pm[8] = {0, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0, 0};
-        const int n = pawn_moves(base, me, en, pm + 1);
-        pm[0] = (uint8_t)n;
-        u128 lo = 0;
-        for (int k = 0; k < n; ++k) lo |= (u128)1 << pm[1 + k];
-        lo |= (u128)legalH << 81;
-        const u128 hi = (u128)(legalH >> 47) | ((u128)legalV << 17);
-        uint32_t *m = mask + 8 * b;
-        for (int k = 0; k < 4; ++k) { m[k] = (uint32_t)(lo >> (32 * k)); m[4 + k] = (uint32_t)(hi >> (32 * k)); }
-        for (int k = 0; k < 8; ++k) pawn[8 * b + k] = pm[k];
+        const LegalWords w = legal_pack(base, me, en, legal[0], legal[1]);
+        memcpy(mask + 8 * b, w.mask, sizeof w.mask);
+        memcpy(pawn + 8 * b, w.pawn, sizeof w.pawn);
     }
 }
 

@@ -20,26 +20,21 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "..", "alphaquoridorgnn_b200", "csrc")
 
 # Number of path searches the prepare step leaves for a state (LegalPrep::offs[4] in legal_steps.cuh), from the host build of the
-# same header: the gated candidates that cut the mover's / the opponent's witness path (all of them when a player has no path).
+# same headers: the popcount of the task sets.
 _COUNT_SRC = r'''
-#include "aq_common.cuh"
+#include "legal_steps.cuh"
 using namespace aq;
 extern "C" void count_searches(const AqState *states, long long B, int *out) {
     for (long long b = 0; b < B; ++b) {
         const AqState s = states[b];
-        int n = 0;
-        if (s.pwalls > 0) {
-            const WallSets ws = wall_sets(s.hwalls, s.vwalls);
-            if (ws.needH | ws.needV) {
-                const Open base = open_from_walls(s.hwalls, s.vwalls);
-                const int me = s.ppos, en = 80 - (int)s.epos;
-                const PathCuts pc[2] = {find_path_cuts(base, me, en, goal_row0()), find_path_cuts(base, en, me, goal_row8())};
-                for (int p = 0; p < 2; ++p)
-                    n += __builtin_popcountll(ws.needH & (pc[p].exists ? pc[p].cutH : ~0ull)) +
-                         __builtin_popcountll(ws.needV & (pc[p].exists ? pc[p].cutV : ~0ull));
-            }
-        }
-        out[b] = n;
+        const Open base = open_from_walls(s.hwalls, s.vwalls);
+        const int me = s.ppos, en = 80 - (int)s.epos;
+        WallSets ws{};
+        if (s.pwalls > 0) ws = wall_sets(s.hwalls, s.vwalls);
+        const PathCuts pc[2] = {find_path_cuts(base, me, en, goal_row0()), find_path_cuts(base, en, me, goal_row8())};
+        u64 set[4];
+        legal_task_sets(ws, pc, set);
+        out[b] = __builtin_popcountll(set[0]) + __builtin_popcountll(set[1]) + __builtin_popcountll(set[2]) + __builtin_popcountll(set[3]);
     }
 }
 '''

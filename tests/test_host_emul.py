@@ -1,6 +1,7 @@
-"""CPU check of the bitboard algorithm used by the CUDA legal-mask kernel: the same device header
-(csrc/aq_common.cuh, __host__ __device__) is compiled for the host and run on every golden
-position.  No GPU needed; the GPU tests then cover the warp-level plumbing."""
+"""CPU check of the bitboard algorithm used by the CUDA legal-mask kernels: the same device headers
+(csrc/aq_common.cuh and the per-state steps of csrc/legal_steps.cuh, __host__ __device__) are compiled
+for the host and run on every golden position.  No GPU needed; the GPU tests then cover the warp-level
+plumbing."""
 import ctypes
 import os
 import subprocess
@@ -15,8 +16,8 @@ LIB = os.path.join(HERE, "host_emul", "libemul.so")
 
 @pytest.fixture(scope="module")
 def emul():
-    hdr = os.path.join(HERE, "..", "alphaquoridorgnn_b200", "csrc", "aq_common.cuh")
-    if not os.path.exists(LIB) or os.path.getmtime(LIB) < max(os.path.getmtime(SRC), os.path.getmtime(hdr)):
+    hdrs = [os.path.join(HERE, "..", "alphaquoridorgnn_b200", "csrc", h) for h in ("aq_common.cuh", "legal_steps.cuh")]
+    if not os.path.exists(LIB) or os.path.getmtime(LIB) < max(os.path.getmtime(f) for f in [SRC] + hdrs):
         subprocess.check_call(["nvcc", "-O2", "-std=c++17", "--expt-relaxed-constexpr", "-Wno-deprecated-gpu-targets",
                                "-Xcompiler", "-fPIC", "-shared", "-o", LIB, SRC],
                               env=dict(os.environ, CC="/usr/bin/gcc"))
