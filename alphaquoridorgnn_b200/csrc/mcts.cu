@@ -6,7 +6,8 @@
 //   aq_mcts_expand_backup  create the children in legal_actions() order with their priors
 //                          (pv_mcts.py:53-56) and back the value up with alternating sign (:60-66)
 // The reference has no virtual loss, no Dirichlet noise and no tree reuse, so batching ACROSS games
-// leaves every game's search unchanged.
+// leaves every game's search unchanged.  Tree reuse between moves (aq_mcts_advance, AlphaGo Zero) is an
+// opt-in addition the reference does not have; without it every search starts from aq_mcts_reset.
 //
 // Arithmetic is kept as the reference computes it under NumPy >= 2 (requirements.txt pins
 // numpy~=2.0.2, NEP 50 promotion): w accumulates in float64; the PUCT score is
@@ -63,6 +64,120 @@ __global__ void mcts_reset_kernel(MctsGame *games, MctsHot *hot, MctsCold *cold,
     rc.first_child = -1; rc.parent = -1; rc.n_children = 0; rc.action = -1; rc.pad = 0;
     hot[g * max_nodes] = rh;  // root node: Node(state, 0), pv_mcts.py:81
     cold[g * max_nodes] = rc;
+}
+
+__device__ __forceinline__ void write_fresh_root(MctsHot *hot, MctsCold *cold) {
+    MctsHot rh;
+    rh.w = 0.0; rh.prior = 0.f; rh.n = 0;
+    MctsCold rc;
+    rc.first_child = -1; rc.parent = -1; rc.n_children = 0; rc.action = -1; rc.pad = 0;
+    hot[0] = rh;
+    cold[0] = rc;
+}
+
+__device__ __forceinline__ bool same_position(const AqState &a, const AqState &b) {
+    return a.hwalls == b.hwalls && a.vwalls == b.vwalls && a.ppos == b.ppos && a.pwalls == b.pwalls && a.epos == b.epos &&
+           a.ewalls == b.ewalls && a.plies == b.plies;
+}
+
+// Breadth-first copy of the subtree below source node `from` into a destination arena, the arena itself serving as the queue:
+// node 0 is `from` (now a root), and every expanded node copied appends its children block at the tail, so blocks stay contiguous
+// and in legal_actions() order.  A copied node's first_child still holds the SOURCE index until the node is dequeued; the dequeue
+// appends that block and rewrites it.  Returns the node count, or 0 when tail + reserve_nodes would pass max_nodes: the copy
+// stops there and the caller writes a fresh root, so nothing depends on how far it had got.
+__device__ int copy_subtree(const MctsHot *__restrict__ shot, const MctsCold *__restrict__ scold, int from, MctsHot *hot, MctsCold *cold,
+                            int lane, int64_t max_nodes, int64_t reserve_nodes) {
+    if (lane == 0) {
+        hot[0] = shot[from];
+        MctsCold rc = scold[from];
+        rc.parent = -1;
+        rc.action = -1;
+        cold[0] = rc;
+    }
+    int tail = 1;
+    for (int head = 0; head < tail;) {
+        __syncwarp();  // the window's records were written by other lanes of this warp
+        const int end = min(head + 32, tail);
+        int sfc = -1, snc = 0;
+        if (head + lane < end) {
+            const MctsCold c = cold[head + lane];
+            sfc = c.first_child;
+            snc = c.n_children;
+        }
+        unsigned expanded = __ballot_sync(0xffffffffu, sfc >= 0);
+        while (expanded) {
+            const int j = __ffs(expanded) - 1;
+            expanded &= expanded - 1;
+            const int fc = __shfl_sync(0xffffffffu, sfc, j), nc = __shfl_sync(0xffffffffu, snc, j);
+            if ((int64_t)tail + nc + reserve_nodes > max_nodes) return 0;
+            for (int c = lane; c < nc; c += 32) {
+                hot[tail + c] = shot[fc + c];
+                MctsCold cc = scold[fc + c];
+                cc.parent = head + j;
+                cold[tail + c] = cc;
+            }
+            if (lane == j) cold[head + j].first_child = tail;
+            tail += nc;
+        }
+        head = end;
+    }
+    return tail;
+}
+
+// One warp per destination game (aq_mcts_advance): follow the path from the source game's root with a ballot over each children
+// block, check the position reached against roots[g], then carry the subtree or start from a fresh root.
+__global__ void __launch_bounds__(128)
+mcts_advance_kernel(const MctsGame *__restrict__ src_games, const MctsHot *__restrict__ src_hot_all, const MctsCold *__restrict__ src_cold_all,
+                    int64_t G_src, MctsGame *dst_games, MctsHot *dst_hot_all, MctsCold *dst_cold_all, int64_t G_dst, int64_t max_nodes,
+                    const AqState *__restrict__ roots, const int64_t *__restrict__ src_game, const int16_t *__restrict__ path, int path_len,
+                    int64_t reserve_nodes, int32_t *__restrict__ kept, int32_t *__restrict__ status) {
+    const int lane = threadIdx.x & 31;
+    const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (g >= G_dst) return;
+    MctsHot *hot = dst_hot_all + g * max_nodes;
+    MctsCold *cold = dst_cold_all + g * max_nodes;
+    const AqState root = load_state(roots + g);
+    const int64_t s = src_game[g];
+    int count = 0;  // nodes carried, 0 = fresh root
+    if (s < -1 || s >= G_src) {
+        if (lane == 0) atomicAdd(status, 1);
+    } else if (s >= 0) {
+        const MctsHot *shot = src_hot_all + s * max_nodes;
+        const MctsCold *scold = src_cold_all + s * max_nodes;
+        AqState st = load_state(&src_games[s].root);
+        int node = 0;  // -1 once the path leaves the tree
+        for (int i = 0; i < path_len; ++i) {
+            const int a = path[g * path_len + i];
+            st = state_after(st, a);
+            if (node < 0) continue;
+            const int first = scold[node].first_child, nc = first < 0 ? 0 : scold[node].n_children;
+            int found = -1;
+            for (int c0 = 0; c0 < nc && found < 0; c0 += 32) {
+                const int c = c0 + lane;
+                const unsigned hit = __ballot_sync(0xffffffffu, c < nc && scold[first + c].action == a);
+                if (hit) found = first + c0 + __ffs(hit) - 1;
+            }
+            node = found;
+        }
+        if (!same_position(st, root)) {
+            if (lane == 0) atomicAdd(status, 1);
+        } else if (node >= 0 && shot[node].n >= 1) {
+            count = copy_subtree(shot, scold, node, hot, cold, lane, max_nodes, reserve_nodes);
+        }
+    }
+    __syncwarp();
+    if (lane == 0) {
+        if (count == 0) write_fresh_root(hot, cold);
+        MctsGame gm;
+        gm.root = root;
+        gm.node_count = count ? count : 1;
+        gm.leaf = 0;
+        gm.leaf_kind = 0;
+        gm.overflow = 0;
+        gm.pad[0] = gm.pad[1] = gm.pad[2] = gm.pad[3] = 0;
+        dst_games[g] = gm;
+        if (kept) kept[g] = count;
+    }
 }
 
 // Descent of game g by its warp (pv_mcts.py:69-78).  The node arrays are read through plain pointers: in the fused kernel the same
@@ -409,6 +524,25 @@ extern "C" int aq_mcts_reset(void *ws, const AqState *roots, int64_t G, int64_t 
     mcts_reset_kernel<<<(unsigned)((G + 127) / 128), 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
         games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), roots, G, max_nodes);
     return aq_check_launch("aq_mcts_reset");
+}
+
+extern "C" int aq_mcts_advance(const void *src_ws, int64_t G_src, void *dst_ws, int64_t G_dst, int64_t max_nodes, const AqState *roots,
+                               const int64_t *src_game, const int16_t *path, int path_len, int64_t reserve_nodes, int32_t *kept,
+                               int32_t *status, void *stream) {
+    if (G_src <= 0 || G_dst <= 0 || max_nodes < 1 || max_nodes > INT32_MAX || path_len < 1 || reserve_nodes < 0 ||
+        reserve_nodes >= max_nodes || !src_ws || !dst_ws || !roots || !src_game || !path || !status)
+        return aq_set_error(AQ_ERR_ARG, "aq_mcts_advance");
+    const uintptr_t s0 = reinterpret_cast<uintptr_t>(src_ws), d0 = reinterpret_cast<uintptr_t>(dst_ws);
+    const uintptr_t s1 = s0 + (uintptr_t)aq_mcts_ws_bytes(G_src, max_nodes), d1 = d0 + (uintptr_t)aq_mcts_ws_bytes(G_dst, max_nodes);
+    if (s0 < d1 && d0 < s1) return aq_set_error(AQ_ERR_ARG, "aq_mcts_advance: the workspaces overlap");
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    cudaError_t e = cudaMemsetAsync(status, 0, sizeof(int32_t), st);
+    if (e != cudaSuccess) return aq_set_error((int)e, "aq_mcts_advance");
+    void *src = const_cast<void *>(src_ws);
+    mcts_advance_kernel<<<(unsigned)((G_dst + 3) / 4), 128, 0, st>>>(games_of(src), hot_of(src, G_src), cold_of(src, G_src, max_nodes), G_src,
+                                                                    games_of(dst_ws), hot_of(dst_ws, G_dst), cold_of(dst_ws, G_dst, max_nodes), G_dst,
+                                                                    max_nodes, roots, src_game, path, path_len, reserve_nodes, kept, status);
+    return aq_check_launch("aq_mcts_advance");
 }
 
 extern "C" int aq_mcts_select(void *ws, int64_t G, int64_t max_nodes, float c_puct, AqState *leaf_states,

@@ -5,6 +5,8 @@ the GPU (csrc/mcts.cu): G games are searched in lock-step, so the leaf of every 
 forms one batch for the network (batched leaf evaluation = model.predict for G states at once,
 pv_mcts.py:47).  The reference has no virtual loss, no Dirichlet noise and no tree reuse
 (pv_mcts.py:81 builds a fresh root per move), so each game's search is exactly the reference's.
+Tree reuse between moves (AlphaGo Zero: the child of the played move becomes the next root with its
+statistics) is opt-in, BatchedMCTS(..., tree_reuse=True); the default keeps the reference's fresh root.
 """
 from copy import deepcopy
 
@@ -32,27 +34,37 @@ class BatchedMCTS:
 
     `evaluator` is either a GNNNetwork (leaf evaluation = aq_leaf_eval into preallocated buffers, and the
     whole simulation step -- select, legal mask, GNN trunk, heads, expand+backup -- is captured once in a
-    CUDA graph and replayed `sims` times) or any callable following the evaluator protocol (eager loop)."""
+    CUDA graph and replayed `sims` times) or any callable following the evaluator protocol (eager loop).
 
-    def __init__(self, evaluator, sims=None, c_puct=C_PUCT, device=None, use_graph=True):
+    tree_reuse=True (AlphaGo Zero; the reference has none): a search may continue the tree of the previous one
+    (search(..., src_row, path)).  `sims` is then required: each game's arena holds 1 + 2 * sims * MAX_CHILDREN nodes, room
+    for one carried search and one new one, and two workspaces are used in turn (the previous search's tree is read from one
+    while the next is built in the other)."""
+
+    def __init__(self, evaluator, sims=None, c_puct=C_PUCT, device=None, use_graph=True, tree_reuse=False):
+        if tree_reuse and not sims:
+            raise ValueError("BatchedMCTS(tree_reuse=True) needs `sims` at construction: it sizes the node arena")
         self.model = evaluator if hasattr(evaluator, "flat_parameters") else None
         self.evaluator = network_evaluator(evaluator) if hasattr(evaluator, "predict_batch") else evaluator
         self.sims = sims
         self.c_puct = float(c_puct)
         self.device = gl._dev(device)
         self.use_graph = use_graph
-        self._ws = None
+        self.tree_reuse = bool(tree_reuse)
+        self._ws = [None, None] if self.tree_reuse else [None]
+        self._last = None     # tree_reuse: (workspace slot, G) of the previous search, the source a next search can continue
+        self.last_kept = None  # tree_reuse: int32[G] nodes carried into each row by the last search (0 = fresh root), else None
         self._buf = {}
         self._graphs = {}
         self._warm = False   # one eager simulation step has run (lazy initialisation is done)
 
-    def _workspace(self, G, max_nodes):
+    def _workspace(self, G, max_nodes, slot=0):
         L = _lib.load()
         need = L.aq_mcts_ws_bytes(G, max_nodes)
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = torch.empty((need,), dtype=torch.uint8, device=self.device)
+        if self._ws[slot] is None or self._ws[slot].numel() < need:
+            self._ws[slot] = torch.empty((need,), dtype=torch.uint8, device=self.device)
             self._graphs.clear()  # graphs hold raw pointers into the old workspace
-        return self._ws
+        return self._ws[slot]
 
     def _buffers(self, G):
         if G not in self._buf:
@@ -104,17 +116,27 @@ class BatchedMCTS:
         return g
 
     @torch.no_grad()
-    def search_async(self, roots, sims=None):
-        """search() without the synchronisation: returns (counts, actions, n_children, status int32[2] on the device); the caller
+    def search_async(self, roots, sims=None, src_row=None, path=None):
+        """search() without the synchronisation: returns (counts, actions, n_children, status int32[3] on the device); the caller
         passes status.tolist() to check_status() when it synchronises anyway."""
         sims = sims or self.sims or PV_EVALUATE_COUNT
         L, P = _lib.load(), _lib.ptr
         dev = self.device
         roots = roots.to(dev).contiguous()
         G_real = roots.shape[0]
+        if src_row is not None:
+            if not self.tree_reuse:
+                raise ValueError("search(src_row=...) continues a tree: construct the searcher with tree_reuse=True")
+            if self._last is None:
+                raise ValueError("search(src_row=...) needs a previous search of this searcher to continue")
+            if path is None:
+                raise ValueError("search(src_row=...) needs the path of actions from each source root")
+        if self.tree_reuse and sims > self.sims:
+            raise ValueError(f"this searcher's node arena holds {self.sims} simulations per search, not {sims}")
         if G_real == 0:
+            self.last_kept = None
             return (torch.empty((0, gl.MAX_LEGAL), dtype=torch.int32, device=dev), torch.empty((0, gl.MAX_LEGAL), dtype=torch.int16, device=dev),
-                    torch.empty((0,), dtype=torch.int16, device=dev), torch.zeros((2,), dtype=torch.int32, device=dev))
+                    torch.empty((0,), dtype=torch.int16, device=dev), torch.zeros((3,), dtype=torch.int32, device=dev))
         # Self-play and the arena drop finished games, so the number of roots shrinks by a few almost every ply.  Batches above 256
         # are padded to the next multiple of 256 with copies of the last root (searched and discarded; games are independent, so the
         # real ones are unaffected): workspaces, buffers and the captured CUDA graph of the simulation step are then reused across
@@ -123,19 +145,41 @@ class BatchedMCTS:
             pad = 256 - G_real % 256
             roots = torch.cat([roots, roots[-1:].expand(pad, -1)]).contiguous()
         G = roots.shape[0]
-        max_nodes = 1 + sims * MAX_CHILDREN
-        ws = self._workspace(G, max_nodes)
+        if self.tree_reuse:
+            max_nodes = 1 + 2 * self.sims * MAX_CHILDREN
+            slot = 0 if self._last is None else 1 - self._last[0]
+        else:
+            max_nodes, slot = 1 + sims * MAX_CHILDREN, 0
+        ws = self._workspace(G, max_nodes, slot)
         buf = self._buffers(G)
+        # [arena overflow, NaN leaf value, inconsistent tree-reuse rows]
+        status = torch.zeros((3,), dtype=torch.int32, device=dev)
         with torch.cuda.device(dev):
             st = _lib.stream_ptr(dev)
-            _lib.check(L.aq_mcts_reset(P(ws), P(roots), G, max_nodes, st), "aq_mcts_reset")
+            if src_row is not None:
+                src_slot, G_src = self._last
+                src = src_row.to(device=dev, dtype=torch.int64).reshape(G_real)
+                path = path.to(device=dev, dtype=torch.int16).reshape(G_real, -1)
+                if G > G_real:  # padded rows start fresh
+                    src = torch.cat([src, src.new_full((G - G_real,), -1)])
+                    path = torch.cat([path, path.new_zeros((G - G_real, path.shape[1]))])
+                src, path = src.contiguous(), path.contiguous()
+                kept = torch.empty((G,), dtype=torch.int32, device=dev)
+                _lib.check(L.aq_mcts_advance(P(self._ws[src_slot]), G_src, P(ws), G, max_nodes, P(roots), P(src), P(path), path.shape[1],
+                                             sims * MAX_CHILDREN, P(kept), P(status[2:]), st), "aq_mcts_advance")
+                self.last_kept = kept[:G_real]
+            else:
+                _lib.check(L.aq_mcts_reset(P(ws), P(roots), G, max_nodes, st), "aq_mcts_reset")
+                self.last_kept = None
+            if self.tree_reuse:
+                self._last = (slot, G)
             if self.model is not None:
                 from .pv_network_gnn import PRECISIONS
                 flat = self.model.flat_parameters()
                 prec = PRECISIONS[self.model.precision]
                 # bf16 operand tiles, refreshed in place if the parameters changed since the last search
                 prep = self.model.prepared_weights() if prec == 1 else None
-                key = (G, max_nodes, flat.data_ptr(), prep.data_ptr() if prep is not None else 0, prec)
+                key = (G, max_nodes, ws.data_ptr(), flat.data_ptr(), prep.data_ptr() if prep is not None else 0, prec)
                 graphs = self._graphs.get(key) if self.use_graph else None
                 done = 0
                 if self.use_graph:
@@ -183,26 +227,34 @@ class BatchedMCTS:
             counts = torch.empty((G, gl.MAX_LEGAL), dtype=torch.int32, device=dev)
             actions = torch.empty((G, gl.MAX_LEGAL), dtype=torch.int16, device=dev)
             n = torch.empty((G,), dtype=torch.int16, device=dev)
-            ovf = torch.zeros((1,), dtype=torch.int32, device=dev)
-            _lib.check(L.aq_mcts_root_counts(P(ws), G, max_nodes, P(counts), P(actions), P(n), P(ovf), st),
+            _lib.check(L.aq_mcts_root_counts(P(ws), G, max_nodes, P(counts), P(actions), P(n), P(status[:1]), st),
                        "aq_mcts_root_counts")
-            bad = torch.isnan(buf["value"]).any().to(torch.int32).reshape(1) if self.model is not None else torch.zeros_like(ovf)
-        return counts[:G_real], actions[:G_real], n[:G_real], torch.cat([ovf, bad])
+            if self.model is not None:
+                status[1:2].copy_(torch.isnan(buf["value"]).any().reshape(1))
+        return counts[:G_real], actions[:G_real], n[:G_real], status
 
     @staticmethod
     def check_status(status):
-        """status: the two flags search_async returns, as host integers."""
+        """status: the three flags search_async returns, as host integers."""
         if status[0]:
             raise _lib.AqError("MCTS node arena overflow")
+        if status[2]:
+            raise _lib.AqError(f"tree reuse: {status[2]} row(s) named a source game out of range or a root that is not the position "
+                               "the path leads to from the source root")
         if status[1]:
             raise _lib.AqError("the network returned NaN for a leaf: with precision 'bf16' that is how an activation beyond the fp16 range of the "
                                "aggregation operand is reported (gnn_tc2.cu); evaluate this network with precision 'fp32'")
 
-    def search(self, roots, sims=None):
+    def search(self, roots, sims=None, src_row=None, path=None):
         """roots: packed uint8[G,32] (non-terminal states).  Runs `sims` simulations per game
         (pv_mcts.py:84) and returns (counts int32[G,136], actions int16[G,136], n_children int16[G]):
-        visit counts of the root's children in State.legal_actions() order (pv_mcts.py:88)."""
-        counts, actions, n, status = self.search_async(roots, sims)
+        visit counts of the root's children in State.legal_actions() order (pv_mcts.py:88).
+
+        With tree_reuse, src_row int64[G] (row of the previous search, -1 = fresh root) and path int16[G, k] (k = 1: the move
+        played from that row's root; 2: and the reply) continue the previous search's trees: row g keeps the subtree below the
+        path's end when that node was visited and its subtree leaves room for `sims` more simulations, else it starts fresh.
+        The counts then include the carried visits; last_kept gives the nodes carried per row."""
+        counts, actions, n, status = self.search_async(roots, sims, src_row, path)
         self.check_status(status.tolist())   # one synchronisation for both flags
         return counts, actions, n
 
@@ -218,19 +270,19 @@ class _SearcherCache(dict):
         return (_SearcherCache, ())
 
 
-def searcher_for(evaluator, sims, device=None):
+def searcher_for(evaluator, sims, device=None, tree_reuse=False):
     """The BatchedMCTS of a network for `sims` simulations, kept on the network object: its node arenas (3.5 GB at 4,096 games x
     200 simulations), leaf buffers and captured graphs are reused by every later self-play / arena / policy call on that network
     instead of being allocated and captured again.  Evaluators that are plain callables get a fresh searcher."""
     dev = gl._dev(device)
     if not hasattr(evaluator, "flat_parameters"):
-        return BatchedMCTS(evaluator, sims, device=dev)
+        return BatchedMCTS(evaluator, sims, device=dev, tree_reuse=tree_reuse)
     cache = evaluator.__dict__.setdefault("_searchers", _SearcherCache())
-    key = (int(sims), str(dev))
+    key = (int(sims), str(dev), bool(tree_reuse))
     if key not in cache:
         if len(cache) >= 4:
             cache.clear()
-        cache[key] = BatchedMCTS(evaluator, sims, device=dev)
+        cache[key] = BatchedMCTS(evaluator, sims, device=dev, tree_reuse=tree_reuse)
     return cache[key]
 
 

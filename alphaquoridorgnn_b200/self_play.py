@@ -42,23 +42,27 @@ def write_data(history, directory='./data/'):
 
 @torch.no_grad()
 def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_TEMPERATURE, seed=None, max_plies=None,
-                      policy_dtype=torch.float64):
+                      policy_dtype=torch.float64, tree_reuse=False):
     """Execute `num_games` self-play games in lock-step (self_play.py:40-68 per game) and keep the record on the device:
     dict(states uint8[T,32] packed, policy [T,209] search policies over all actions (self_play.py:51-54), value f32[T]
     back-filled game results seen from the player to move (self_play.py:63-66), game int64[T], ply int64[T],
-    flags uint8[G] (bit 0 = the player to move at the end has lost, bit 1 = draw), plies int64[G], sims int = simulations run).
+    flags uint8[G] (bit 0 = the player to move at the end has lost, bit 1 = draw), plies int64[G], sims int = new simulations
+    run, reused int = searches that continued a carried tree).
 
     Per ply: one search (200 graph-replayed simulation steps in a handful of launches) and ONE library call,
     aq_selfplay_advance -- search policy, its dense 209-wide record, the sampled move, the next states and the compaction of the
     games still running -- then one synchronisation that reads the search's status flags and the number of survivors together.
-    A game's moves are drawn from a hash of (seed, game, ply): they do not depend on the other games of the batch."""
+    A game's moves are drawn from a hash of (seed, game, ply): they do not depend on the other games of the batch.
+
+    tree_reuse=True (AlphaGo Zero; the reference builds a fresh root per move): each search continues the tree of the game's
+    previous one below the move played, so its policy counts the carried root visits as well as the `sims` new ones."""
     if policy_dtype not in (torch.float64, torch.float32):
         raise ValueError("policy_dtype must be torch.float64 or torch.float32")
     dev = gl._dev(device)
     L, P = _lib.load(), _lib.ptr
     seed = (int(seed) if seed is not None else int(torch.seed())) & (2 ** 64 - 1)
     sims = sims or pv_mcts.PV_EVALUATE_COUNT
-    mcts = pv_mcts.searcher_for(model, sims, dev)
+    mcts = pv_mcts.searcher_for(model, sims, dev, tree_reuse=tree_reuse)
     states = start_states(num_games, dev)
     game_id = torch.arange(num_games, device=dev)
     rec_state, rec_policy, rec_game, sizes = [], [], [], []
@@ -66,31 +70,41 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
     final_plies = torch.zeros(max(num_games, 1), dtype=torch.int64, device=dev)
     ws = torch.empty((max(1, L.aq_selfplay_ws_bytes(num_games)),), dtype=torch.uint8, device=dev)
     alive = torch.zeros((1,), dtype=torch.int32, device=dev)
-    ply, sims_run = 0, 0
+    ply, sims_run, reused = 0, 0, 0
+    src_row = path = None
     with torch.cuda.device(dev):
         while states.shape[0] > 0 and (max_plies is None or ply < max_plies):
             G = states.shape[0]
-            counts, actions, n, status = mcts.search_async(states)
+            counts, actions, n, status = mcts.search_async(states, src_row=src_row, path=path)
             sims_run += G * sims
             dense = torch.empty((G, POLICY_OUTPUT_SIZE), dtype=policy_dtype, device=dev)
             nxt = torch.empty_like(states)
             nxt_id = torch.empty_like(game_id)
+            chosen = torch.empty((G,), dtype=torch.int16, device=dev) if tree_reuse else None
             _lib.check(L.aq_selfplay_advance(P(states), P(counts), P(actions), P(n), P(game_id), G, float(temperature), seed, ply,
-                                             P(dense), int(policy_dtype == torch.float64), None, P(nxt), P(nxt_id), P(final_flags),
+                                             P(dense), int(policy_dtype == torch.float64), P(chosen), P(nxt), P(nxt_id), P(final_flags),
                                              P(final_plies), P(alive), P(ws), _lib.stream_ptr(dev)), "aq_selfplay_advance")
-            flags = torch.cat([status, alive]).tolist()      # the ply's only synchronisation
-            mcts.check_status(flags)
+            parts = [status, alive]
+            if mcts.last_kept is not None:
+                parts.append((mcts.last_kept > 0).sum(dtype=torch.int32).reshape(1))
+            flags = torch.cat(parts).tolist()      # the ply's only synchronisation
+            mcts.check_status(flags[:3])
+            reused += flags[4] if len(flags) > 4 else 0
             rec_state.append(states)
             rec_policy.append(dense)
             rec_game.append(game_id)
             sizes.append(G)
             ply += 1
-            states, game_id = nxt[:flags[2]], nxt_id[:flags[2]]
+            if tree_reuse:
+                # the compaction keeps game_id ascending, so a survivor's previous row is found by binary search
+                src_row = torch.searchsorted(game_id, nxt_id[:flags[3]])
+                path = chosen[src_row].reshape(-1, 1)
+            states, game_id = nxt[:flags[3]], nxt_id[:flags[3]]
     if not sizes:
         z = torch.zeros((0,), dtype=torch.int64, device=dev)
         return {"states": states, "policy": torch.zeros((0, POLICY_OUTPUT_SIZE), dtype=policy_dtype, device=dev),
                 "value": torch.zeros((0,), dtype=torch.float32, device=dev), "game": z, "ply": z, "flags": final_flags[:num_games],
-                "plies": final_plies[:num_games], "sims": 0}
+                "plies": final_plies[:num_games], "sims": 0, "reused": 0}
     game = torch.cat(rec_game)
     plyv = torch.repeat_interleave(torch.arange(len(sizes), device=dev), torch.tensor(sizes, device=dev))
     final_flags, final_plies = final_flags[:num_games], final_plies[:num_games]
@@ -100,13 +114,13 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
     fpv = torch.where(lost, torch.where(final_plies[game] % 2 == 0, -1.0, 1.0), 0.0)
     value = torch.where(plyv % 2 == 0, fpv, -fpv).to(torch.float32)
     return {"states": torch.cat(rec_state), "policy": torch.cat(rec_policy), "value": value, "game": game, "ply": plyv,
-            "flags": final_flags, "plies": final_plies, "sims": sims_run}
+            "flags": final_flags, "plies": final_plies, "sims": sims_run, "reused": reused}
 
 
-def play_batch(model, num_games, device=None, sims=None, temperature=SP_TEMPERATURE, seed=None, max_plies=None):
+def play_batch(model, num_games, device=None, sims=None, temperature=SP_TEMPERATURE, seed=None, max_plies=None, tree_reuse=False):
     """play_batch_device + conversion to the reference's history: a list of [[player, enemy, walls], policy (209 floats), value]
     (self_play.py:51-54, 63-66), games in order, plies in order within a game.  Returns (history, dict with per-game results)."""
-    rec = play_batch_device(model, num_games, device, sims, temperature, seed, max_plies)
+    rec = play_batch_device(model, num_games, device, sims, temperature, seed, max_plies, tree_reuse=tree_reuse)
     rows, _ = gl.unpack_rows(rec["states"])
     rows = rows.cpu().numpy()
     pols = rec["policy"].cpu().numpy()
@@ -126,14 +140,15 @@ def play(model, device=None):
     return history
 
 
-def self_play(game_count=None, model_path=None, data_dir='./data/', rank=0, world_size=1, sims=None, seed=None):
+def self_play(game_count=None, model_path=None, data_dir='./data/', rank=0, world_size=1, sims=None, seed=None, tree_reuse=False):
     """Perform self-play games and save the training data (self_play.py:71-98).  With
-    world_size > 1 each rank plays its share of the games on its own GPU and rank 0 writes the file."""
+    world_size > 1 each rank plays its share of the games on its own GPU and rank 0 writes the file.
+    tree_reuse=True keeps each game's search tree between moves (see play_batch_device)."""
     game_count = SP_GAME_COUNT if game_count is None else game_count
     model = GNNNetwork()
     model.prep_for_inference(model_path=model_path or (PV_NETWORK_PATH + 'best.pth'))
     mine = game_count // world_size + (1 if rank < game_count % world_size else 0)
-    history, _ = play_batch(model, mine, sims=sims, seed=None if seed is None else seed + rank) if mine else ([], None)
+    history, _ = play_batch(model, mine, sims=sims, seed=None if seed is None else seed + rank, tree_reuse=tree_reuse) if mine else ([], None)
     if world_size > 1:
         import torch.distributed as dist
         gathered = [None] * world_size if rank == 0 else None

@@ -53,7 +53,7 @@ typedef struct AqState {
     uint64_t reserved; /* reserved, 0 */
 } AqState;
 
-#define AQ_VERSION 205 /* bumped with every change of a signature below; the ctypes loader refuses a library of another version */
+#define AQ_VERSION 206 /* bumped with every change of a signature below; the ctypes loader refuses a library of another version */
 int aq_version(void);
 const char *aq_last_error_string(void);
 /* Number of kernels this library has launched in the process so far (monotonic; kernels replayed through a CUDA graph the caller
@@ -257,6 +257,19 @@ int aq_host_ctx_stats(void *host_ctx, int64_t *out2);
  *   (pv_mcts.py:88), n_children[g]; overflow[0] != 0 if any arena was exhausted. */
 int64_t aq_mcts_ws_bytes(int64_t G, int64_t max_nodes);
 int aq_mcts_reset(void *ws, const AqState *roots, int64_t G, int64_t max_nodes, void *stream);
+/* Tree reuse between moves (AlphaGo Zero; the reference has none): destination game g continues the tree of source game
+ * src_game[g] (-1 = fresh root).  Walk path[g, 0..path_len) from that game's root: path_len = 1 for the own move, 2 for the own
+ * move and the opponent's reply.  If the node reached was visited (n >= 1) and its subtree has at most max_nodes - reserve_nodes
+ * nodes, that subtree becomes game g's tree, with w, n, prior, child order and n_children bit-identical.  Otherwise game g starts
+ * from a fresh root, exactly as aq_mcts_reset makes it.
+ *   roots [G_dst]    the new root states (also used for fresh rows); for a carried row, state_after(src root, path) must
+ *                    equal roots[g].  A mismatch, or src_game out of range, makes the row fresh and is counted in status[0]
+ *   kept  [G_dst]    nodes carried, 0 = fresh (may be NULL)
+ *   src_ws, dst_ws   workspaces laid out for G_src / G_dst games with the same max_nodes; they must not overlap
+ * AQ_ERR_ARG for sizes < 1, path_len < 1, reserve_nodes outside [0, max_nodes) or overlapping workspaces. */
+int aq_mcts_advance(const void *src_ws, int64_t G_src, void *dst_ws, int64_t G_dst, int64_t max_nodes, const AqState *roots,
+                    const int64_t *src_game, const int16_t *path, int path_len, int64_t reserve_nodes, int32_t *kept,
+                    int32_t *status, void *stream);
 int aq_mcts_select(void *ws, int64_t G, int64_t max_nodes, float c_puct, AqState *leaf_states, int32_t *leaf_kind,
                    void *stream);
 int aq_mcts_expand_backup(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values,
