@@ -13,10 +13,11 @@ typedef unsigned long long u64;
 
 int aq_set_error(int code, const char *what);
 int aq_check_launch(const char *what);
+int aq_num_sms();  // multiprocessors of the current device (148 if the query fails)
 
-// Programmatic dependent launch (PDL).  A kernel launched with aq_launch_pdl may start while its predecessor in the stream is still
-// draining; it must call aq_pdl_wait() before it touches anything the predecessor (or anything earlier in the stream) writes, and may
-// run a prologue that reads only long-lived inputs (parameters) before that.  A predecessor that calls aq_pdl_trigger() at its start
+// Programmatic dependent launch (PDL).  A kernel launched by aq_launch with pdl = true may start while its predecessor in the stream is
+// still draining; it must call aq_pdl_wait() before it touches anything the predecessor (or anything earlier in the stream) writes, and
+// may run a prologue that reads only long-lived inputs (parameters) before that.  A predecessor that calls aq_pdl_trigger() at its start
 // lets the dependent grid be scheduled as soon as SM resources free up; without the trigger the dependent starts when the
 // predecessor's blocks have exited, as with a normal launch.  Both device calls are no-ops for normally launched kernels.
 // RULE: what the predecessor wrote must be read with coherent loads (__ldcg / plain loads through a non-restrict pointer) after
@@ -25,19 +26,30 @@ int aq_check_launch(const char *what);
 #ifdef __CUDACC__
 __device__ __forceinline__ void aq_pdl_wait() { asm volatile("griddepcontrol.wait;\n" ::: "memory"); }
 __device__ __forceinline__ void aq_pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;\n" ::: "memory"); }
+// Every kernel launch of the library: raises the kernel's dynamic shared-memory limit to `smem` when it uses any, launches (with the
+// programmatic-stream-serialization attribute when `pdl` is set) and counts the launch.  Returns 0, or the error reported under `what`.
 template <typename... KArgs, typename... Args>
-static inline cudaError_t aq_launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kernel, args...);
+static inline int aq_launch(const char *what, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, bool pdl,
+                            Args... args) {
+    cudaError_t e = smem > 0 ? cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) : cudaSuccess;
+    if (e == cudaSuccess) {
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = grid;
+        cfg.blockDim = block;
+        cfg.dynamicSmemBytes = smem;
+        cfg.stream = st;
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        attr[0].val.programmaticStreamSerializationAllowed = 1;
+        cfg.attrs = attr;
+        cfg.numAttrs = pdl ? 1 : 0;
+        e = cudaLaunchKernelEx(&cfg, kernel, args...);
+    }
+    if (e != cudaSuccess) {
+        (void)cudaGetLastError();  // the failed call is also this thread's last error: clear it so that the next launch is not blamed
+        return aq_set_error((int)e, what);
+    }
+    return aq_check_launch(what);
 }
 #endif
 

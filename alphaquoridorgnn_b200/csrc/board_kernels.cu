@@ -23,8 +23,9 @@ int aq_set_error(int code, const char *what) {
     return code;
 }
 
-// every kernel launch of the library is followed by aq_check_launch: the successful ones are counted (aq_launch_count), so
-// that a caller can state how many of this library's kernels ran in a region instead of assuming it (bench.py: gpu_launches)
+// every kernel launch of the library goes through aq_launch (aq_common.cuh), which ends in aq_check_launch: the successful ones are
+// counted (aq_launch_count), so that a caller can state how many of this library's kernels ran in a region instead of assuming it
+// (bench.py: gpu_launches)
 static std::atomic<long long> g_launches{0};
 
 int aq_check_launch(const char *what) {
@@ -35,6 +36,17 @@ int aq_check_launch(const char *what) {
 }
 
 extern "C" int64_t aq_launch_count(void) { return (int64_t)g_launches.load(std::memory_order_relaxed); }
+
+int aq_num_sms() {
+    static int sms = 0;
+    if (sms == 0) {
+        int dev = 0, n = 0;
+        cudaGetDevice(&dev);
+        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
+        sms = n > 0 ? n : 148;
+    }
+    return sms;
+}
 
 extern "C" int aq_version(void) { return AQ_VERSION; }
 extern "C" const char *aq_last_error_string(void) { return g_err; }
@@ -401,15 +413,13 @@ static inline unsigned blocks_for(int64_t n, int per) { return (unsigned)((n + p
 extern "C" int aq_pack_states(const uint8_t *rows68, const int16_t *plies, int64_t B, AqState *out, void *stream) {
     if (B < 0 || (B > 0 && (!rows68 || !out))) return aq_set_error(AQ_ERR_ARG, "aq_pack_states");
     if (B == 0) return 0;
-    pack_states_kernel<<<blocks_for(B, 8), 256, 0, S(stream)>>>(rows68, plies, B, out);
-    return aq_check_launch("aq_pack_states");
+    return aq_launch("aq_pack_states", pack_states_kernel, blocks_for(B, 8), 256, 0, S(stream), false, rows68, plies, B, out);
 }
 
 extern "C" int aq_unpack_states(const AqState *states, int64_t B, uint8_t *rows68, int16_t *plies, void *stream) {
     if (B < 0 || (B > 0 && (!rows68 || !states))) return aq_set_error(AQ_ERR_ARG, "aq_unpack_states");
     if (B == 0) return 0;
-    unpack_states_kernel<<<blocks_for(B, 8), 256, 0, S(stream)>>>(states, B, rows68, plies);
-    return aq_check_launch("aq_unpack_states");
+    return aq_launch("aq_unpack_states", unpack_states_kernel, blocks_for(B, 8), 256, 0, S(stream), false, states, B, rows68, plies);
 }
 
 static inline size_t legal_task_cap(int64_t B) { const int64_t n = B < kLegalChunk ? B : kLegalChunk; return (size_t)(8 * n + 4096); }
@@ -425,12 +435,13 @@ extern "C" int aq_legal_mask_ws(const AqState *states, int64_t B, uint32_t *mask
     if (!ws || B <= 4096) {
         const int lanes = B <= 1024 ? 32 : B <= 16384 ? 8 : 2;
         if (lanes == 32)
-            legal_mask_kernel<32><<<blocks_for(B, kLegalWarps * 1), kLegalWarps * 32, 0, S(stream)>>>(states, B, mask, pawn);
-        else if (lanes == 8)
-            legal_mask_kernel<8><<<blocks_for(B, kLegalWarps * 4), kLegalWarps * 32, 0, S(stream)>>>(states, B, mask, pawn);
-        else
-            legal_mask_kernel<2><<<blocks_for(B, kLegalWarps * 16), kLegalWarps * 32, 0, S(stream)>>>(states, B, mask, pawn);
-        return aq_check_launch("aq_legal_mask");
+            return aq_launch("aq_legal_mask", legal_mask_kernel<32>, blocks_for(B, kLegalWarps * 1), kLegalWarps * 32, 0, S(stream), false,
+                             states, B, mask, pawn);
+        if (lanes == 8)
+            return aq_launch("aq_legal_mask", legal_mask_kernel<8>, blocks_for(B, kLegalWarps * 4), kLegalWarps * 32, 0, S(stream), false,
+                             states, B, mask, pawn);
+        return aq_launch("aq_legal_mask", legal_mask_kernel<2>, blocks_for(B, kLegalWarps * 16), kLegalWarps * 32, 0, S(stream), false,
+                         states, B, mask, pawn);
     }
     // any workspace >= 4 KB + 256 B works (a state whose searches do not fit the list runs them itself); aq_legal_mask_ws_bytes(B)
     // is the size at which that practically never happens
@@ -442,17 +453,14 @@ extern "C" int aq_legal_mask_ws(const AqState *states, int64_t B, uint32_t *mask
         const int64_t n = B - lo < kLegalChunk ? B - lo : kLegalChunk;
         cudaError_t e = cudaMemsetAsync(counter, 0, 2 * sizeof(unsigned), S(stream));
         if (e != cudaSuccess) return aq_set_error((int)e, "aq_legal_mask(memset)");
-        legal_prepare_kernel<<<blocks_for(n, kLegalWarps * 16), kLegalWarps * 32, 0, S(stream)>>>(states + lo, n, mask + 8 * lo, pawn + 8 * lo,
-                                                                                                     tasks, cap, counter);
-        const int rc0 = aq_check_launch("aq_legal_mask(prepare)");
-        if (rc0) return rc0;
+        int rc = aq_launch("aq_legal_mask(prepare)", legal_prepare_kernel, blocks_for(n, kLegalWarps * 16), kLegalWarps * 32, 0, S(stream),
+                           false, states + lo, n, mask + 8 * lo, pawn + 8 * lo, tasks, cap, counter);
+        if (rc) return rc;
         // persistent warps fed through the cursor: enough of them for the expected number of searches (2-4 per state), at most 8 CTAs
         // of 128 threads per SM
         const unsigned grid = (unsigned)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (3 * n + 127) / 128));
-        e = aq_launch_pdl(legal_search_kernel, dim3(grid), dim3(128), 0, S(stream), states + lo, (const uint32_t *)tasks, (const unsigned *)counter,
-                          counter + 1, cap, mask + 8 * lo);
-        if (e != cudaSuccess) return aq_set_error((int)e, "aq_legal_mask(search launch)");
-        const int rc = aq_check_launch("aq_legal_mask");
+        rc = aq_launch("aq_legal_mask", legal_search_kernel, grid, 128, 0, S(stream), true, states + lo, (const uint32_t *)tasks,
+                       (const unsigned *)counter, counter + 1, cap, mask + 8 * lo);
         if (rc) return rc;
     }
     return 0;
@@ -467,24 +475,22 @@ extern "C" int aq_legal_actions_list(const uint32_t *mask, const uint8_t *pawn, 
                                      int16_t *n_actions, void *stream) {
     if (B < 0 || (B > 0 && (!mask || !pawn || !actions))) return aq_set_error(AQ_ERR_ARG, "aq_legal_actions_list");
     if (B == 0) return 0;
-    legal_list_kernel<<<blocks_for(B, 8), 256, 0, S(stream)>>>(mask, pawn, B, actions, n_actions);
-    return aq_check_launch("aq_legal_actions_list");
+    return aq_launch("aq_legal_actions_list", legal_list_kernel, blocks_for(B, 8), 256, 0, S(stream), false, mask, pawn, B, actions, n_actions);
 }
 
 extern "C" int aq_state_next(const AqState *states, const int16_t *actions, int64_t B, AqState *out, uint8_t *terminal,
                              void *stream) {
     if (B < 0 || (B > 0 && (!states || !actions || !out))) return aq_set_error(AQ_ERR_ARG, "aq_state_next");
     if (B == 0) return 0;
-    state_next_kernel<<<blocks_for(B, 256), 256, 0, S(stream)>>>(states, actions, B, out, terminal);
-    return aq_check_launch("aq_state_next");
+    return aq_launch("aq_state_next", state_next_kernel, blocks_for(B, 256), 256, 0, S(stream), false, states, actions, B, out, terminal);
 }
 
 extern "C" int aq_build_graph(const AqState *states, int64_t B, uint8_t *open_mask, float *dinv, float *x,
                               int32_t *edge_count, void *stream) {
     if (B < 0 || (B > 0 && !states)) return aq_set_error(AQ_ERR_ARG, "aq_build_graph");
     if (B == 0) return 0;
-    build_graph_kernel<<<blocks_for(B, 8), 256, 0, S(stream)>>>(states, B, open_mask, dinv, x, edge_count);
-    return aq_check_launch("aq_build_graph");
+    return aq_launch("aq_build_graph", build_graph_kernel, blocks_for(B, 8), 256, 0, S(stream), false, states, B, open_mask, dinv, x,
+                     edge_count);
 }
 
 extern "C" int aq_build_edge_index(const uint8_t *open_mask, const int64_t *edge_offset, int64_t B, int64_t *src,
@@ -492,8 +498,8 @@ extern "C" int aq_build_edge_index(const uint8_t *open_mask, const int64_t *edge
     if (B < 0 || (B > 0 && (!open_mask || !edge_offset || !src || !dst)))
         return aq_set_error(AQ_ERR_ARG, "aq_build_edge_index");
     if (B == 0) return 0;
-    build_edge_index_kernel<<<blocks_for(B, 8), 256, 0, S(stream)>>>(open_mask, edge_offset, B, src, dst);
-    return aq_check_launch("aq_build_edge_index");
+    return aq_launch("aq_build_edge_index", build_edge_index_kernel, blocks_for(B, 8), 256, 0, S(stream), false, open_mask, edge_offset, B,
+                     src, dst);
 }
 
 extern "C" int aq_edges_to_open_mask(const int64_t *src, const int64_t *dst, int64_t E, int64_t B, uint8_t *open_mask,
@@ -507,25 +513,25 @@ extern "C" int aq_edges_to_open_mask(const int64_t *src, const int64_t *dst, int
     e = cudaMemsetAsync(bad, 0, sizeof(int32_t), S(stream));
     if (e != cudaSuccess) return aq_set_error((int)e, "aq_edges_to_open_mask");
     if (E == 0) return 0;
-    edges_to_open_mask_kernel<<<blocks_for(E, 256), 256, 0, S(stream)>>>(src, dst, E, B, reinterpret_cast<unsigned *>(open_mask), bad);
-    const int rc = aq_check_launch("aq_edges_to_open_mask");
+    const int rc = aq_launch("aq_edges_to_open_mask", edges_to_open_mask_kernel, blocks_for(E, 256), 256, 0, S(stream), false, src, dst, E, B,
+                             reinterpret_cast<unsigned *>(open_mask), bad);
     if (rc) return rc;
-    open_mask_symmetry_kernel<<<blocks_for(B * AQ_SQUARES, 256), 256, 0, S(stream)>>>(open_mask, B, bad);
-    return aq_check_launch("aq_edges_to_open_mask(symmetry)");
+    return aq_launch("aq_edges_to_open_mask(symmetry)", open_mask_symmetry_kernel, blocks_for(B * AQ_SQUARES, 256), 256, 0, S(stream), false,
+                     open_mask, B, bad);
 }
 
 extern "C" int aq_shortest_paths(const AqState *states, int64_t B, int16_t *dist, double *heuristic, int32_t *leaf48,
                                  void *stream) {
     if (B < 0 || (B > 0 && (!states || (!dist && !heuristic && !leaf48)))) return aq_set_error(AQ_ERR_ARG, "aq_shortest_paths");
     if (B == 0) return 0;
-    shortest_paths_kernel<<<blocks_for(B, 128), 128, 0, S(stream)>>>(states, B, dist, heuristic, leaf48);
-    return aq_check_launch("aq_shortest_paths");
+    return aq_launch("aq_shortest_paths", shortest_paths_kernel, blocks_for(B, 128), 128, 0, S(stream), false, states, B, dist, heuristic,
+                     leaf48);
 }
 
 extern "C" int aq_negamax_backup(const int32_t *child_value, const int64_t *child_offset, int64_t P, const int32_t *fixed,
                                  int32_t *value, int32_t *best, void *stream) {
     if (P < 0 || (P > 0 && (!child_offset || !value))) return aq_set_error(AQ_ERR_ARG, "aq_negamax_backup");
     if (P == 0) return 0;
-    negamax_backup_kernel<<<blocks_for(P, 8), 256, 0, S(stream)>>>(child_value, child_offset, P, fixed, value, best);
-    return aq_check_launch("aq_negamax_backup");
+    return aq_launch("aq_negamax_backup", negamax_backup_kernel, blocks_for(P, 8), 256, 0, S(stream), false, child_value, child_offset, P,
+                     fixed, value, best);
 }

@@ -269,17 +269,11 @@ extern "C" int aq_comm_set_step(void *comm, int64_t step, float beta1, float bet
 int aq_dp_adam_launch(void *comm, const float *grads_in, const float *partial, int gcn_slots, int head_slots, float *params, float *exp_avg,
                       float *exp_avg_sq, float *grads_out, float lr, float beta1, float beta2, float eps, bool pdl, cudaStream_t st) {
     AqComm *c = reinterpret_cast<AqComm *>(comm);
-    cudaError_t e;
-    if (partial) {
-        if (pdl) e = aq_launch_pdl(dp_adam_kernel<true>, dim3(kChunks), dim3(kDpThreads), 0, st, c->p, grads_in, partial, gcn_slots, head_slots, params,
-                                   exp_avg, exp_avg_sq, grads_out, lr, beta1, beta2, eps);
-        else { dp_adam_kernel<true><<<kChunks, kDpThreads, 0, st>>>(c->p, grads_in, partial, gcn_slots, head_slots, params, exp_avg, exp_avg_sq, grads_out, lr, beta1, beta2, eps); e = cudaSuccess; }
-    } else {
-        dp_adam_kernel<false><<<kChunks, kDpThreads, 0, st>>>(c->p, grads_in, partial, gcn_slots, head_slots, params, exp_avg, exp_avg_sq, grads_out, lr, beta1, beta2, eps);
-        e = cudaSuccess;
-    }
-    if (e != cudaSuccess) return aq_set_error((int)e, "dp_adam_kernel(launch)");
-    return aq_check_launch("dp_adam_kernel");
+    if (partial)
+        return aq_launch("dp_adam_kernel", dp_adam_kernel<true>, kChunks, kDpThreads, 0, st, pdl, c->p, grads_in, partial, gcn_slots, head_slots,
+                         params, exp_avg, exp_avg_sq, grads_out, lr, beta1, beta2, eps);
+    return aq_launch("dp_adam_kernel", dp_adam_kernel<false>, kChunks, kDpThreads, 0, st, pdl, c->p, grads_in, partial, gcn_slots, head_slots,
+                     params, exp_avg, exp_avg_sq, grads_out, lr, beta1, beta2, eps);
 }
 
 // All-reduce (sum over the ranks of `comm`) of a flat gradient + Adam step, one kernel.  grads: this rank's gradient (n = 64,082

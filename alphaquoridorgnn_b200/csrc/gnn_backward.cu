@@ -69,7 +69,7 @@ heads_backward_kernel(const float *__restrict__ params, const float *saved,   //
 #pragma unroll 8
     for (int i = tid; i < kHH * kH; i += (int)blockDim.x) sm.wv0[i] = __ldg(params + kOffWV0 + i);
     if (tid < kHH) sm.wv2[tid] = __ldg(params + kOffWV2 + tid);
-    aq_pdl_wait();     // launched with aq_launch_pdl: the weight fill above overlaps the tail of the loss kernel; dpolicy / dvalue are read below
+    aq_pdl_wait();     // launched programmatically: the weight fill above overlaps the tail of the loss kernel; dpolicy / dvalue are read below
     __syncthreads();
     const SavedLayout L{B};
     const BwdWs W{B};
@@ -587,11 +587,8 @@ static int backward_to_partials(const float *params, const float *saved, const f
     const SavedLayout L{B};
     const BwdWs W{B};
     const bool fused_loss = ptarget != nullptr;
-    cudaError_t e;
-    e = cudaFuncSetAttribute(gcn_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(GcnBwdSmem));
-    if (e != cudaSuccess) return aq_set_error((int)e, "gcn_backward smem");
     if (fused_loss && loss) {
-        e = cudaMemsetAsync(loss, 0, 2 * sizeof(float), st);
+        const cudaError_t e = cudaMemsetAsync(loss, 0, 2 * sizeof(float), st);
         if (e != cudaSuccess) return aq_set_error((int)e, "aq_loss_backward(memset)");
     }
     const int hb_threads = B <= 1184 ? 256 : kHbThreads;  // 148 CTAs x 8 boards cover 1,184 boards in one pass
@@ -601,31 +598,26 @@ static int backward_to_partials(const float *params, const float *saved, const f
     const dim3 hgrid((unsigned)(hb < kSlots ? hb : kSlots));
     const float inv_total = 1.0f / (float)(B_total > 0 ? B_total : B);
     // the backward kernels are chained by programmatic dependent launches: each reads only the parameters before its aq_pdl_wait()
-    auto launch_hb = [&](auto kernel, size_t smem) -> cudaError_t {
-        cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (err != cudaSuccess) return err;
-        return aq_launch_pdl(kernel, hgrid, dim3(hb_threads), smem, st, params, saved, dpolicy, dvalue, ptarget, vtarget, inv_total, loss, B,
-                             workspace);
+    auto launch_hb = [&](auto kernel, size_t smem) {
+        return aq_launch("heads_backward_kernel", kernel, hgrid, hb_threads, smem, st, true, params, saved, dpolicy, dvalue, ptarget, vtarget,
+                         inv_total, loss, B, workspace);
     };
+    int rc;
     if (fused_loss) {
-        if (nb == 4) e = launch_hb(heads_backward_kernel<true, 4>, sizeof(HeadBwdSmem<4>));
-        else if (nb == 2) e = launch_hb(heads_backward_kernel<true, 2>, sizeof(HeadBwdSmem<2>));
-        else e = launch_hb(heads_backward_kernel<true, 1>, sizeof(HeadBwdSmem<1>));
+        if (nb == 4) rc = launch_hb(heads_backward_kernel<true, 4>, sizeof(HeadBwdSmem<4>));
+        else if (nb == 2) rc = launch_hb(heads_backward_kernel<true, 2>, sizeof(HeadBwdSmem<2>));
+        else rc = launch_hb(heads_backward_kernel<true, 1>, sizeof(HeadBwdSmem<1>));
     } else {
-        if (nb == 4) e = launch_hb(heads_backward_kernel<false, 4>, sizeof(HeadBwdSmem<4>));
-        else if (nb == 2) e = launch_hb(heads_backward_kernel<false, 2>, sizeof(HeadBwdSmem<2>));
-        else e = launch_hb(heads_backward_kernel<false, 1>, sizeof(HeadBwdSmem<1>));
+        if (nb == 4) rc = launch_hb(heads_backward_kernel<false, 4>, sizeof(HeadBwdSmem<4>));
+        else if (nb == 2) rc = launch_hb(heads_backward_kernel<false, 2>, sizeof(HeadBwdSmem<2>));
+        else rc = launch_hb(heads_backward_kernel<false, 1>, sizeof(HeadBwdSmem<1>));
     }
-    if (e != cudaSuccess) return aq_set_error((int)e, "heads_backward_kernel(launch)");
-    int rc = aq_check_launch("heads_backward_kernel");
     if (rc) return rc;
-    if (precision == 1) {  // tensor-core trunk backward: fills the GCN ranges of every partial slot itself
+    if (precision == 1)  // tensor-core trunk backward: fills the GCN ranges of every partial slot itself
         rc = aq_gcn_backward_tc2(params, const_cast<float *>(saved), workspace + W.dg(), B, workspace + W.partial(), st);
-        if (rc) return rc;
-    } else {
-        gcn_backward_kernel<<<kSlots, kGcnThreads, sizeof(GcnBwdSmem), st>>>(params, saved, B, workspace);
-        if ((rc = aq_check_launch("gcn_backward_kernel"))) return rc;
-    }
+    else
+        rc = aq_launch("gcn_backward_kernel", gcn_backward_kernel, kSlots, kGcnThreads, sizeof(GcnBwdSmem), st, false, params, saved, B, workspace);
+    if (rc) return rc;
 
     if (precision == 1)   // head weight gradients on the tensor cores (the trunk backward above filled the GCN ranges of the slots)
         return aq_heads_wgrad_tc(workspace + W.dhp(), workspace + W.dhv(), workspace + W.dz(), workspace + W.du(), saved + L.pooled(),
@@ -649,9 +641,8 @@ static int backward_to_partials(const float *params, const float *saved, const f
     add(workspace + W.dhv(), kHH, kHH, saved + L.pooled(), kH, kH, B, kOffWV0, kOffBV0);
     add(workspace + W.du(), 1, 1, saved + L.hv(), kHH, kHH, B, kOffWV2, kOffBV2);
     jobs.n = nj;
-    e = aq_launch_pdl(atb_jobs_kernel, dim3(precision != 1 ? kSlots : head_slots, kMaxMTiles, nj), dim3(256), 0, st, jobs, workspace + W.partial());
-    if (e != cudaSuccess) return aq_set_error((int)e, "atb_jobs_kernel(launch)");
-    return aq_check_launch("atb_jobs_kernel");
+    return aq_launch("atb_jobs_kernel", atb_jobs_kernel, dim3(precision != 1 ? kSlots : head_slots, kMaxMTiles, nj), 256, 0, st, true, jobs,
+                     workspace + W.partial());
 }
 
 extern "C" int aq_gnn_backward(const float *params, const float *saved, const float *dpolicy, const float *dvalue,
@@ -661,10 +652,8 @@ extern "C" int aq_gnn_backward(const float *params, const float *saved, const fl
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     int rc = backward_to_partials(params, saved, dpolicy, dvalue, nullptr, nullptr, B, B, nullptr, workspace, precision, st);
     if (rc) return rc;
-    cudaError_t e = aq_launch_pdl(reduce_partials_kernel, dim3((kNumParams / 2 + kRedPairs - 1) / kRedPairs), dim3(kRedPairs * 4), 0, st,
-                                  (const float *)(workspace + BwdWs{B}.partial()), grads, head_slot_count(B, precision));
-    if (e != cudaSuccess) return aq_set_error((int)e, "reduce_partials_kernel(launch)");
-    return aq_check_launch("reduce_partials_kernel");
+    return aq_launch("reduce_partials_kernel", reduce_partials_kernel, (kNumParams / 2 + kRedPairs - 1) / kRedPairs, kRedPairs * 4, 0, st, true,
+                     (const float *)(workspace + BwdWs{B}.partial()), grads, head_slot_count(B, precision));
 }
 
 // One training step behind the forward pass, as the reference's `loss = ...; optimizer.zero_grad(); loss.backward(); optimizer.step()`
@@ -694,9 +683,8 @@ extern "C" int aq_loss_grad(const float *policy, const float *value, const float
         if (e != cudaSuccess) return aq_set_error((int)e, "aq_loss_grad(memset)");
     }
     const int64_t nb = (B + 7) / 8;
-    loss_grad_kernel<<<(unsigned)(nb < 1184 ? nb : 1184), 256, 0, st>>>(policy, value, policy_target, value_target, B,
-                                                                       1.0f / (float)B_total, loss, dpolicy, dvalue);
-    return aq_check_launch("loss_grad_kernel");
+    return aq_launch("loss_grad_kernel", loss_grad_kernel, (unsigned)(nb < 1184 ? nb : 1184), 256, 0, st, false, policy, value, policy_target,
+                     value_target, B, 1.0f / (float)B_total, loss, dpolicy, dvalue);
 }
 
 extern "C" int aq_adam_step(float *params, const float *grads, float *exp_avg, float *exp_avg_sq, int64_t n,
@@ -707,7 +695,6 @@ extern "C" int aq_adam_step(float *params, const float *grads, float *exp_avg, f
     const double bc2 = 1.0 - pow((double)beta2, (double)step);
     const float step_size = (float)((double)lr / bc1);
     const float bc2_sqrt = (float)sqrt(bc2);
-    adam_kernel<<<(unsigned)((n + 255) / 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-        params, grads, exp_avg, exp_avg_sq, n, step_size, bc2_sqrt, beta1, beta2, eps, grad_scale);
-    return aq_check_launch("adam_kernel");
+    return aq_launch("adam_kernel", adam_kernel, (unsigned)((n + 255) / 256), 256, 0, reinterpret_cast<cudaStream_t>(stream), false, params,
+                     grads, exp_avg, exp_avg_sq, n, step_size, bc2_sqrt, beta1, beta2, eps, grad_scale);
 }

@@ -265,23 +265,6 @@ heads_forward_kernel(const float *__restrict__ params, const float *__restrict__
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
-static int g_num_sms = 0;
-static int num_sms() {
-    if (g_num_sms == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev);
-        if (g_num_sms <= 0) g_num_sms = 148;
-    }
-    return g_num_sms;
-}
-
-template <typename K>
-static int set_smem(K kernel, size_t bytes) {
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    return e == cudaSuccess ? 0 : (int)e;
-}
-
 int aq_gcn_forward_tc2(const float *params, const void *prepared, const AqState *states, int64_t B, float *pooled, float *saved,
                        uint32_t *mask, uint8_t *pawn, bool after_legal, cudaStream_t st);  // gnn_tc2.cu
 int aq_heads_forward_tc(const float *params, const void *prepared, const float *pooled, int64_t B, float *policy, float *value,
@@ -294,16 +277,12 @@ static int launch_trunk(const float *params, const void *prepared, const AqState
         if (!states) return aq_set_error(AQ_ERR_UNSUPPORTED, "aq_gnn_forward(bf16 path needs packed states)");
         return aq_gcn_forward_tc2(params, prepared, states, B, pooled, saved, saved ? nullptr : legal_out, pawn_out, saved ? false : after_legal, st);
     }
-    const unsigned grid = (unsigned)(B < num_sms() ? B : num_sms());
-    int rc;
-    if (saved) {
-        if ((rc = set_smem(gcn_forward_fp32_kernel<true>, sizeof(GcnSmem)))) return aq_set_error(rc, "gcn_forward smem");
-        gcn_forward_fp32_kernel<true><<<grid, kGcnThreads, sizeof(GcnSmem), st>>>(params, states, x, open_mask, B, pooled, saved);
-    } else {
-        if ((rc = set_smem(gcn_forward_fp32_kernel<false>, sizeof(GcnSmem)))) return aq_set_error(rc, "gcn_forward smem");
-        gcn_forward_fp32_kernel<false><<<grid, kGcnThreads, sizeof(GcnSmem), st>>>(params, states, x, open_mask, B, pooled, nullptr);
-    }
-    return aq_check_launch("gcn_forward_fp32_kernel");
+    const unsigned grid = (unsigned)(B < aq_num_sms() ? B : aq_num_sms());
+    if (saved)
+        return aq_launch("gcn_forward_fp32_kernel", gcn_forward_fp32_kernel<true>, grid, kGcnThreads, sizeof(GcnSmem), st, false, params, states,
+                         x, open_mask, B, pooled, saved);
+    return aq_launch("gcn_forward_fp32_kernel", gcn_forward_fp32_kernel<false>, grid, kGcnThreads, sizeof(GcnSmem), st, false, params, states,
+                     x, open_mask, B, pooled, (float *)nullptr);
 }
 
 static int launch_heads(const float *params, const void *prepared, const float *pooled, int64_t B, float *policy,
@@ -313,19 +292,15 @@ static int launch_heads(const float *params, const void *prepared, const float *
     if (precision == 1 && (!saved || !legal_mask))
         return aq_heads_forward_tc(params, prepared, pooled, B, policy, value, legal_mask, saved, after_trunk, st);
     const int64_t hb = (B + 7) / 8;
-    const unsigned hgrid = (unsigned)(hb < num_sms() ? hb : num_sms());
-    int rc;
-    if (legal_mask) {
-        if ((rc = set_smem(heads_forward_kernel<false, true>, sizeof(HeadSmem)))) return aq_set_error(rc, "heads smem");
-        heads_forward_kernel<false, true><<<hgrid, kHeadThreads, sizeof(HeadSmem), st>>>(params, pooled, B, policy, value, legal_mask, nullptr);
-    } else if (saved) {
-        if ((rc = set_smem(heads_forward_kernel<true, false>, sizeof(HeadSmem)))) return aq_set_error(rc, "heads smem");
-        heads_forward_kernel<true, false><<<hgrid, kHeadThreads, sizeof(HeadSmem), st>>>(params, pooled, B, policy, value, nullptr, saved);
-    } else {
-        if ((rc = set_smem(heads_forward_kernel<false, false>, sizeof(HeadSmem)))) return aq_set_error(rc, "heads smem");
-        heads_forward_kernel<false, false><<<hgrid, kHeadThreads, sizeof(HeadSmem), st>>>(params, pooled, B, policy, value, nullptr, nullptr);
-    }
-    return aq_check_launch("heads_forward_kernel");
+    const unsigned hgrid = (unsigned)(hb < aq_num_sms() ? hb : aq_num_sms());
+    if (legal_mask)
+        return aq_launch("heads_forward_kernel", heads_forward_kernel<false, true>, hgrid, kHeadThreads, sizeof(HeadSmem), st, false, params,
+                         pooled, B, policy, value, legal_mask, (float *)nullptr);
+    if (saved)
+        return aq_launch("heads_forward_kernel", heads_forward_kernel<true, false>, hgrid, kHeadThreads, sizeof(HeadSmem), st, false, params,
+                         pooled, B, policy, value, (const uint32_t *)nullptr, saved);
+    return aq_launch("heads_forward_kernel", heads_forward_kernel<false, false>, hgrid, kHeadThreads, sizeof(HeadSmem), st, false, params,
+                     pooled, B, policy, value, (const uint32_t *)nullptr, (float *)nullptr);
 }
 
 extern "C" int aq_gcn_trunk_forward(const float *params, const void *prepared, const AqState *states, int64_t B,
@@ -709,17 +684,14 @@ compact_priors_kernel(const float *priors, const uint32_t *mask, const uint8_t *
 
 static int compact_priors_impl(const float *priors, const uint32_t *mask, const uint8_t *pawn, int64_t B, int32_t *offsets, void *compact,
                                int wire, cudaStream_t st) {
-    cudaError_t e = aq_launch_pdl(legal_count_scan_kernel, dim3(1), dim3(1024), 0, st, mask, B, offsets);
-    if (e != cudaSuccess) return aq_set_error((int)e, "aq_compact_priors(scan launch)");
-    int rc = aq_check_launch("aq_compact_priors(scan)");
+    const int rc = aq_launch("aq_compact_priors(scan)", legal_count_scan_kernel, 1, 1024, 0, st, true, mask, B, offsets);
     if (rc || B == 0) return rc;
-    const dim3 grid((unsigned)((B + 7) / 8));
+    const unsigned grid = (unsigned)((B + 7) / 8);
     if (wire == AQ_WIRE_F16)
-        e = aq_launch_pdl(compact_priors_kernel<__half>, grid, dim3(256), 0, st, priors, mask, pawn, (const int32_t *)offsets, B, reinterpret_cast<__half *>(compact));
-    else
-        e = aq_launch_pdl(compact_priors_kernel<float>, grid, dim3(256), 0, st, priors, mask, pawn, (const int32_t *)offsets, B, reinterpret_cast<float *>(compact));
-    if (e != cudaSuccess) return aq_set_error((int)e, "aq_compact_priors(launch)");
-    return aq_check_launch("aq_compact_priors");
+        return aq_launch("aq_compact_priors", compact_priors_kernel<__half>, grid, 256, 0, st, true, priors, mask, pawn, (const int32_t *)offsets,
+                         B, reinterpret_cast<__half *>(compact));
+    return aq_launch("aq_compact_priors", compact_priors_kernel<float>, grid, 256, 0, st, true, priors, mask, pawn, (const int32_t *)offsets, B,
+                     reinterpret_cast<float *>(compact));
 }
 
 extern "C" int aq_compact_priors(const float *priors, const uint32_t *mask, const uint8_t *pawn, int64_t B, int32_t *offsets,

@@ -65,7 +65,6 @@ extern "C" int64_t aq_prepared_bytes(void) { return kPrepBytes; }
 extern "C" int aq_prepare_inference(const float *params, void *prepared, void *stream) {
     if (!params || !prepared) return aq_set_error(AQ_ERR_ARG, "aq_prepare_inference");
     const int chunks = 4096 + 128 + 2048 + 224 * 8;
-    prepare_inference_kernel<<<(chunks + 255) / 256, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-        params, reinterpret_cast<unsigned char *>(prepared));
-    return aq_check_launch("prepare_inference_kernel");
+    return aq_launch("prepare_inference_kernel", prepare_inference_kernel, (chunks + 255) / 256, 256, 0, reinterpret_cast<cudaStream_t>(stream),
+                     false, params, reinterpret_cast<unsigned char *>(prepared));
 }

@@ -755,40 +755,17 @@ gcn_forward_tc2_kernel(const float *__restrict__ params, const unsigned char *__
 // the mask.
 int aq_gcn_forward_tc2(const float *params, const void *prepared, const AqState *states, int64_t B, float *pooled, float *saved,
                        uint32_t *mask, uint8_t *pawn, bool after_legal, cudaStream_t st) {
-    static int sms = 0;
     const uint32_t wait_ns = 0;  // suspend-time hint of the mbarrier waits (0 = spin; measured best)
-    if (sms == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (sms <= 0) sms = 148;
-    }
     const size_t smem = sizeof(Tc2Smem) + 1024;
     const int64_t want = (B + kG - 1) / kG;
-    const unsigned grid = (unsigned)(want < sms ? want : sms);
+    const unsigned grid = (unsigned)(want < aq_num_sms() ? want : aq_num_sms());
     const unsigned char *prep = reinterpret_cast<const unsigned char *>(prepared);
-    cudaError_t e;
-    if (saved) {
-        e = cudaFuncSetAttribute(gcn_forward_tc2_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return aq_set_error((int)e, "gcn_forward_tc2 smem");
-        gcn_forward_tc2_kernel<true, false><<<grid, kTrunkThreads, smem, st>>>(params, prep, states, B, pooled, saved, wait_ns, nullptr, nullptr);
-    } else if (mask) {
-        const size_t smem_l = smem + sizeof(Tc2Legal);
-        e = cudaFuncSetAttribute(gcn_forward_tc2_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_l);
-        if (e != cudaSuccess) return aq_set_error((int)e, "gcn_forward_tc2 smem");
-        gcn_forward_tc2_kernel<false, true><<<grid, kTrunkThreads + kLegalThreads, smem_l, st>>>(params, prep, states, B, pooled, nullptr, wait_ns,
-                                                                                                 mask, pawn);
-    } else {
-        e = cudaFuncSetAttribute(gcn_forward_tc2_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return aq_set_error((int)e, "gcn_forward_tc2 smem");
-        if (after_legal) {
-            e = aq_launch_pdl(gcn_forward_tc2_kernel<false, false>, dim3(grid), dim3(kTrunkThreads), smem, st, params, prep, states, B, pooled,
-                              (float *)nullptr, wait_ns, (uint32_t *)nullptr, (uint8_t *)nullptr);
-            if (e != cudaSuccess) return aq_set_error((int)e, "gcn_forward_tc2_kernel(launch)");
-        } else {
-            gcn_forward_tc2_kernel<false, false><<<grid, kTrunkThreads, smem, st>>>(params, prep, states, B, pooled, nullptr, wait_ns, nullptr,
-                                                                                    nullptr);
-        }
-    }
-    return aq_check_launch("gcn_forward_tc2_kernel");
+    if (saved)
+        return aq_launch("gcn_forward_tc2_kernel", gcn_forward_tc2_kernel<true, false>, grid, kTrunkThreads, smem, st, false, params, prep, states,
+                         B, pooled, saved, wait_ns, (uint32_t *)nullptr, (uint8_t *)nullptr);
+    if (mask)
+        return aq_launch("gcn_forward_tc2_kernel", gcn_forward_tc2_kernel<false, true>, grid, kTrunkThreads + kLegalThreads, smem + sizeof(Tc2Legal),
+                         st, false, params, prep, states, B, pooled, (float *)nullptr, wait_ns, mask, pawn);
+    return aq_launch("gcn_forward_tc2_kernel", gcn_forward_tc2_kernel<false, false>, grid, kTrunkThreads, smem, st, after_legal, params, prep,
+                     states, B, pooled, (float *)nullptr, wait_ns, (uint32_t *)nullptr, (uint8_t *)nullptr);
 }

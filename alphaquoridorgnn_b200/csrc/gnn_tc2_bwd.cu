@@ -287,7 +287,7 @@ gcn_backward_tc2_kernel(const float *__restrict__ params, float *__restrict__ sa
     };
 
     int buf = 0;
-    // launched with aq_launch_pdl: everything above (W^T tiles, zeroed adjacency, barriers, tensor-memory allocation) read only the parameters
+    // launched programmatically: everything above (W^T tiles, zeroed adjacency, barriers, tensor-memory allocation) read only the parameters
     // and overlapped the tail of the heads backward; the saved activations and dg are read from here on
     aq_pdl_wait();
     prefetch_board(blockIdx.x, 0);
@@ -478,10 +478,6 @@ gcn_backward_tc2_kernel(const float *__restrict__ params, float *__restrict__ sa
 
 // partial: [kSlots = 148][64082] floats; this kernel fills the GCN ranges (W1,B1,W2,B2,W3,B3) of every slot
 int aq_gcn_backward_tc2(const float *params, float *saved, const float *dg, int64_t B, float *partial, cudaStream_t st) {
-    const size_t smem = sizeof(Bwd2Smem) + 1024;
-    cudaError_t e = cudaFuncSetAttribute(gcn_backward_tc2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return aq_set_error((int)e, "gcn_backward_tc2 smem");
-    e = aq_launch_pdl(gcn_backward_tc2_kernel, dim3(148), dim3(kBwdThreads), smem, st, params, saved, dg, B, partial);
-    if (e != cudaSuccess) return aq_set_error((int)e, "gcn_backward_tc2_kernel(launch)");
-    return aq_check_launch("gcn_backward_tc2_kernel");
+    return aq_launch("gcn_backward_tc2_kernel", gcn_backward_tc2_kernel, dim3(148), kBwdThreads, sizeof(Bwd2Smem) + 1024, st, true, params, saved,
+                     dg, B, partial);
 }

@@ -340,23 +340,6 @@ heads_forward_tc_kernel(const float *__restrict__ params, const unsigned char *_
 
 }  // namespace
 
-// launch with the programmatic-stream-serialization attribute: the grid may start while its predecessor in the stream is still
-// draining; the kernel orders itself behind the predecessor's results with griddepcontrol.wait
-template <typename Kernel, typename... Args>
-static cudaError_t launch_pdl(bool pdl, Kernel kernel, unsigned grid, size_t smem, cudaStream_t st, Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid, 1, 1);
-    cfg.blockDim = dim3(kHtThreads, 1, 1);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kernel, args...);
-}
-
 // pdl: the predecessor in the stream is the trunk kernel of the same forward pass (it triggers its dependents early and does not write the
 // parameters this kernel reads before its griddepcontrol.wait); standalone calls launch normally
 int aq_heads_forward_tc(const float *params, const void *prepared_v, const float *pooled, int64_t B, float *policy,
@@ -364,16 +347,9 @@ int aq_heads_forward_tc(const float *params, const void *prepared_v, const float
     const unsigned char *prepared = reinterpret_cast<const unsigned char *>(prepared_v);
     const size_t smem = sizeof(HtSmem) + 1024;
     const unsigned grid = (unsigned)((B + kTile - 1) / kTile);
-    cudaError_t e, rc_launch = cudaSuccess;
-    if (legal_mask) {
-        e = cudaFuncSetAttribute(heads_forward_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return aq_set_error((int)e, "heads_forward_tc smem");
-        rc_launch = launch_pdl(pdl, heads_forward_tc_kernel<true>, grid, smem, st, params, prepared, pooled, B, policy, value, legal_mask, saved);
-    } else {
-        e = cudaFuncSetAttribute(heads_forward_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return aq_set_error((int)e, "heads_forward_tc smem");
-        rc_launch = launch_pdl(pdl, heads_forward_tc_kernel<false>, grid, smem, st, params, prepared, pooled, B, policy, value, (const uint32_t *)nullptr, saved);
-    }
-    if (rc_launch != cudaSuccess) return aq_set_error((int)rc_launch, "heads_forward_tc_kernel(launch)");
-    return aq_check_launch("heads_forward_tc_kernel");
+    if (legal_mask)
+        return aq_launch("heads_forward_tc_kernel", heads_forward_tc_kernel<true>, grid, kHtThreads, smem, st, pdl, params, prepared, pooled, B,
+                         policy, value, legal_mask, saved);
+    return aq_launch("heads_forward_tc_kernel", heads_forward_tc_kernel<false>, grid, kHtThreads, smem, st, pdl, params, prepared, pooled, B,
+                     policy, value, (const uint32_t *)nullptr, saved);
 }

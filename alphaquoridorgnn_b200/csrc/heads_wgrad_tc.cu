@@ -322,10 +322,6 @@ int aq_heads_wgrad_tc(const float *dhp, const float *dhv, const float *dz, const
                       const float *hv, int64_t B, float *partial, cudaStream_t st) {
     const int slots = aq_heads_wgrad_tc_slots(B);
     if (slots <= 0) return 0;
-    const size_t smem = sizeof(WgSmem) + 1024;
-    cudaError_t e = cudaFuncSetAttribute(heads_wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return aq_set_error((int)e, "heads_wgrad_tc smem");
-    e = aq_launch_pdl(heads_wgrad_tc_kernel, dim3((unsigned)slots), dim3(kWgThreads), smem, st, dhp, dhv, dz, du, pooled, hp, hv, B, partial);
-    if (e != cudaSuccess) return aq_set_error((int)e, "heads_wgrad_tc_kernel(launch)");
-    return aq_check_launch("heads_wgrad_tc_kernel");
+    return aq_launch("heads_wgrad_tc_kernel", heads_wgrad_tc_kernel, (unsigned)slots, kWgThreads, sizeof(WgSmem) + 1024, st, true, dhp, dhv, dz,
+                     du, pooled, hp, hv, B, partial);
 }

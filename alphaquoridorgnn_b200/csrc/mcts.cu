@@ -521,9 +521,8 @@ static inline MctsCold *cold_of(void *ws, int64_t G, int64_t max_nodes) {
 
 extern "C" int aq_mcts_reset(void *ws, const AqState *roots, int64_t G, int64_t max_nodes, void *stream) {
     if (G <= 0 || max_nodes < 1 || !ws || !roots) return aq_set_error(AQ_ERR_ARG, "aq_mcts_reset");
-    mcts_reset_kernel<<<(unsigned)((G + 127) / 128), 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-        games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), roots, G, max_nodes);
-    return aq_check_launch("aq_mcts_reset");
+    return aq_launch("aq_mcts_reset", mcts_reset_kernel, (unsigned)((G + 127) / 128), 128, 0, reinterpret_cast<cudaStream_t>(stream), false,
+                     games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), roots, G, max_nodes);
 }
 
 extern "C" int aq_mcts_advance(const void *src_ws, int64_t G_src, void *dst_ws, int64_t G_dst, int64_t max_nodes, const AqState *roots,
@@ -539,34 +538,31 @@ extern "C" int aq_mcts_advance(const void *src_ws, int64_t G_src, void *dst_ws, 
     cudaError_t e = cudaMemsetAsync(status, 0, sizeof(int32_t), st);
     if (e != cudaSuccess) return aq_set_error((int)e, "aq_mcts_advance");
     void *src = const_cast<void *>(src_ws);
-    mcts_advance_kernel<<<(unsigned)((G_dst + 3) / 4), 128, 0, st>>>(games_of(src), hot_of(src, G_src), cold_of(src, G_src, max_nodes), G_src,
-                                                                    games_of(dst_ws), hot_of(dst_ws, G_dst), cold_of(dst_ws, G_dst, max_nodes), G_dst,
-                                                                    max_nodes, roots, src_game, path, path_len, reserve_nodes, kept, status);
-    return aq_check_launch("aq_mcts_advance");
+    return aq_launch("aq_mcts_advance", mcts_advance_kernel, (unsigned)((G_dst + 3) / 4), 128, 0, st, false, games_of(src), hot_of(src, G_src),
+                     cold_of(src, G_src, max_nodes), G_src, games_of(dst_ws), hot_of(dst_ws, G_dst), cold_of(dst_ws, G_dst, max_nodes), G_dst,
+                     max_nodes, roots, src_game, path, path_len, reserve_nodes, kept, status);
 }
 
 extern "C" int aq_mcts_select(void *ws, int64_t G, int64_t max_nodes, float c_puct, AqState *leaf_states,
                               int32_t *leaf_kind, void *stream) {
     if (G <= 0 || !ws || !leaf_states || !leaf_kind) return aq_set_error(AQ_ERR_ARG, "aq_mcts_select");
-    mcts_select_kernel<<<(unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-        games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, c_puct, leaf_states, leaf_kind);
-    return aq_check_launch("aq_mcts_select");
+    return aq_launch("aq_mcts_select", mcts_select_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream), false,
+                     games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, c_puct, leaf_states, leaf_kind);
 }
 
 extern "C" int aq_mcts_expand_backup(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values,
                                      const uint32_t *mask, const uint8_t *pawn, void *stream) {
     if (G <= 0 || !ws || !priors || !values || !mask || !pawn) return aq_set_error(AQ_ERR_ARG, "aq_mcts_expand_backup");
-    mcts_expand_backup_kernel<<<(unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-        games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, priors, values, mask, pawn);
-    return aq_check_launch("aq_mcts_expand_backup");
+    return aq_launch("aq_mcts_expand_backup", mcts_expand_backup_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream),
+                     false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, priors, values, mask, pawn);
 }
 
 extern "C" int aq_mcts_expand_select(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values, const uint32_t *mask,
                                      const uint8_t *pawn, float c_puct, AqState *leaf_states, int32_t *leaf_kind, void *stream) {
     if (G <= 0 || !ws || !priors || !values || !mask || !pawn || !leaf_states || !leaf_kind) return aq_set_error(AQ_ERR_ARG, "aq_mcts_expand_select");
-    mcts_expand_select_kernel<<<(unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-        games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, priors, values, mask, pawn, c_puct, leaf_states, leaf_kind);
-    return aq_check_launch("aq_mcts_expand_select");
+    return aq_launch("aq_mcts_expand_select", mcts_expand_select_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream),
+                     false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, priors, values, mask, pawn, c_puct, leaf_states,
+                     leaf_kind);
 }
 
 extern "C" int aq_mcts_root_counts(void *ws, int64_t G, int64_t max_nodes, int32_t *counts, int16_t *actions,
@@ -577,9 +573,8 @@ extern "C" int aq_mcts_root_counts(void *ws, int64_t G, int64_t max_nodes, int32
         cudaError_t e = cudaMemsetAsync(overflow, 0, sizeof(int32_t), st);
         if (e != cudaSuccess) return aq_set_error((int)e, "aq_mcts_root_counts");
     }
-    mcts_root_counts_kernel<<<(unsigned)((G + 3) / 4), 128, 0, st>>>(games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, counts,
-                                                                     actions, n_children, overflow);
-    return aq_check_launch("aq_mcts_root_counts");
+    return aq_launch("aq_mcts_root_counts", mcts_root_counts_kernel, (unsigned)((G + 3) / 4), 128, 0, st, false, games_of(ws), hot_of(ws, G),
+                     cold_of(ws, G, max_nodes), G, max_nodes, counts, actions, n_children, overflow);
 }
 
 extern "C" int64_t aq_selfplay_ws_bytes(int64_t G) {
@@ -599,14 +594,14 @@ extern "C" int aq_selfplay_advance(const AqState *states, const int32_t *counts,
     const int greedy = temperature == 0.0;
     const double inv_t = greedy ? 1.0 : 1.0 / temperature;
     const unsigned grid = (unsigned)((G + 3) / 4);
+    int rc;
     if (policy_f64)
-        selfplay_move_kernel<double><<<grid, 128, 0, st>>>(states, counts, actions, n_children, game_id, G, inv_t, greedy, seed, ply,
-                                                          reinterpret_cast<double *>(policy), chosen, moved, term);
+        rc = aq_launch("aq_selfplay_advance(move)", selfplay_move_kernel<double>, grid, 128, 0, st, false, states, counts, actions, n_children,
+                       game_id, G, inv_t, greedy, seed, ply, reinterpret_cast<double *>(policy), chosen, moved, term);
     else
-        selfplay_move_kernel<float><<<grid, 128, 0, st>>>(states, counts, actions, n_children, game_id, G, inv_t, greedy, seed, ply,
-                                                         reinterpret_cast<float *>(policy), chosen, moved, term);
-    int rc = aq_check_launch("aq_selfplay_advance(move)");
+        rc = aq_launch("aq_selfplay_advance(move)", selfplay_move_kernel<float>, grid, 128, 0, st, false, states, counts, actions, n_children,
+                       game_id, G, inv_t, greedy, seed, ply, reinterpret_cast<float *>(policy), chosen, moved, term);
     if (rc) return rc;
-    selfplay_compact_kernel<<<1, 1024, 0, st>>>(moved, term, game_id, G, ply, next_states, next_game_id, final_flags, final_plies, alive_count);
-    return aq_check_launch("aq_selfplay_advance(compact)");
+    return aq_launch("aq_selfplay_advance(compact)", selfplay_compact_kernel, 1, 1024, 0, st, false, moved, term, game_id, G, ply, next_states,
+                     next_game_id, final_flags, final_plies, alive_count);
 }

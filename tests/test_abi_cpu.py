@@ -35,6 +35,18 @@ def test_sass_is_sm100a():
     assert "sm_100a" in out
 
 
+def test_every_kernel_launch_goes_through_aq_launch():
+    """aq_launch (csrc/aq_common.cuh) sets the shared-memory limit, chooses a programmatic launch and counts the launch
+    (aq_launch_count, bench.py's gpu_launches); a launch written any other way would go uncounted."""
+    csrc = os.path.join(ROOT, "alphaquoridorgnn_b200", "csrc")
+    for name in sorted(os.listdir(csrc)):
+        with open(os.path.join(csrc, name)) as f:
+            text = f.read()
+        assert "<<<" not in text, name
+        if name != "aq_common.cuh":
+            assert "cudaLaunchKernelEx" not in text and "cudaFuncSetAttribute" not in text, name
+
+
 def test_host_packing_matches_struct_layout(traj):
     rows, plies = traj["rows"][:5000], traj["plies"][:5000]
     packed = gl.pack_rows_host(rows, plies)
