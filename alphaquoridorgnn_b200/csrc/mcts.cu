@@ -6,8 +6,9 @@
 //   aq_mcts_expand_backup  create the children in legal_actions() order with their priors
 //                          (pv_mcts.py:53-56) and back the value up with alternating sign (:60-66)
 // The reference has no virtual loss, no Dirichlet noise and no tree reuse, so batching ACROSS games
-// leaves every game's search unchanged.  Tree reuse between moves (aq_mcts_advance, AlphaGo Zero) is an
-// opt-in addition the reference does not have; without it every search starts from aq_mcts_reset.
+// leaves every game's search unchanged.  Tree reuse between moves (aq_mcts_advance, AlphaGo Zero) and
+// Dirichlet noise on the root priors (aq_mcts_root_noise, AlphaZero) are opt-in additions the reference
+// does not have; without them every search starts from aq_mcts_reset with the network's priors.
 //
 // Arithmetic is kept as the reference computes it under NumPy >= 2 (requirements.txt pins
 // numpy~=2.0.2, NEP 50 promotion): w accumulates in float64; the PUCT score is
@@ -40,7 +41,7 @@ struct __align__(16) MctsGame {
     int leaf;       // node selected by the last aq_mcts_select
     int leaf_kind;  // 0 = evaluate with the network, 1 = terminal loss (-1), 2 = terminal draw (0)
     int overflow;   // arena exhausted (caller error: max_nodes too small)
-    int pad[4];
+    int pad[4];     // pad[0] != 0: the root's priors carry Dirichlet noise (aq_mcts_root_noise); reset / advance zero it
 };
 static_assert(sizeof(MctsGame) == 64, "MctsGame must be 64 bytes");
 
@@ -506,6 +507,102 @@ selfplay_compact_kernel(const AqState *__restrict__ moved, const uint8_t *__rest
 }
 
 // ------------------------------------------------------------------------------------------
+// Dirichlet noise on the root priors (AlphaZero; the reference has none).  For game g with K = n_children root children:
+//   eta ~ Dirichlet(alpha, ..., alpha),  p'_c = float32((1 - fraction) * (double)p_c + fraction * eta_c)  (double, rounded once)
+// eta is a pure function of (seed, game_id, ply, K, alpha).  Counter layout (tests/mcts_noise_oracle.py restates it):
+//   key        = mix64(mix64((seed ^ kNoiseDomain) + 0x9E3779B97F4A7C15 * (game_id + 1)) + 0xD1B54A32D192ED03 * (ply + 1))
+//                (the move draw of selfplay_move_kernel without the domain constant: the two draws are independent)
+//   U(c, j)    = ((mix64(key + 0x9E3779B97F4A7C15 * (c * kNoiseDraws + j + 1)) >> 11) + 1) * 2^-53, in (0, 1]
+//   gamma_c    : shape a = alpha + 1 if alpha < 1 else alpha, Marsaglia-Tsang with d = a - 1/3, k = 1 / sqrt(9 d).  Attempt
+//                i = 0 .. kNoiseAttempts-1 takes x = sqrt(-2 log U(c,3i+1)) * cos(2 pi U(c,3i+2)) (Box-Muller), t = 1 + k x, and
+//                accepts when t > 0 and log U(c,3i+3) < ((0.5 x x + d) - d v) + d log v with v = t t t: log G = log(d v).  No
+//                attempt accepted (probability < 1e-20): log G = log d.  For alpha < 1: log gamma_c = log G + log U(c,0) / alpha.
+//   eta_c      = exp(log gamma_c - max_k log gamma_k) / S, S summed as the warp does it: lane l adds its children l, l+32, ...
+//                in order from 0.0, then S_l += S_(l xor m) for m = 16, 8, 4, 2, 1.
+// The logs matter: at alpha = 0.03 U^(1/alpha) underflows to 0 for every child often enough to make the linear form 0/0.
+// All double products and sums are rounded one at a time (no contraction), as numpy computes them.
+// ------------------------------------------------------------------------------------------
+constexpr uint64_t kNoiseDomain = 0x243F6A8885A308D3ull;   // fractional digits of pi
+constexpr int kNoiseAttempts = 16;                          // Marsaglia-Tsang accepts > 95 % of attempts for a >= 1
+constexpr int kNoiseDraws = 1 + 3 * kNoiseAttempts;         // counters per child: the boost uniform, then 3 per attempt
+
+__device__ __forceinline__ double noise_uniform(uint64_t key, int c, int j) {
+    const uint64_t bits = mix64(key + 0x9E3779B97F4A7C15ull * (uint64_t)(c * kNoiseDraws + j + 1));
+    return (double)((bits >> 11) + 1) * 0x1p-53;
+}
+
+__device__ __forceinline__ double noise_log_gamma(uint64_t key, int c, double alpha) {
+    const bool boost = alpha < 1.0;
+    const double a = boost ? alpha + 1.0 : alpha;
+    const double d = a - 1.0 / 3.0, k = 1.0 / sqrt(9.0 * d);
+    double lg = log(d);
+    for (int i = 0; i < kNoiseAttempts; ++i) {
+        const double r = sqrt(-2.0 * log(noise_uniform(key, c, 3 * i + 1)));
+        const double x = __dmul_rn(r, cos(__dmul_rn(6.283185307179586, noise_uniform(key, c, 3 * i + 2))));
+        const double t = __dadd_rn(1.0, __dmul_rn(k, x));
+        if (!(t > 0.0)) continue;
+        const double v = __dmul_rn(__dmul_rn(t, t), t);
+        const double rhs = __dadd_rn(__dsub_rn(__dadd_rn(__dmul_rn(__dmul_rn(0.5, x), x), d), __dmul_rn(d, v)), __dmul_rn(d, log(v)));
+        if (log(noise_uniform(key, c, 3 * i + 3)) < rhs) {
+            lg = log(__dmul_rn(d, v));
+            break;
+        }
+    }
+    if (boost) lg = __dadd_rn(lg, log(noise_uniform(key, c, 0)) / alpha);
+    return lg;
+}
+
+// One warp per game, child c in lane c % 32 (as selfplay_move_kernel).  A root is noised when it is expanded and not yet noised.
+__global__ void __launch_bounds__(128)
+mcts_root_noise_kernel(MctsGame *games, MctsHot *hot_all, const MctsCold *__restrict__ cold_all, int64_t G, int64_t max_nodes,
+                       const int64_t *__restrict__ game_id, uint64_t seed, int ply, double alpha, double fraction,
+                       float *__restrict__ root_priors) {
+    const int lane = threadIdx.x & 31;
+    const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (g >= G) return;
+    MctsHot *hot = hot_all + g * max_nodes;
+    const MctsCold *cold = cold_all + g * max_nodes;
+    const int first = cold[0].first_child;
+    const int nc = first < 0 ? 0 : cold[0].n_children;
+    if (first >= 0 && games[g].pad[0] == 0) {
+        const uint64_t id = game_id ? (uint64_t)game_id[g] : (uint64_t)g;
+        const uint64_t key = mix64(mix64((seed ^ kNoiseDomain) + 0x9E3779B97F4A7C15ull * (id + 1)) + 0xD1B54A32D192ED03ull * (uint64_t)(ply + 1));
+        double e[kChildSlots];
+        double mx = -INFINITY;
+#pragma unroll
+        for (int s = 0; s < kChildSlots; ++s) {
+            const int c = lane + 32 * s;
+            e[s] = c < nc ? noise_log_gamma(key, c, alpha) : -INFINITY;
+            mx = fmax(mx, e[s]);
+        }
+#pragma unroll
+        for (int m = 16; m; m >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, m));
+        double sum = 0.0;
+#pragma unroll
+        for (int s = 0; s < kChildSlots; ++s) {
+            e[s] = lane + 32 * s < nc ? exp(e[s] - mx) : 0.0;
+            sum = __dadd_rn(sum, e[s]);
+        }
+#pragma unroll
+        for (int m = 16; m; m >>= 1) sum = __dadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, m));
+        const double keep = 1.0 - fraction;
+#pragma unroll
+        for (int s = 0; s < kChildSlots; ++s) {
+            const int c = lane + 32 * s;
+            if (c < nc) {
+                const double p = (double)hot[first + c].prior;
+                hot[first + c].prior = (float)__dadd_rn(__dmul_rn(keep, p), __dmul_rn(fraction, e[s] / sum));
+            }
+        }
+        if (lane == 0) games[g].pad[0] = 1;
+    }
+    if (root_priors) {
+        __syncwarp();
+        for (int c = lane; c < AQ_MAX_LEGAL; c += 32) root_priors[g * AQ_MAX_LEGAL + c] = c < nc ? hot[first + c].prior : 0.f;
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 extern "C" int64_t aq_mcts_ws_bytes(int64_t G, int64_t max_nodes) {
     return (int64_t)(mcts_nodes_offset(G) + (size_t)G * (size_t)max_nodes * kNodeBytes);
 }
@@ -575,6 +672,15 @@ extern "C" int aq_mcts_root_counts(void *ws, int64_t G, int64_t max_nodes, int32
     }
     return aq_launch("aq_mcts_root_counts", mcts_root_counts_kernel, (unsigned)((G + 3) / 4), 128, 0, st, false, games_of(ws), hot_of(ws, G),
                      cold_of(ws, G, max_nodes), G, max_nodes, counts, actions, n_children, overflow);
+}
+
+extern "C" int aq_mcts_root_noise(void *ws, int64_t G, int64_t max_nodes, const int64_t *game_id, uint64_t seed, int32_t ply, float alpha,
+                                  float fraction, float *root_priors, void *stream) {
+    if (G < 1 || max_nodes < 1 || !ws || !(alpha > 0.f) || !isfinite(alpha) || !(fraction >= 0.f && fraction <= 1.f))
+        return aq_set_error(AQ_ERR_ARG, "aq_mcts_root_noise");
+    return aq_launch("aq_mcts_root_noise", mcts_root_noise_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream), false,
+                     games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, game_id, seed, (int)ply, (double)alpha,
+                     (double)fraction, root_priors);
 }
 
 extern "C" int64_t aq_selfplay_ws_bytes(int64_t G) {

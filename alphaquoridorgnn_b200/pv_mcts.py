@@ -7,7 +7,10 @@ pv_mcts.py:47).  The reference has no virtual loss, no Dirichlet noise and no tr
 (pv_mcts.py:81 builds a fresh root per move), so each game's search is exactly the reference's.
 Tree reuse between moves (AlphaGo Zero: the child of the played move becomes the next root with its
 statistics) is opt-in, BatchedMCTS(..., tree_reuse=True); the default keeps the reference's fresh root.
+Dirichlet noise on the root priors (AlphaZero self-play exploration) is opt-in too,
+BatchedMCTS(..., dirichlet_alpha=0.3); the default searches with the network's priors.
 """
+import math
 from copy import deepcopy
 
 import numpy as np
@@ -39,11 +42,21 @@ class BatchedMCTS:
     tree_reuse=True (AlphaGo Zero; the reference has none): a search may continue the tree of the previous one
     (search(..., src_row, path)).  `sims` is then required: each game's arena holds 1 + 2 * sims * MAX_CHILDREN nodes, room
     for one carried search and one new one, and two workspaces are used in turn (the previous search's tree is read from one
-    while the next is built in the other)."""
+    while the next is built in the other).
 
-    def __init__(self, evaluator, sims=None, c_puct=C_PUCT, device=None, use_graph=True, tree_reuse=False):
+    dirichlet_alpha (AlphaZero; the reference has none): each search mixes eta ~ Dirichlet(dirichlet_alpha) into its root's child
+    priors, p' = (1 - noise_fraction) * p + noise_fraction * eta (aq_mcts_root_noise), once, before the first descent that reads
+    them: a carried root right after it is carried, a fresh root right after simulation 1 expands it.  The draw is keyed by
+    search(..., noise_seed, game_id, ply).  None (the default) runs exactly the search without noise."""
+
+    def __init__(self, evaluator, sims=None, c_puct=C_PUCT, device=None, use_graph=True, tree_reuse=False, dirichlet_alpha=None,
+                 noise_fraction=0.25):
         if tree_reuse and not sims:
             raise ValueError("BatchedMCTS(tree_reuse=True) needs `sims` at construction: it sizes the node arena")
+        if dirichlet_alpha is not None and not (math.isfinite(dirichlet_alpha) and dirichlet_alpha > 0):
+            raise ValueError(f"dirichlet_alpha must be a finite number > 0 (or None), not {dirichlet_alpha!r}")
+        if not 0.0 <= noise_fraction <= 1.0:
+            raise ValueError(f"noise_fraction must be in [0, 1], not {noise_fraction!r}")
         self.model = evaluator if hasattr(evaluator, "flat_parameters") else None
         self.evaluator = network_evaluator(evaluator) if hasattr(evaluator, "predict_batch") else evaluator
         self.sims = sims
@@ -51,6 +64,8 @@ class BatchedMCTS:
         self.device = gl._dev(device)
         self.use_graph = use_graph
         self.tree_reuse = bool(tree_reuse)
+        self.dirichlet_alpha = None if dirichlet_alpha is None else float(dirichlet_alpha)
+        self.noise_fraction = float(noise_fraction)
         self._ws = [None, None] if self.tree_reuse else [None]
         self._last = None     # tree_reuse: (workspace slot, G) of the previous search, the source a next search can continue
         self.last_kept = None  # tree_reuse: int32[G] nodes carried into each row by the last search (0 = fresh root), else None
@@ -115,8 +130,29 @@ class BatchedMCTS:
         torch.cuda.current_stream(dev).wait_stream(side)
         return g
 
+    def _noise_call(self, ws, G, max_nodes, G_real, noise_seed, game_id, ply):
+        """-> enqueue(stream) of aq_mcts_root_noise for this search, or None without noise.  Padded rows (G > G_real) get game id 0:
+        their results are discarded."""
+        if self.dirichlet_alpha is None:
+            return None
+        L, P = _lib.load(), _lib.ptr
+        if noise_seed is None:
+            noise_seed = int(torch.randint(0, 2 ** 63 - 1, (1,)).item())
+        gid = None
+        if game_id is not None:
+            gid = game_id.to(device=self.device, dtype=torch.int64).reshape(G_real)
+            if G > G_real:
+                gid = torch.cat([gid, gid.new_zeros((G - G_real,))])
+            gid = gid.contiguous()
+        seed, ply = int(noise_seed) & (2 ** 64 - 1), int(ply)
+
+        def enqueue(st):
+            _lib.check(L.aq_mcts_root_noise(P(ws), G, max_nodes, P(gid), seed, ply, self.dirichlet_alpha, self.noise_fraction, None, st),
+                       "aq_mcts_root_noise")
+        return enqueue
+
     @torch.no_grad()
-    def search_async(self, roots, sims=None, src_row=None, path=None):
+    def search_async(self, roots, sims=None, src_row=None, path=None, noise_seed=None, game_id=None, ply=0):
         """search() without the synchronisation: returns (counts, actions, n_children, status int32[3] on the device); the caller
         passes status.tolist() to check_status() when it synchronises anyway."""
         sims = sims or self.sims or PV_EVALUATE_COUNT
@@ -173,6 +209,12 @@ class BatchedMCTS:
                 self.last_kept = None
             if self.tree_reuse:
                 self._last = (slot, G)
+            # with noise: noise a carried root now; simulation 1 runs on its own and a fresh root, which it expands, is noised after it
+            noise = self._noise_call(ws, G, max_nodes, G_real, noise_seed, game_id, ply)
+            first = 0
+            if noise is not None:
+                noise(st)
+                first = 1
             if self.model is not None:
                 from .pv_network_gnn import PRECISIONS
                 flat = self.model.flat_parameters()
@@ -193,12 +235,13 @@ class BatchedMCTS:
                         if len(self._graphs) >= 32:
                             self._graphs.clear()
                         self._graphs[key] = graphs = {}
-                    left = sims - done
+                    alone = first > done   # simulation 1 still to run on its own: a replay of the one-step graph
+                    left = sims - max(done, first)
                     try:
                         # GRAPH_CHUNK simulations back to back in one graph (+ a one-step graph for the remainder, captured only when
                         # there is one): a search is a handful of graph launches instead of one per simulation -- a launch costs the
                         # host 10-100 us depending on the box, the step 75 us of GPU time at 4,096 games
-                        for steps in ((GRAPH_CHUNK,) if left >= GRAPH_CHUNK else ()) + ((1,) if left % GRAPH_CHUNK else ()):
+                        for steps in ((GRAPH_CHUNK,) if left >= GRAPH_CHUNK else ()) + ((1,) if left % GRAPH_CHUNK or alone else ()):
                             if steps not in graphs:
                                 graphs[steps] = self._capture(lambda cst, k=steps: self._step_network(ws, G, max_nodes, buf, flat, prep, prec, cst, k))
                     except _lib.AqError:
@@ -210,6 +253,14 @@ class BatchedMCTS:
                         self._graphs.clear()
                         torch.cuda.synchronize(dev)
                 left = sims - done
+                if first > done:   # simulation 1 on its own, then the noise of a fresh root
+                    if graphs is not None:
+                        graphs[1].replay()
+                    else:
+                        self._step_network(ws, G, max_nodes, buf, flat, prep, prec, st)
+                    left -= 1
+                if noise is not None:
+                    noise(st)
                 if graphs is not None:
                     for _ in range(left // GRAPH_CHUNK):
                         graphs[GRAPH_CHUNK].replay()
@@ -219,11 +270,13 @@ class BatchedMCTS:
                     for _ in range(left):
                         self._step_network(ws, G, max_nodes, buf, flat, prep, prec, st)
             else:
-                for _ in range(sims):
+                for i in range(sims):
                     _lib.check(L.aq_mcts_select(P(ws), G, max_nodes, self.c_puct, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_select")
                     out = self.evaluator(buf["leaf"])  # terminal leaves are evaluated too and ignored by the backup
                     _lib.check(L.aq_mcts_expand_backup(P(ws), G, max_nodes, P(out["priors"]), P(out["value"]), P(out["mask"]),
                                                        P(out["pawn"]), st), "aq_mcts_expand_backup")
+                    if i == 0 and noise is not None:
+                        noise(st)
             counts = torch.empty((G, gl.MAX_LEGAL), dtype=torch.int32, device=dev)
             actions = torch.empty((G, gl.MAX_LEGAL), dtype=torch.int16, device=dev)
             n = torch.empty((G,), dtype=torch.int16, device=dev)
@@ -245,7 +298,7 @@ class BatchedMCTS:
             raise _lib.AqError("the network returned NaN for a leaf: with precision 'bf16' that is how an activation beyond the fp16 range of the "
                                "aggregation operand is reported (gnn_tc2.cu); evaluate this network with precision 'fp32'")
 
-    def search(self, roots, sims=None, src_row=None, path=None):
+    def search(self, roots, sims=None, src_row=None, path=None, noise_seed=None, game_id=None, ply=0):
         """roots: packed uint8[G,32] (non-terminal states).  Runs `sims` simulations per game
         (pv_mcts.py:84) and returns (counts int32[G,136], actions int16[G,136], n_children int16[G]):
         visit counts of the root's children in State.legal_actions() order (pv_mcts.py:88).
@@ -253,8 +306,11 @@ class BatchedMCTS:
         With tree_reuse, src_row int64[G] (row of the previous search, -1 = fresh root) and path int16[G, k] (k = 1: the move
         played from that row's root; 2: and the reply) continue the previous search's trees: row g keeps the subtree below the
         path's end when that node was visited and its subtree leaves room for `sims` more simulations, else it starts fresh.
-        The counts then include the carried visits; last_kept gives the nodes carried per row."""
-        counts, actions, n, status = self.search_async(roots, sims, src_row, path)
+        The counts then include the carried visits; last_kept gives the nodes carried per row.
+
+        With dirichlet_alpha, the root noise of row g is drawn from (noise_seed, game_id[g], ply): game_id int64[G] (None = the row
+        index) names the game, so a game's noise does not depend on the other rows; noise_seed None draws one from torch's generator."""
+        counts, actions, n, status = self.search_async(roots, sims, src_row, path, noise_seed, game_id, ply)
         self.check_status(status.tolist())   # one synchronisation for both flags
         return counts, actions, n
 
@@ -270,19 +326,21 @@ class _SearcherCache(dict):
         return (_SearcherCache, ())
 
 
-def searcher_for(evaluator, sims, device=None, tree_reuse=False):
+def searcher_for(evaluator, sims, device=None, tree_reuse=False, dirichlet_alpha=None, noise_fraction=0.25):
     """The BatchedMCTS of a network for `sims` simulations, kept on the network object: its node arenas (3.5 GB at 4,096 games x
     200 simulations), leaf buffers and captured graphs are reused by every later self-play / arena / policy call on that network
     instead of being allocated and captured again.  Evaluators that are plain callables get a fresh searcher."""
     dev = gl._dev(device)
+    opts = dict(tree_reuse=tree_reuse, dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction)
     if not hasattr(evaluator, "flat_parameters"):
-        return BatchedMCTS(evaluator, sims, device=dev, tree_reuse=tree_reuse)
+        return BatchedMCTS(evaluator, sims, device=dev, **opts)
     cache = evaluator.__dict__.setdefault("_searchers", _SearcherCache())
-    key = (int(sims), str(dev), bool(tree_reuse))
+    key = (int(sims), str(dev), bool(tree_reuse), None if dirichlet_alpha is None else float(dirichlet_alpha),
+           None if dirichlet_alpha is None else float(noise_fraction))
     if key not in cache:
         if len(cache) >= 4:
             cache.clear()
-        cache[key] = BatchedMCTS(evaluator, sims, device=dev, tree_reuse=tree_reuse)
+        cache[key] = BatchedMCTS(evaluator, sims, device=dev, **opts)
     return cache[key]
 
 

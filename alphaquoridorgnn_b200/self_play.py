@@ -42,7 +42,7 @@ def write_data(history, directory='./data/'):
 
 @torch.no_grad()
 def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_TEMPERATURE, seed=None, max_plies=None,
-                      policy_dtype=torch.float64, tree_reuse=False):
+                      policy_dtype=torch.float64, tree_reuse=False, dirichlet_alpha=None, noise_fraction=0.25):
     """Execute `num_games` self-play games in lock-step (self_play.py:40-68 per game) and keep the record on the device:
     dict(states uint8[T,32] packed, policy [T,209] search policies over all actions (self_play.py:51-54), value f32[T]
     back-filled game results seen from the player to move (self_play.py:63-66), game int64[T], ply int64[T],
@@ -55,14 +55,18 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
     A game's moves are drawn from a hash of (seed, game, ply): they do not depend on the other games of the batch.
 
     tree_reuse=True (AlphaGo Zero; the reference builds a fresh root per move): each search continues the tree of the game's
-    previous one below the move played, so its policy counts the carried root visits as well as the `sims` new ones."""
+    previous one below the move played, so its policy counts the carried root visits as well as the `sims` new ones.
+
+    dirichlet_alpha (AlphaZero; the reference has none): every search mixes Dirichlet(dirichlet_alpha) noise into its root priors
+    with weight noise_fraction (BatchedMCTS), drawn from (seed, game, ply) like the moves, so a game still does not depend on the
+    other games of the batch and a seed reproduces the run.  The record is the same as without noise."""
     if policy_dtype not in (torch.float64, torch.float32):
         raise ValueError("policy_dtype must be torch.float64 or torch.float32")
     dev = gl._dev(device)
     L, P = _lib.load(), _lib.ptr
     seed = (int(seed) if seed is not None else int(torch.seed())) & (2 ** 64 - 1)
     sims = sims or pv_mcts.PV_EVALUATE_COUNT
-    mcts = pv_mcts.searcher_for(model, sims, dev, tree_reuse=tree_reuse)
+    mcts = pv_mcts.searcher_for(model, sims, dev, tree_reuse=tree_reuse, dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction)
     states = start_states(num_games, dev)
     game_id = torch.arange(num_games, device=dev)
     rec_state, rec_policy, rec_game, sizes = [], [], [], []
@@ -75,7 +79,7 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
     with torch.cuda.device(dev):
         while states.shape[0] > 0 and (max_plies is None or ply < max_plies):
             G = states.shape[0]
-            counts, actions, n, status = mcts.search_async(states, src_row=src_row, path=path)
+            counts, actions, n, status = mcts.search_async(states, src_row=src_row, path=path, noise_seed=seed, game_id=game_id, ply=ply)
             sims_run += G * sims
             dense = torch.empty((G, POLICY_OUTPUT_SIZE), dtype=policy_dtype, device=dev)
             nxt = torch.empty_like(states)
@@ -117,10 +121,12 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
             "flags": final_flags, "plies": final_plies, "sims": sims_run, "reused": reused}
 
 
-def play_batch(model, num_games, device=None, sims=None, temperature=SP_TEMPERATURE, seed=None, max_plies=None, tree_reuse=False):
+def play_batch(model, num_games, device=None, sims=None, temperature=SP_TEMPERATURE, seed=None, max_plies=None, tree_reuse=False,
+               dirichlet_alpha=None, noise_fraction=0.25):
     """play_batch_device + conversion to the reference's history: a list of [[player, enemy, walls], policy (209 floats), value]
     (self_play.py:51-54, 63-66), games in order, plies in order within a game.  Returns (history, dict with per-game results)."""
-    rec = play_batch_device(model, num_games, device, sims, temperature, seed, max_plies, tree_reuse=tree_reuse)
+    rec = play_batch_device(model, num_games, device, sims, temperature, seed, max_plies, tree_reuse=tree_reuse,
+                            dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction)
     rows, _ = gl.unpack_rows(rec["states"])
     rows = rows.cpu().numpy()
     pols = rec["policy"].cpu().numpy()
@@ -140,15 +146,18 @@ def play(model, device=None):
     return history
 
 
-def self_play(game_count=None, model_path=None, data_dir='./data/', rank=0, world_size=1, sims=None, seed=None, tree_reuse=False):
+def self_play(game_count=None, model_path=None, data_dir='./data/', rank=0, world_size=1, sims=None, seed=None, tree_reuse=False,
+              dirichlet_alpha=None, noise_fraction=0.25):
     """Perform self-play games and save the training data (self_play.py:71-98).  With
     world_size > 1 each rank plays its share of the games on its own GPU and rank 0 writes the file.
-    tree_reuse=True keeps each game's search tree between moves (see play_batch_device)."""
+    tree_reuse=True keeps each game's search tree between moves; dirichlet_alpha adds AlphaZero root noise to every search
+    (see play_batch_device)."""
     game_count = SP_GAME_COUNT if game_count is None else game_count
     model = GNNNetwork()
     model.prep_for_inference(model_path=model_path or (PV_NETWORK_PATH + 'best.pth'))
     mine = game_count // world_size + (1 if rank < game_count % world_size else 0)
-    history, _ = play_batch(model, mine, sims=sims, seed=None if seed is None else seed + rank, tree_reuse=tree_reuse) if mine else ([], None)
+    history, _ = play_batch(model, mine, sims=sims, seed=None if seed is None else seed + rank, tree_reuse=tree_reuse,
+                            dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction) if mine else ([], None)
     if world_size > 1:
         import torch.distributed as dist
         gathered = [None] * world_size if rank == 0 else None

@@ -53,7 +53,7 @@ typedef struct AqState {
     uint64_t reserved; /* reserved, 0 */
 } AqState;
 
-#define AQ_VERSION 206 /* bumped with every change of a signature below; the ctypes loader refuses a library of another version */
+#define AQ_VERSION 207 /* bumped with every change of a signature below; the ctypes loader refuses a library of another version */
 int aq_version(void);
 const char *aq_last_error_string(void);
 /* Number of kernels this library has launched in the process so far (monotonic; kernels replayed through a CUDA graph the caller
@@ -280,6 +280,23 @@ int aq_mcts_expand_select(void *ws, int64_t G, int64_t max_nodes, const float *p
                           const uint8_t *pawn, float c_puct, AqState *leaf_states, int32_t *leaf_kind, void *stream);
 int aq_mcts_root_counts(void *ws, int64_t G, int64_t max_nodes, int32_t *counts /*[G,136]*/,
                         int16_t *actions /*[G,136]*/, int16_t *n_children /*[G]*/, int32_t *overflow, void *stream);
+/* Dirichlet noise on the priors of every expanded, not yet noised root (AlphaZero; the reference has none).
+ *   game_id [G] int64 (NULL: the row index), seed / ply: the key of the draw; alpha > 0, 0 <= fraction <= 1
+ *   root_priors [G,136] f32 (may be NULL): the root's child priors after the call, legal_actions() order, 0 beyond n_children
+ * A root is noised at most once between aq_mcts_reset / aq_mcts_advance and the next one; calling again is a no-op for it.
+ * For game g with K = n_children root children, priors p_c in legal_actions() order:
+ *   eta ~ Dirichlet(alpha, ..., alpha) over the K children, a pure function of (seed, game_id[g], ply, K, alpha): a counter-based
+ *         draw (splitmix64, keyed like the move draw of aq_selfplay_advance with its own domain constant), independent of the
+ *         other games of the batch, of the row and of padding rows.  Gamma variates: Marsaglia-Tsang with Box-Muller normals at
+ *         shape alpha (alpha >= 1) or alpha + 1 boosted by u^(1/alpha) (alpha < 1), in logs, normalised with the maximum
+ *         subtracted; csrc/mcts.cu documents the exact counter layout
+ *   p'_c = float32((1 - fraction) * (double)p_c + fraction * eta_c), computed in double and rounded once (fraction 0: p'_c = p_c)
+ * Callers noise a search's root once before its first descent that reads the root's children: right after aq_mcts_advance for a
+ * carried root, right after simulation 1 (which expands it) for a fresh one; calling before and after simulation 1 does both.
+ * The noised priors stay in the tree for the rest of the search.  AQ_ERR_ARG for G < 1, a null ws, alpha <= 0 or not finite,
+ * fraction outside [0, 1] or NaN. */
+int aq_mcts_root_noise(void *ws, int64_t G, int64_t max_nodes, const int64_t *game_id, uint64_t seed, int32_t ply,
+                       float alpha, float fraction, float *root_priors, void *stream);
 
 /* One ply of G lock-step self-play games after their searches (self_play.py:47-60), two launches:
  *   scores = counts ** (1 / temperature) / sum over the root's children (pv_mcts.py:88-95; temperature 0 = one-hot on
