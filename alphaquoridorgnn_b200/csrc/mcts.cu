@@ -47,26 +47,7 @@ static_assert(sizeof(MctsGame) == 64, "MctsGame must be 64 bytes");
 
 static inline size_t mcts_nodes_offset(int64_t G) { return ((size_t)G * sizeof(MctsGame) + 255) & ~(size_t)255; }
 
-__global__ void mcts_reset_kernel(MctsGame *games, MctsHot *hot, MctsCold *cold, const AqState *__restrict__ roots, int64_t G,
-                                  int64_t max_nodes) {
-    const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= G) return;
-    MctsGame gm;
-    gm.root = load_state(roots + g);
-    gm.node_count = 1;
-    gm.leaf = 0;
-    gm.leaf_kind = 0;
-    gm.overflow = 0;
-    gm.pad[0] = gm.pad[1] = gm.pad[2] = gm.pad[3] = 0;
-    games[g] = gm;
-    MctsHot rh;
-    rh.w = 0.0; rh.prior = 0.f; rh.n = 0;
-    MctsCold rc;
-    rc.first_child = -1; rc.parent = -1; rc.n_children = 0; rc.action = -1; rc.pad = 0;
-    hot[g * max_nodes] = rh;  // root node: Node(state, 0), pv_mcts.py:81
-    cold[g * max_nodes] = rc;
-}
-
+// root node: Node(state, 0), pv_mcts.py:81
 __device__ __forceinline__ void write_fresh_root(MctsHot *hot, MctsCold *cold) {
     MctsHot rh;
     rh.w = 0.0; rh.prior = 0.f; rh.n = 0;
@@ -74,6 +55,22 @@ __device__ __forceinline__ void write_fresh_root(MctsHot *hot, MctsCold *cold) {
     rc.first_child = -1; rc.parent = -1; rc.n_children = 0; rc.action = -1; rc.pad = 0;
     hot[0] = rh;
     cold[0] = rc;
+}
+
+// A game at the start of a search: nothing selected, no overflow, root priors without noise.
+__device__ __forceinline__ MctsGame start_game(const AqState &root, int node_count) {
+    MctsGame gm = {};
+    gm.root = root;
+    gm.node_count = node_count;
+    return gm;
+}
+
+__global__ void mcts_reset_kernel(MctsGame *games, MctsHot *hot, MctsCold *cold, const AqState *__restrict__ roots, int64_t G,
+                                  int64_t max_nodes) {
+    const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= G) return;
+    games[g] = start_game(load_state(roots + g), 1);
+    write_fresh_root(hot + g * max_nodes, cold + g * max_nodes);
 }
 
 __device__ __forceinline__ bool same_position(const AqState &a, const AqState &b) {
@@ -169,14 +166,7 @@ mcts_advance_kernel(const MctsGame *__restrict__ src_games, const MctsHot *__res
     __syncwarp();
     if (lane == 0) {
         if (count == 0) write_fresh_root(hot, cold);
-        MctsGame gm;
-        gm.root = root;
-        gm.node_count = count ? count : 1;
-        gm.leaf = 0;
-        gm.leaf_kind = 0;
-        gm.overflow = 0;
-        gm.pad[0] = gm.pad[1] = gm.pad[2] = gm.pad[3] = 0;
-        dst_games[g] = gm;
+        dst_games[g] = start_game(root, count ? count : 1);
         if (kept) kept[g] = count;
     }
 }

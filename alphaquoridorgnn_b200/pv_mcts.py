@@ -35,9 +35,9 @@ def network_evaluator(model):
 class BatchedMCTS:
     """Lock-step PV-MCTS over G independent root states.
 
-    `evaluator` is either a GNNNetwork (leaf evaluation = aq_leaf_eval into preallocated buffers, and the
-    whole simulation step -- select, legal mask, GNN trunk, heads, expand+backup -- is captured once in a
-    CUDA graph and replayed `sims` times) or any callable following the evaluator protocol (eager loop).
+    `evaluator` is either a GNNNetwork (leaf evaluation = aq_leaf_eval into preallocated buffers; the simulation
+    step -- select, legal mask, GNN trunk, heads, expand+backup -- is captured in CUDA graphs of GRAPH_CHUNK steps
+    and of one step, and a search replays those) or any callable following the evaluator protocol (eager loop).
 
     tree_reuse=True (AlphaGo Zero; the reference has none): a search may continue the tree of the previous one
     (search(..., src_row, path)).  `sims` is then required: each game's arena holds 1 + 2 * sims * MAX_CHILDREN nodes, room
@@ -98,58 +98,52 @@ class BatchedMCTS:
             }
         return self._buf[G]
 
-    def _step_network(self, ws, G, max_nodes, buf, flat, prep, prec, st, steps=1):
-        """`steps` simulations for all games with the network evaluator: select, then `steps` leaf evaluations (three kernels each)
-        joined by the fused expand + backup + next select, then the last expand + backup."""
+    def _step(self, ws, G, max_nodes, buf, evaluate, st, steps=1):
+        """`steps` simulations for all games: select, then `steps` leaf evaluations out = evaluate(stream) (terminal leaves are
+        evaluated too and ignored by the backup) joined by the fused expand + backup + next select, then the last expand + backup."""
         L, P = _lib.load(), _lib.ptr
         _lib.check(L.aq_mcts_select(P(ws), G, max_nodes, self.c_puct, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_select")
         for i in range(steps):
-            _lib.check(L.aq_leaf_eval(P(flat), P(prep), P(buf["leaf"]), G, P(buf["priors"]), P(buf["value"]), P(buf["mask"]), P(buf["pawn"]),
-                                      P(buf["pooled"]), prec, st), "aq_leaf_eval")
+            out = evaluate(st)
+            leaves = (P(ws), G, max_nodes, P(out["priors"]), P(out["value"]), P(out["mask"]), P(out["pawn"]))
             if i + 1 < steps:
-                _lib.check(L.aq_mcts_expand_select(P(ws), G, max_nodes, P(buf["priors"]), P(buf["value"]), P(buf["mask"]), P(buf["pawn"]),
-                                                   self.c_puct, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_expand_select")
+                _lib.check(L.aq_mcts_expand_select(*leaves, self.c_puct, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_expand_select")
             else:
-                _lib.check(L.aq_mcts_expand_backup(P(ws), G, max_nodes, P(buf["priors"]), P(buf["value"]), P(buf["mask"]),
-                                                   P(buf["pawn"]), st), "aq_mcts_expand_backup")
+                _lib.check(L.aq_mcts_expand_backup(*leaves, st), "aq_mcts_expand_backup")
 
-    def _capture(self, enqueue):
-        """Capture enqueue(stream pointer) into a CUDA graph.  `torch.cuda.graph` is not used on purpose: on entry it empties the
-        caching allocator (the 3.5 GB workspace of a finished searcher goes back to the driver and the next one pays cudaMalloc
-        again) -- 50-350 ms per capture on the boxes measured, and self-play captures once per batch size."""
-        dev = self.device
-        g = torch.cuda.CUDAGraph()
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        with torch.cuda.stream(side):
-            g.capture_begin(capture_error_mode="thread_local")
-            try:
-                enqueue(_lib.stream_ptr(dev))
-            finally:
-                g.capture_end()
-        torch.cuda.current_stream(dev).wait_stream(side)
-        return g
-
-    def _noise_call(self, ws, G, max_nodes, G_real, noise_seed, game_id, ply):
-        """-> enqueue(stream) of aq_mcts_root_noise for this search, or None without noise.  Padded rows (G > G_real) get game id 0:
-        their results are discarded."""
-        if self.dirichlet_alpha is None:
-            return None
-        L, P = _lib.load(), _lib.ptr
-        if noise_seed is None:
-            noise_seed = int(torch.randint(0, 2 ** 63 - 1, (1,)).item())
-        gid = None
-        if game_id is not None:
-            gid = game_id.to(device=self.device, dtype=torch.int64).reshape(G_real)
-            if G > G_real:
-                gid = torch.cat([gid, gid.new_zeros((G - G_real,))])
-            gid = gid.contiguous()
-        seed, ply = int(noise_seed) & (2 ** 64 - 1), int(ply)
-
-        def enqueue(st):
-            _lib.check(L.aq_mcts_root_noise(P(ws), G, max_nodes, P(gid), seed, ply, self.dirichlet_alpha, self.noise_fraction, None, st),
-                       "aq_mcts_root_noise")
-        return enqueue
+    def _simulate(self, n, step, key, st):
+        """n simulations; step(stream, k) enqueues k of them.  With a graph key (network evaluator) and use_graph, they are replays of
+        CUDA graphs captured for the key; else one eager step per simulation."""
+        if self.use_graph and key is not None:
+            if not self._warm and n:
+                # the searcher's first step runs outside capture: lazy initialisation (module load, function attributes) must not
+                # happen inside one; a failure here is a real error and propagates
+                step(st, 1)
+                n, self._warm = n - 1, True
+                torch.cuda.synchronize(self.device)
+            graphs = self._graphs.get(key)
+            if graphs is None:
+                if len(self._graphs) >= 32:
+                    self._graphs.clear()
+                graphs = self._graphs[key] = {}
+            # GRAPH_CHUNK simulations back to back in one graph (+ a one-step graph for the remainder, captured only when there is
+            # one): a search is a handful of graph launches instead of one per simulation -- a launch costs the host 10-100 us
+            # depending on the box, the step 75 us of GPU time at 4,096 games
+            for k in ((GRAPH_CHUNK,) if n >= GRAPH_CHUNK else ()) + ((1,) if n % GRAPH_CHUNK else ()):
+                if k not in graphs:
+                    graphs[k] = _lib.capture_graph(self.device, lambda cst: step(cst, k), "the MCTS simulation step")
+                    if graphs[k] is None:
+                        self.use_graph = False
+                        self._graphs.clear()
+                        break
+            if self.use_graph:
+                for _ in range(n // GRAPH_CHUNK):
+                    graphs[GRAPH_CHUNK].replay()
+                for _ in range(n % GRAPH_CHUNK):
+                    graphs[1].replay()
+                return
+        for _ in range(n):
+            step(st, 1)
 
     @torch.no_grad()
     def search_async(self, roots, sims=None, src_row=None, path=None, noise_seed=None, game_id=None, ply=0):
@@ -178,14 +172,14 @@ class BatchedMCTS:
         # real ones are unaffected): workspaces, buffers and the captured CUDA graph of the simulation step are then reused across
         # plies instead of being rebuilt for every distinct size.
         if self.model is not None and self.use_graph and G_real > 256 and G_real % 256:
-            pad = 256 - G_real % 256
-            roots = torch.cat([roots, roots[-1:].expand(pad, -1)]).contiguous()
+            roots = torch.cat([roots, roots[-1:].expand(256 - G_real % 256, -1)]).contiguous()
         G = roots.shape[0]
-        if self.tree_reuse:
-            max_nodes = 1 + 2 * self.sims * MAX_CHILDREN
-            slot = 0 if self._last is None else 1 - self._last[0]
-        else:
-            max_nodes, slot = 1 + sims * MAX_CHILDREN, 0
+
+        def pad(t, fill):   # a per-game argument for the padded rows: they start fresh (src_row -1) and draw the noise of game 0
+            return (torch.cat([t, t.new_full((G - G_real,) + t.shape[1:], fill)]) if G > G_real else t).contiguous()
+
+        max_nodes = 1 + (2 * self.sims if self.tree_reuse else sims) * MAX_CHILDREN
+        slot = 0 if self._last is None else 1 - self._last[0]
         ws = self._workspace(G, max_nodes, slot)
         buf = self._buffers(G)
         # [arena overflow, NaN leaf value, inconsistent tree-reuse rows]
@@ -194,12 +188,8 @@ class BatchedMCTS:
             st = _lib.stream_ptr(dev)
             if src_row is not None:
                 src_slot, G_src = self._last
-                src = src_row.to(device=dev, dtype=torch.int64).reshape(G_real)
-                path = path.to(device=dev, dtype=torch.int16).reshape(G_real, -1)
-                if G > G_real:  # padded rows start fresh
-                    src = torch.cat([src, src.new_full((G - G_real,), -1)])
-                    path = torch.cat([path, path.new_zeros((G - G_real, path.shape[1]))])
-                src, path = src.contiguous(), path.contiguous()
+                src = pad(src_row.to(device=dev, dtype=torch.int64).reshape(G_real), -1)
+                path = pad(path.to(device=dev, dtype=torch.int16).reshape(G_real, -1), 0)
                 kept = torch.empty((G,), dtype=torch.int32, device=dev)
                 _lib.check(L.aq_mcts_advance(P(self._ws[src_slot]), G_src, P(ws), G, max_nodes, P(roots), P(src), P(path), path.shape[1],
                                              sims * MAX_CHILDREN, P(kept), P(status[2:]), st), "aq_mcts_advance")
@@ -209,12 +199,6 @@ class BatchedMCTS:
                 self.last_kept = None
             if self.tree_reuse:
                 self._last = (slot, G)
-            # with noise: noise a carried root now; simulation 1 runs on its own and a fresh root, which it expands, is noised after it
-            noise = self._noise_call(ws, G, max_nodes, G_real, noise_seed, game_id, ply)
-            first = 0
-            if noise is not None:
-                noise(st)
-                first = 1
             if self.model is not None:
                 from .pv_network_gnn import PRECISIONS
                 flat = self.model.flat_parameters()
@@ -222,61 +206,25 @@ class BatchedMCTS:
                 # bf16 operand tiles, refreshed in place if the parameters changed since the last search
                 prep = self.model.prepared_weights() if prec == 1 else None
                 key = (G, max_nodes, ws.data_ptr(), flat.data_ptr(), prep.data_ptr() if prep is not None else 0, prec)
-                graphs = self._graphs.get(key) if self.use_graph else None
-                done = 0
-                if self.use_graph:
-                    if graphs is None:
-                        if not self._warm:
-                            # the searcher's first step runs outside capture (= simulation 1): lazy initialisation (module load,
-                            # function attributes) must not happen inside one; a failure here is a real error and propagates
-                            self._step_network(ws, G, max_nodes, buf, flat, prep, prec, st)
-                            done, self._warm = 1, True
-                            torch.cuda.synchronize(dev)
-                        if len(self._graphs) >= 32:
-                            self._graphs.clear()
-                        self._graphs[key] = graphs = {}
-                    alone = first > done   # simulation 1 still to run on its own: a replay of the one-step graph
-                    left = sims - max(done, first)
-                    try:
-                        # GRAPH_CHUNK simulations back to back in one graph (+ a one-step graph for the remainder, captured only when
-                        # there is one): a search is a handful of graph launches instead of one per simulation -- a launch costs the
-                        # host 10-100 us depending on the box, the step 75 us of GPU time at 4,096 games
-                        for steps in ((GRAPH_CHUNK,) if left >= GRAPH_CHUNK else ()) + ((1,) if left % GRAPH_CHUNK or alone else ()):
-                            if steps not in graphs:
-                                graphs[steps] = self._capture(lambda cst, k=steps: self._step_network(ws, G, max_nodes, buf, flat, prep, prec, cst, k))
-                    except _lib.AqError:
-                        raise
-                    except Exception as e:  # capture unsupported: stay eager, but say so
-                        import warnings
-                        warnings.warn(f"CUDA-graph capture of the MCTS simulation step failed ({e!r}); running the step eagerly")
-                        self.use_graph, graphs = False, None
-                        self._graphs.clear()
-                        torch.cuda.synchronize(dev)
-                left = sims - done
-                if first > done:   # simulation 1 on its own, then the noise of a fresh root
-                    if graphs is not None:
-                        graphs[1].replay()
-                    else:
-                        self._step_network(ws, G, max_nodes, buf, flat, prep, prec, st)
-                    left -= 1
-                if noise is not None:
-                    noise(st)
-                if graphs is not None:
-                    for _ in range(left // GRAPH_CHUNK):
-                        graphs[GRAPH_CHUNK].replay()
-                    for _ in range(left % GRAPH_CHUNK):
-                        graphs[1].replay()
-                else:
-                    for _ in range(left):
-                        self._step_network(ws, G, max_nodes, buf, flat, prep, prec, st)
+
+                def evaluate(s):
+                    _lib.check(L.aq_leaf_eval(P(flat), P(prep), P(buf["leaf"]), G, P(buf["priors"]), P(buf["value"]), P(buf["mask"]),
+                                              P(buf["pawn"]), P(buf["pooled"]), prec, s), "aq_leaf_eval")
+                    return buf
             else:
-                for i in range(sims):
-                    _lib.check(L.aq_mcts_select(P(ws), G, max_nodes, self.c_puct, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_select")
-                    out = self.evaluator(buf["leaf"])  # terminal leaves are evaluated too and ignored by the backup
-                    _lib.check(L.aq_mcts_expand_backup(P(ws), G, max_nodes, P(out["priors"]), P(out["value"]), P(out["mask"]),
-                                                       P(out["pawn"]), st), "aq_mcts_expand_backup")
-                    if i == 0 and noise is not None:
-                        noise(st)
+                key, evaluate = None, lambda s: self.evaluator(buf["leaf"])
+            step = lambda s, k: self._step(ws, G, max_nodes, buf, evaluate, s, k)
+            if self.dirichlet_alpha is None:
+                self._simulate(sims, step, key, st)
+            else:
+                seed = (int(torch.randint(0, 2 ** 63 - 1, (1,)).item()) if noise_seed is None else int(noise_seed)) & (2 ** 64 - 1)
+                gid = None if game_id is None else pad(game_id.to(device=dev, dtype=torch.int64).reshape(G_real), 0)
+                # aq_mcts_root_noise skips a root that is unexpanded or noised already, so noising before and after simulation 1 is the
+                # whole rule: the first call noises a carried root, the second a fresh root, which simulation 1 expanded
+                for n in (1, sims - 1):
+                    _lib.check(L.aq_mcts_root_noise(P(ws), G, max_nodes, P(gid), seed, int(ply), self.dirichlet_alpha, self.noise_fraction,
+                                                    None, st), "aq_mcts_root_noise")
+                    self._simulate(n, step, key, st)
             counts = torch.empty((G, gl.MAX_LEGAL), dtype=torch.int32, device=dev)
             actions = torch.empty((G, gl.MAX_LEGAL), dtype=torch.int16, device=dev)
             n = torch.empty((G,), dtype=torch.int16, device=dev)

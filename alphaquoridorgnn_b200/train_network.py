@@ -176,10 +176,9 @@ class FlatTrainer:
                                      torch.empty((b,), dtype=torch.float32, device=dev))
         return buf
 
-    def _enqueue(self, buf, packed, policy_target, value_target, b, global_batch, lr):
-        """The library calls of one step (eagerly, or under CUDA-graph capture)."""
+    def _enqueue(self, buf, packed, policy_target, value_target, b, global_batch, lr, st):
+        """The library calls of one step on stream `st` (eagerly, or under CUDA-graph capture)."""
         L, P = _lib.load(), _lib.ptr
-        st = _lib.stream_ptr(self.flat.device)
         c0 = L.aq_launch_count()
         _lib.check(L.aq_gnn_forward(P(self.flat), P(packed), None, None, b, P(buf["policy"]), P(buf["value"]), P(buf["saved"]), self.prec, st),
                    "aq_gnn_forward")
@@ -225,30 +224,17 @@ class FlatTrainer:
                     # replayed as one CUDA graph; the first step with a key runs eagerly, the second is captured
                     key = (b, int(global_batch), lr, packed.data_ptr(), policy_target.data_ptr(), value_target.data_ptr())
                     graph = self._graphs.get(key) if self.use_graph else None
-                    if not self.use_graph or (graph is None and key not in self._graphs):
+                    if self.use_graph and graph is None and key in self._graphs:
+                        graph = self._graphs[key] = _lib.capture_graph(dev, lambda cst: self._enqueue(*args, cst), "the training step")
+                        self.use_graph = graph is not None
+                    if graph is not None:
+                        graph.replay()   # also right after the capture: capture records, it does not execute
+                    else:
                         if self.use_graph:
                             if len(self._graphs) >= 16:
                                 self._graphs.clear()
                             self._graphs[key] = None
-                        self._enqueue(*args)
-                    elif graph is None:
-                        try:
-                            torch.cuda.synchronize(dev)
-                            g = torch.cuda.CUDAGraph()
-                            with torch.cuda.graph(g):
-                                self._enqueue(*args)
-                            self._graphs[key] = g
-                            g.replay()   # capture records, it does not execute
-                        except _lib.AqError:
-                            raise
-                        except Exception as e:  # capture unsupported: stay eager, but say so
-                            import warnings
-                            warnings.warn(f"CUDA-graph capture of the training step failed ({e!r}); running eagerly")
-                            self.use_graph = False
-                            torch.cuda.synchronize(dev)
-                            self._enqueue(*args)
-                    else:
-                        graph.replay()
+                        self._enqueue(*args, st)
                 self.step_count += 1
             else:
                 if b > 0:

@@ -21,12 +21,20 @@ ws, buf = m._workspace(G, max_nodes), m._buffers(G)
 st = _lib.stream_ptr()
 L.aq_mcts_reset(P(ws), P(roots), G, max_nodes, st)
 flat, prep = net.flat_parameters(), net.prepared_weights()
+
+
+def evaluate(s):
+    _lib.check(L.aq_leaf_eval(P(flat), P(prep), P(buf["leaf"]), G, P(buf["priors"]), P(buf["value"]), P(buf["mask"]), P(buf["pawn"]),
+                              P(buf["pooled"]), PRECISIONS["bf16"], s), "aq_leaf_eval")
+    return buf
+
+
 for _ in range(60):
-    m._step_network(ws, G, max_nodes, buf, flat, prep, PRECISIONS["bf16"], st)
+    m._step(ws, G, max_nodes, buf, evaluate, st)
 torch.cuda.synchronize()
 torch.cuda.profiler.start()
 for _ in range(3):
-    m._step_network(ws, G, max_nodes, buf, flat, prep, PRECISIONS["bf16"], st)
+    m._step(ws, G, max_nodes, buf, evaluate, st)
 torch.cuda.synchronize()
 torch.cuda.profiler.stop()
 print("done")
