@@ -573,7 +573,7 @@ int aq_dp_adam_launch(void *comm, const float *grads_in, const float *partial, i
 int aq_heads_wgrad_tc_slots(int64_t B);  // heads_wgrad_tc.cu
 int aq_heads_wgrad_tc(const float *dhp, const float *dhv, const float *dz, const float *du, const float *pooled, const float *hp,
                       const float *hv, int64_t B, float *partial, cudaStream_t st);
-// partial slots that hold head gradients: fp32 path (atb_jobs_kernel) one row chunk per 64 boards; tensor-core path one per 128-board tile
+// partial slots that hold head gradients: fp32 path (atb_jobs_kernel) one row chunk per 64 boards; tensor-core path one per 64-board tile
 static inline int head_slot_count(int64_t B, int precision) {
     if (precision == 1) return aq_heads_wgrad_tc_slots(B);
     return (int)std::min<int64_t>(kSlots, (B + AQ_HEAD_CHUNK_ROWS - 1) / AQ_HEAD_CHUNK_ROWS);

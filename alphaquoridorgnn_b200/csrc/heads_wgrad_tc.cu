@@ -6,7 +6,7 @@
 // K = boards.  Both operands of a product are stored as the producer has them -- one row per board, the M (or N) index contiguous --
 // i.e. MN-major for tcgen05.mma: bf16 tiles [32-wide MN blocks][K atoms of 8 boards][8][64 B], SWIZZLE_64B, the layout the trunk uses
 // for its feature-major activations.  A "ones" column appended to each B operand makes the bias gradient (column sums of A over the
-// boards) one more accumulator column.  One CTA per 128-board tile (grid-stride beyond 148 tiles), accumulators in tensor memory
+// boards) one more accumulator column.  One CTA per 64-board tile (kWgTile; grid-stride beyond 148 tiles), accumulators in tensor memory
 // across the CTA's tiles, written once into the CTA's partial-gradient slot; the slot reduction that follows is the existing one.
 // Replaces atb_jobs_kernel (FFMA, 39 us at B = 4,096) for the tensor-core training path; the fp32 path keeps atb_jobs_kernel.
 #include <cstddef>
@@ -312,7 +312,7 @@ heads_wgrad_tc_kernel(const float *dhp, const float *dhv, const float *dz, const
 
 }  // namespace
 
-// Number of partial slots the kernel fills (= its grid): one per 128-board tile, at most one per SM.
+// Number of partial slots the kernel fills (= its grid): one per 64-board tile (kWgTile), at most one per SM.
 int aq_heads_wgrad_tc_slots(int64_t B) {
     const int64_t tiles = (B + kWgTile - 1) / kWgTile;
     return (int)(tiles < 148 ? tiles : 148);

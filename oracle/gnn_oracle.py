@@ -17,6 +17,7 @@ tests/test_oracle_gnn.py compares with the edge-list formulation.
 state_dict keys equal the reference's (gcn_layers.{i}.lin.weight, gcn_layers.{i}.bias,
 policy_head.{0,2}.{weight,bias}, value_head.{0,2}.{weight,bias}).
 """
+import copy
 import math
 
 import numpy as np
@@ -219,3 +220,48 @@ def forward_tc_emulation(model, x, edge_index, batch):
     hv = F.relu(g @ _Round.apply(vh[0].weight, bf).t() + vh[0].bias)
     value = torch.tanh(hv @ vh[2].weight.t() + vh[2].bias)
     return policy, value
+
+
+# ---- training-gradient references (test infrastructure) ------------------------------------------------------------------------
+def oracle_grads_fp64(ref, rows, pt, vt, chunk=512, emulate_tc=False):
+    """fp64 oracle autograd of the reference loss (train_network.py:54-55,85-89: both 'mean' over the batch), accumulated over chunks
+    of boards so that the edge-list formulation fits in memory: mean over B = sum over chunks of (chunk mean x n_chunk / B).
+    emulate_tc: the forward pass carries the tensor-core path's rounding points (forward_tc_emulation).
+    Returns (loss, {parameter name: gradient})."""
+    ref64 = copy.deepcopy(ref).double()
+    B = len(rows)
+    total = 0.0
+    for lo in range(0, B, chunk):
+        hi = min(B, lo + chunk)
+        x, ei, batch = graph_inputs_from_rows(rows[lo:hi], dtype=torch.float64)
+        p64, v64 = forward_tc_emulation(ref64, x, ei, batch) if emulate_tc else ref64(x, ei, batch)
+        loss, _, _ = training_loss(p64, v64, pt[lo:hi].double(), vt[lo:hi].double())
+        (loss * ((hi - lo) / B)).backward()
+        total += loss.item() * (hi - lo) / B
+    return total, {n: p.grad for n, p in ref64.named_parameters()}
+
+
+def probe_upstream(row_ids):
+    """Upstream gradient of probe boards: dpolicy ~ N(0,1)[209] and dvalue ~ N(0,1) in float32, drawn from a generator seeded by each
+    board's row id -- the same board gets the same upstream gradient in every batch it is placed in.  -> (dpolicy [n,209], dvalue [n])."""
+    dp = np.empty((len(row_ids), POLICY_OUTPUT_SIZE), np.float32)
+    dv = np.empty((len(row_ids),), np.float32)
+    for i, r in enumerate(row_ids):
+        g = np.random.default_rng(int(r))
+        dp[i] = g.standard_normal(POLICY_OUTPUT_SIZE, dtype=np.float32)
+        dv[i] = g.standard_normal(dtype=np.float32)
+    return dp, dv
+
+
+def probe_grads_fp64(ref, rows, dpolicy, dvalue, emulate_tc=False):
+    """fp64 gradient with respect to the parameters of sum_b (policy_b . dpolicy_b + value_b * dvalue_b) over the given boards.
+    Every operation from the outputs back to the weights is linear in the upstream gradient, so this is also the gradient of any
+    larger batch that holds these boards and has zero upstream rows everywhere else (as long as its activations are finite): a
+    reference for a few probe boards of a batch of any size.  emulate_tc as in oracle_grads_fp64.  -> {parameter name: gradient}."""
+    ref64 = copy.deepcopy(ref).double()
+    x, ei, batch = graph_inputs_from_rows(rows, dtype=torch.float64)
+    p64, v64 = forward_tc_emulation(ref64, x, ei, batch) if emulate_tc else ref64(x, ei, batch)
+    dp = torch.as_tensor(np.asarray(dpolicy), dtype=torch.float64).reshape(p64.shape)
+    dv = torch.as_tensor(np.asarray(dvalue), dtype=torch.float64).reshape(v64.shape)
+    ((p64 * dp).sum() + (v64 * dv).sum()).backward()
+    return {n: p.grad for n, p in ref64.named_parameters()}

@@ -583,23 +583,6 @@ def test_bf16_leaf_eval_at_the_benchmarked_batch_matches_oracle():
         evl.close()
 
 
-def _oracle_grads_fp64(ref, rows, pt, vt, chunk=512, emulate_tc=False):
-    """fp64 oracle autograd of the reference loss (train_network.py:54-55,85-89: both 'mean' over the batch), accumulated over chunks
-    of boards so that the edge-list formulation fits in memory: mean over B = sum over chunks of (chunk mean x n_chunk / B).
-    emulate_tc: the forward pass carries the tensor-core path's rounding points (gnn_oracle.forward_tc_emulation)."""
-    ref64 = copy.deepcopy(ref).double()
-    B = len(rows)
-    total = 0.0
-    for lo in range(0, B, chunk):
-        hi = min(B, lo + chunk)
-        x, ei, batch = gnn_oracle.graph_inputs_from_rows(rows[lo:hi], dtype=torch.float64)
-        p64, v64 = gnn_oracle.forward_tc_emulation(ref64, x, ei, batch) if emulate_tc else ref64(x, ei, batch)
-        loss, _, _ = gnn_oracle.training_loss(p64, v64, pt[lo:hi].double(), vt[lo:hi].double())
-        (loss * ((hi - lo) / B)).backward()
-        total += loss.item() * (hi - lo) / B
-    return total, {n: p.grad for n, p in ref64.named_parameters()}
-
-
 @pytest.mark.parametrize("B", [256, 4096])
 def test_bf16_training_gradients_at_the_benchmarked_batches(B):
     """The training step bench.py times (B = 256: BASELINE configs[0]; B = 4096: 28 boards per CTA through the double-buffered
@@ -624,8 +607,8 @@ def test_bf16_training_gradients_at_the_benchmarked_batches(B):
     torch.manual_seed(5)
     pt = torch.softmax(2 * torch.randn(B, 209), dim=1)
     vt = torch.randint(-1, 2, (B,)).float()
-    loss64, g_ref = _oracle_grads_fp64(ref, rows, pt, vt)
-    loss_em, g_em = _oracle_grads_fp64(ref, rows, pt, vt, emulate_tc=True)
+    loss64, g_ref = gnn_oracle.oracle_grads_fp64(ref, rows, pt, vt)
+    loss_em, g_em = gnn_oracle.oracle_grads_fp64(ref, rows, pt, vt, emulate_tc=True)
     flat_ref = torch.cat([g_ref[n].reshape(-1) for n in FLAT_PARAM_ORDER])
     flat_em = torch.cat([g_em[n].reshape(-1) for n in FLAT_PARAM_ORDER])
     implied = ((flat_em - flat_ref).norm() / flat_ref.norm()).item()   # what bf16 operands alone do to this batch's gradient
