@@ -14,6 +14,8 @@
 // numpy~=2.0.2, NEP 50 promotion): w accumulates in float64; the PUCT score is
 //   float32(-w/n computed in float64) + ((float32(1.25) * p) * float32(sqrt(t))) / float32(1 + n)
 // all in float32, and np.argmax takes the FIRST maximum.
+#include <cfloat>
+
 #include "aq_common.cuh"
 
 using namespace aq;
@@ -30,7 +32,7 @@ struct __align__(16) MctsCold {
     int parent;         // -1 = root
     short n_children;
     short action;       // action that leads here from the parent
-    int pad;
+    int pad;            // 0; a child of a Gumbel root: the bits of its float base score (aq_mcts_gumbel_root)
 };
 static_assert(sizeof(MctsHot) == 16 && sizeof(MctsCold) == 16, "node halves must be 16 bytes");
 constexpr size_t kNodeBytes = sizeof(MctsHot) + sizeof(MctsCold);
@@ -42,6 +44,7 @@ struct __align__(16) MctsGame {
     int leaf_kind;  // 0 = evaluate with the network, 1 = terminal loss (-1), 2 = terminal draw (0)
     int overflow;   // arena exhausted (caller error: max_nodes too small)
     int pad[4];     // pad[0] != 0: the root's priors carry Dirichlet noise (aq_mcts_root_noise); reset / advance zero it
+                    // pad[1..3]: the Gumbel root (aq_mcts_gumbel_root): the bits of v_hat (float), m (0 = no Gumbel root), n
 };
 static_assert(sizeof(MctsGame) == 64, "MctsGame must be 64 bytes");
 
@@ -171,14 +174,137 @@ mcts_advance_kernel(const MctsGame *__restrict__ src_games, const MctsHot *__res
     }
 }
 
+// ------------------------------------------------------------------------------------------
+// Gumbel root (Gumbel AlphaZero: Danihelka et al., ICLR 2022; DeepMind mctx gumbel_muzero_policy; the reference has none).  Every
+// node below the root keeps PUCT.  For a game whose root has K children with priors p_c (legal_actions() order) and
+// logit_c = log p_c (-inf for p_c = 0), aq_mcts_gumbel_root stores, once, right after simulation 1 expanded the root (root.n == 1):
+//   g_c    = gumbel_scale * (-log(-log U_c)),  U_c a splitmix64 counter draw keyed by (seed, game_id, ply) (mcts_gumbel_root_kernel)
+//   base_c = float32(g_c + (logit_c - max logit))   in the root child's MctsCold.pad
+//   v_hat  = root.w (the network value of the root), m = min(considered, K), n = sims - 1 (root-child visits of the search)
+// At every root descent and in the result, with n_c, w_c the children's visits and values and N = sum n_c:
+//   q_c    = -(w_c / n_c) for n_c > 0 (the root mover's view, as the PUCT scan reads it)
+//   v_mix  = (v_hat + N * (S_pq / S_p)) / (N + 1),  S_p = sum_{n_c>0} pt_c, S_pq = sum_{n_c>0} pt_c * q_c, pt = max(p, FLT_MIN)
+//            (S_pq / S_p taken as 0 when N = 0)
+//   cq_c   = q_c if n_c > 0 else v_mix;  qh_c = (cq_c - min cq) / max(max cq - min cq, 1e-8)
+//   sigma_c = ((50 + max_b n_b) * 0.1) * qh_c                                          (mctx maxvisit_init = 50, value_scale = 0.1)
+//   score_c = max(-1e9, base_c + sigma_c)
+//   descent at simulation index k = N: the first argmax of score_c over the children with n_c == considered_visit(m, n, k)
+//   choice: the first argmax of score_c over the children with n_c == max_b n_b;  improved policy: softmax(logit_c + sigma_c)
+// (no child matching: child 0, as jnp.argmax over all -inf).  Scores are float64 with every operation rounded as written; sums
+// run in warp order: lane l adds its children l, l + 32, ... in order from 0.0, then S_l += S_(l xor m) for m = 16, 8, 4, 2, 1.
+// tests/mcts_gumbel_oracle.py restates all of it.
+// ------------------------------------------------------------------------------------------
+
+// mctx get_sequence_of_considered_visits(m, n)[k] (sequential halving), continued past k = n - 1 by the same rule: phases of
+// `extra` rounds over the first nc children, extra = max(1, n / (ceil(log2 m) * nc)), nc halving from m down to 2.  The children a
+// phase considers have equal visit counts, so entry k of a phase is the visits before it plus k / nc.
+__device__ __forceinline__ int considered_visit(int m, int n, int k) {
+    if (m <= 1) return k;
+    const int log2max = 32 - __clz(m - 1);
+    int nc = m, base = 0;
+    while (true) {
+        const int extra = max(1, n / (log2max * nc));
+        if (k < extra * nc) return base + k / nc;
+        k -= extra * nc;
+        base += extra;
+        nc = max(2, nc / 2);
+    }
+}
+
+struct GumbelQ {
+    double v_mix, q_lo, q_range, visit_scale;
+    int max_n;
+};
+
+__device__ __forceinline__ double completed_q(const MctsHot &ch, double v_mix) { return ch.n > 0 ? -__ddiv_rn(ch.w, (double)ch.n) : v_mix; }
+
+__device__ __forceinline__ double warp_sum(double s) {
+#pragma unroll
+    for (int m = 16; m; m >>= 1) s = __dadd_rn(s, __shfl_xor_sync(0xffffffffu, s, m));
+    return s;
+}
+
+// What completes and rescales the root children's Q values (N = sum of their visits); the same in every lane.
+__device__ __forceinline__ GumbelQ gumbel_q(const MctsGame &gm, const MctsHot *hot, int first, int nc, int N, int lane) {
+    double sp = 0.0, spq = 0.0;
+    int mx = 0;
+#pragma unroll 1
+    for (int c = lane; c < nc; c += 32) {
+        const MctsHot ch = hot[first + c];
+        const double pt = ch.n > 0 ? (double)fmaxf(ch.prior, FLT_MIN) : 0.0;
+        sp = __dadd_rn(sp, pt);
+        spq = __dadd_rn(spq, ch.n > 0 ? __dmul_rn(pt, completed_q(ch, 0.0)) : 0.0);
+        mx = max(mx, ch.n);
+    }
+    sp = warp_sum(sp);
+    spq = warp_sum(spq);
+    GumbelQ r;
+    r.max_n = __reduce_max_sync(0xffffffffu, mx);
+    const double v_hat = (double)__int_as_float(gm.pad[1]);
+    r.v_mix = __ddiv_rn(__dadd_rn(v_hat, __dmul_rn((double)N, N > 0 ? __ddiv_rn(spq, sp) : 0.0)), (double)(N + 1));
+    double lo = INFINITY, hi = -INFINITY;
+#pragma unroll 1
+    for (int c = lane; c < nc; c += 32) {
+        const double q = completed_q(hot[first + c], r.v_mix);
+        lo = fmin(lo, q);
+        hi = fmax(hi, q);
+    }
+#pragma unroll
+    for (int m = 16; m; m >>= 1) {
+        lo = fmin(lo, __shfl_xor_sync(0xffffffffu, lo, m));
+        hi = fmax(hi, __shfl_xor_sync(0xffffffffu, hi, m));
+    }
+    r.q_lo = lo;
+    r.q_range = fmax(__dsub_rn(hi, lo), 1e-8);
+    r.visit_scale = __dmul_rn(__dadd_rn(50.0, (double)r.max_n), 0.1);
+    return r;
+}
+
+__device__ __forceinline__ double gumbel_sigma(const GumbelQ &r, const MctsHot &ch) {
+    return __dmul_rn(r.visit_scale, __ddiv_rn(__dsub_rn(completed_q(ch, r.v_mix), r.q_lo), r.q_range));
+}
+
+// First argmax of score_c over the root children with n_c == visits (child 0 when there is none); the same in every lane.
+__device__ __forceinline__ int gumbel_pick(const GumbelQ &r, const MctsHot *hot, const MctsCold *cold, int first, int nc, int visits, int lane) {
+    double best = -INFINITY;
+    int best_c = 0x7fffffff;
+#pragma unroll 1
+    for (int c = lane; c < nc; c += 32) {
+        const MctsHot ch = hot[first + c];
+        if (ch.n != visits) continue;
+        const double sc = fmax(-1e9, __dadd_rn((double)__int_as_float(cold[first + c].pad), gumbel_sigma(r, ch)));
+        if (sc > best || best_c == 0x7fffffff) { best = sc; best_c = c; }   // ascending c: the first maximum of the lane
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) {
+        const double ob = __shfl_xor_sync(0xffffffffu, best, d);
+        const int oc = __shfl_xor_sync(0xffffffffu, best_c, d);
+        const bool take = (oc != 0x7fffffff) && (best_c == 0x7fffffff || ob > best || (ob == best && oc < best_c));
+        if (take) { best = ob; best_c = oc; }
+    }
+    return best_c == 0x7fffffff ? 0 : best_c;
+}
+
 // Descent of game g by its warp (pv_mcts.py:69-78).  The node arrays are read through plain pointers: in the fused kernel the same
-// warp has just written them (expansion + backup), so the loads must be coherent ones.
+// warp has just written them (expansion + backup), so the loads must be coherent ones.  kGumbel: the root of a game with a Gumbel
+// root (MctsGame.pad[2] > 0) is left by the Gumbel rule, every other node by PUCT.
+template <bool kGumbel>
 __device__ __forceinline__ void select_game(MctsGame *games, const MctsHot *hot, const MctsCold *cold, int64_t g, int lane, float c_puct,
                                             AqState *leaf_states, int32_t *leaf_kind) {
     AqState s = games[g].root;
     int node = 0, kind = 0;
     // what the descent needs from a node: first_child, n_children (cold half) and n (hot half, known from the scan of its parent)
     int first = cold[0].first_child, nc = cold[0].n_children, nn = hot[0].n;
+    if (kGumbel && games[g].pad[2] > 0 && first >= 0 && nc > 0 && !terminal_flags(s)) {   // the Gumbel root's step; PUCT below it
+        const MctsGame &gm = games[g];
+        const GumbelQ r = gumbel_q(gm, hot, first, nc, nn - 1, lane);
+        node = first + gumbel_pick(r, hot, cold, first, nc, considered_visit(gm.pad[2], gm.pad[3], nn - 1), lane);
+        nn = hot[node].n;
+        const MctsCold cc = cold[node];
+        first = cc.first_child;
+        nc = cc.n_children;
+        s = state_after(s, cc.action);
+    }
     while (true) {
         const int tf = terminal_flags(s);  // pv_mcts.py:35-42: terminal test comes first
         if (tf) { kind = (tf & 1) ? 1 : 2; break; }
@@ -231,7 +357,17 @@ mcts_select_kernel(MctsGame *games, const MctsHot *hot_all, const MctsCold *cold
     const int lane = threadIdx.x & 31;
     const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (g >= G) return;
-    select_game(games, hot_all + g * max_nodes, cold_all + g * max_nodes, g, lane, c_puct, leaf_states, leaf_kind);
+    select_game<false>(games, hot_all + g * max_nodes, cold_all + g * max_nodes, g, lane, c_puct, leaf_states, leaf_kind);
+}
+
+// mcts_select_kernel with the Gumbel rule at the roots of games that have one
+__global__ void __launch_bounds__(128)
+mcts_select_gumbel_kernel(MctsGame *games, const MctsHot *hot_all, const MctsCold *cold_all, int64_t G, int64_t max_nodes, float c_puct,
+                          AqState *leaf_states, int32_t *leaf_kind) {
+    const int lane = threadIdx.x & 31;
+    const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (g >= G) return;
+    select_game<true>(games, hot_all + g * max_nodes, cold_all + g * max_nodes, g, lane, c_puct, leaf_states, leaf_kind);
 }
 
 // Expansion of the selected leaf of game g with the evaluated priors (pv_mcts.py:47-56) and the backup of its value (:60-66).
@@ -333,7 +469,22 @@ mcts_expand_select_kernel(MctsGame *games, MctsHot *hot_all, MctsCold *cold_all,
     MctsCold *cold = cold_all + g * max_nodes;
     expand_backup_game(games, hot, cold, g, lane, max_nodes, priors, values, mask, pawn);
     __syncwarp();   // orders the warp's node writes (children by all lanes, the backup by lane 0) before the descent's reads
-    select_game(games, hot, cold, g, lane, c_puct, leaf_states, leaf_kind);
+    select_game<false>(games, hot, cold, g, lane, c_puct, leaf_states, leaf_kind);
+}
+
+// mcts_expand_select_kernel with the Gumbel rule at the roots of games that have one
+__global__ void __launch_bounds__(128)
+mcts_expand_select_gumbel_kernel(MctsGame *games, MctsHot *hot_all, MctsCold *cold_all, int64_t G, int64_t max_nodes,
+                                 const float *__restrict__ priors, const float *__restrict__ values, const uint32_t *__restrict__ mask,
+                                 const uint8_t *__restrict__ pawn, float c_puct, AqState *leaf_states, int32_t *leaf_kind) {
+    const int lane = threadIdx.x & 31;
+    const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (g >= G) return;
+    MctsHot *hot = hot_all + g * max_nodes;
+    MctsCold *cold = cold_all + g * max_nodes;
+    expand_backup_game(games, hot, cold, g, lane, max_nodes, priors, values, mask, pawn);
+    __syncwarp();
+    select_game<true>(games, hot, cold, g, lane, c_puct, leaf_states, leaf_kind);
 }
 
 __global__ void mcts_root_counts_kernel(const MctsGame *__restrict__ games, const MctsHot *__restrict__ hot_all,
@@ -366,6 +517,8 @@ __global__ void mcts_root_counts_kernel(const MctsGame *__restrict__ games, cons
 //            depend on which other games are still running
 //   state  = state.next(action) (self_play.py:60), with its terminal flags.
 // One warp per game; child c of the root lives in lane c % 32, slot c / 32.
+// kChosen (aq_selfplay_advance_chosen): policy[action] = child_policy[c] and the move is child choice[g], both from the search
+// (the Gumbel root's improved policy and choice); no counts, temperature or draw.
 // ------------------------------------------------------------------------------------------
 constexpr int kChildSlots = (AQ_MAX_LEGAL + 31) / 32;
 
@@ -375,12 +528,12 @@ __device__ __forceinline__ uint64_t mix64(uint64_t z) {  // splitmix64 finaliser
     return z ^ (z >> 31);
 }
 
-template <typename T>
+template <typename T, bool kChosen>
 __global__ void __launch_bounds__(128)
 selfplay_move_kernel(const AqState *__restrict__ states, const int32_t *__restrict__ counts, const int16_t *__restrict__ actions,
                      const int16_t *__restrict__ n_children, const int64_t *__restrict__ game_id, int64_t G, double inv_t, int greedy,
-                     uint64_t seed, int ply, T *__restrict__ policy, int16_t *__restrict__ chosen, AqState *__restrict__ moved,
-                     uint8_t *__restrict__ term) {
+                     uint64_t seed, int ply, const float *__restrict__ child_policy, const int16_t *__restrict__ choice,
+                     T *__restrict__ policy, int16_t *__restrict__ chosen, AqState *__restrict__ moved, uint8_t *__restrict__ term) {
     __shared__ T rows[4][AQ_ACTIONS];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     const int64_t g = (int64_t)blockIdx.x * 4 + w;
@@ -388,47 +541,60 @@ selfplay_move_kernel(const AqState *__restrict__ states, const int32_t *__restri
     const int n = n_children[g];
     double x[kChildSlots];
     int act[kChildSlots];
-    long long best = -1;
+    int pick = -1;
+    double total = 1.0;   // kChosen: child_policy is recorded as it is
+    if constexpr (kChosen) {
 #pragma unroll
-    for (int k = 0; k < kChildSlots; ++k) {
-        const int c = lane + 32 * k;
-        const int cnt = c < n ? counts[g * AQ_MAX_LEGAL + c] : 0;
-        act[k] = c < n ? (int)actions[g * AQ_MAX_LEGAL + c] : -1;
-        x[k] = inv_t == 1.0 ? (double)cnt : (cnt > 0 ? pow((double)cnt, inv_t) : 0.0);
-        if (c < n) best = max(best, ((long long)cnt << 8) | (long long)(255 - c));   // largest count, then smallest index
-    }
-    if (greedy) {
-#pragma unroll
-        for (int d = 16; d; d >>= 1) best = max(best, __shfl_xor_sync(0xffffffffu, best, d));
-        const int arg = 255 - (int)(best & 255);
-#pragma unroll
-        for (int k = 0; k < kChildSlots; ++k) x[k] = (lane + 32 * k == arg && n > 0) ? 1.0 : 0.0;
-    }
-    // running sums in child order: a warp scan per slot on top of the slots before it (fixed order: deterministic)
-    double cum[kChildSlots], base = 0.0;
-#pragma unroll
-    for (int k = 0; k < kChildSlots; ++k) {
-        double v = x[k];
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const double up = __shfl_up_sync(0xffffffffu, v, d);
-            if (lane >= d) v += up;
+        for (int k = 0; k < kChildSlots; ++k) {
+            const int c = lane + 32 * k;
+            act[k] = c < n ? (int)actions[g * AQ_MAX_LEGAL + c] : -1;
+            x[k] = c < n ? (double)child_policy[g * AQ_MAX_LEGAL + c] : 0.0;
         }
-        cum[k] = base + v;
-        base = __shfl_sync(0xffffffffu, cum[k], 31);
-    }
-    const double total = base;
-    const uint64_t bits = mix64(mix64(seed + 0x9E3779B97F4A7C15ull * (uint64_t)(game_id[g] + 1)) + 0xD1B54A32D192ED03ull * (uint64_t)(ply + 1));
-    const double target = (double)(bits >> 11) * (1.0 / 9007199254740992.0) * total;   // u in [0, 1) times the sum
-    int pick = -1, last = -1;
+        pick = choice[g];
+        if (pick >= n) pick = -1;
+    } else {
+        long long best = -1;
 #pragma unroll
-    for (int k = 0; k < kChildSlots; ++k) {
-        const unsigned over = __ballot_sync(0xffffffffu, x[k] > 0.0 && target < cum[k]);
-        const unsigned any = __ballot_sync(0xffffffffu, x[k] > 0.0);
-        if (pick < 0 && over) pick = 32 * k + __ffs(over) - 1;
-        if (any) last = 32 * k + 31 - __clz(any);
+        for (int k = 0; k < kChildSlots; ++k) {
+            const int c = lane + 32 * k;
+            const int cnt = c < n ? counts[g * AQ_MAX_LEGAL + c] : 0;
+            act[k] = c < n ? (int)actions[g * AQ_MAX_LEGAL + c] : -1;
+            x[k] = inv_t == 1.0 ? (double)cnt : (cnt > 0 ? pow((double)cnt, inv_t) : 0.0);
+            if (c < n) best = max(best, ((long long)cnt << 8) | (long long)(255 - c));   // largest count, then smallest index
+        }
+        if (greedy) {
+#pragma unroll
+            for (int d = 16; d; d >>= 1) best = max(best, __shfl_xor_sync(0xffffffffu, best, d));
+            const int arg = 255 - (int)(best & 255);
+#pragma unroll
+            for (int k = 0; k < kChildSlots; ++k) x[k] = (lane + 32 * k == arg && n > 0) ? 1.0 : 0.0;
+        }
+        // running sums in child order: a warp scan per slot on top of the slots before it (fixed order: deterministic)
+        double cum[kChildSlots], base = 0.0;
+#pragma unroll
+        for (int k = 0; k < kChildSlots; ++k) {
+            double v = x[k];
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) {
+                const double up = __shfl_up_sync(0xffffffffu, v, d);
+                if (lane >= d) v += up;
+            }
+            cum[k] = base + v;
+            base = __shfl_sync(0xffffffffu, cum[k], 31);
+        }
+        total = base;
+        const uint64_t bits = mix64(mix64(seed + 0x9E3779B97F4A7C15ull * (uint64_t)(game_id[g] + 1)) + 0xD1B54A32D192ED03ull * (uint64_t)(ply + 1));
+        const double target = (double)(bits >> 11) * (1.0 / 9007199254740992.0) * total;   // u in [0, 1) times the sum
+        int last = -1;
+#pragma unroll
+        for (int k = 0; k < kChildSlots; ++k) {
+            const unsigned over = __ballot_sync(0xffffffffu, x[k] > 0.0 && target < cum[k]);
+            const unsigned any = __ballot_sync(0xffffffffu, x[k] > 0.0);
+            if (pick < 0 && over) pick = 32 * k + __ffs(over) - 1;
+            if (any) last = 32 * k + 31 - __clz(any);
+        }
+        if (pick < 0) pick = last;   // target == total after rounding: the last child with a positive score
     }
-    if (pick < 0) pick = last;   // target == total after rounding: the last child with a positive score
     int a = -1;
 #pragma unroll
     for (int k = 0; k < kChildSlots; ++k) {
@@ -593,6 +759,108 @@ mcts_root_noise_kernel(MctsGame *games, MctsHot *hot_all, const MctsCold *__rest
 }
 
 // ------------------------------------------------------------------------------------------
+// Gumbel root state (the rule is stated above select_game).  The Gumbel draw of child c of game g:
+//   key = mix64(mix64((seed ^ kGumbelDomain) + 0x9E3779B97F4A7C15 * (game_id + 1)) + 0xD1B54A32D192ED03 * (ply + 1))
+//   U_c = ((mix64(key + 0x9E3779B97F4A7C15 * (c + 1)) >> 11) + 0.5) * 2^-53, in (0, 1)
+// so a game's draw depends on (seed, game id, ply) alone, not on its batch, its row or padding rows.
+// ------------------------------------------------------------------------------------------
+constexpr uint64_t kGumbelDomain = 0x13198A2E03707344ull;   // the fractional digits of pi after kNoiseDomain's
+
+// One warp per game, child c in lane c % 32.  A root gets its Gumbel state when simulation 1 has expanded it and nothing has
+// visited it since (root.n == 1, so root.w is the network value) and it has none yet; any other root is left as it is.
+__global__ void __launch_bounds__(128)
+mcts_gumbel_root_kernel(MctsGame *games, const MctsHot *__restrict__ hot_all, MctsCold *cold_all, int64_t G, int64_t max_nodes,
+                        const int64_t *__restrict__ game_id, uint64_t seed, int ply, int considered, double gumbel_scale, int sims,
+                        float *__restrict__ root_scores) {
+    const int lane = threadIdx.x & 31;
+    const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (g >= G) return;
+    const MctsHot *hot = hot_all + g * max_nodes;
+    MctsCold *cold = cold_all + g * max_nodes;
+    const int first = cold[0].first_child;
+    const int nc = first < 0 ? 0 : cold[0].n_children;
+    if (nc > 0 && hot[0].n == 1 && games[g].pad[2] == 0) {
+        const uint64_t id = game_id ? (uint64_t)game_id[g] : (uint64_t)g;
+        const uint64_t key = mix64(mix64((seed ^ kGumbelDomain) + 0x9E3779B97F4A7C15ull * (id + 1)) + 0xD1B54A32D192ED03ull * (uint64_t)(ply + 1));
+        double gd[kChildSlots], lg[kChildSlots];   // g_c, logit_c
+        double mx = -INFINITY;
+#pragma unroll
+        for (int s = 0; s < kChildSlots; ++s) {
+            const int c = lane + 32 * s;
+            const double u = (double)((mix64(key + 0x9E3779B97F4A7C15ull * (uint64_t)(c + 1)) >> 11) + 0.5) * 0x1p-53;
+            gd[s] = __dmul_rn(gumbel_scale, -log(-log(u)));
+            lg[s] = c < nc ? log((double)hot[first + c].prior) : -INFINITY;
+            mx = fmax(mx, lg[s]);
+        }
+#pragma unroll
+        for (int m = 16; m; m >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, m));
+#pragma unroll
+        for (int s = 0; s < kChildSlots; ++s) {
+            const int c = lane + 32 * s;
+            if (c < nc) cold[first + c].pad = __float_as_int((float)__dadd_rn(gd[s], __dsub_rn(lg[s], mx)));
+        }
+        if (lane == 0) {
+            games[g].pad[1] = __float_as_int((float)hot[0].w);
+            games[g].pad[2] = min(considered, nc);
+            games[g].pad[3] = sims - 1;
+        }
+    }
+    if (root_scores) {
+        __syncwarp();
+        for (int c = lane; c < AQ_MAX_LEGAL; c += 32) root_scores[g * AQ_MAX_LEGAL + c] = c < nc ? __int_as_float(cold[first + c].pad) : 0.f;
+    }
+}
+
+// One warp per game: the improved policy softmax(logit + sigma) over the root's children (0 beyond them) and the choice, the first
+// argmax of the score over the most visited children.  A game without a Gumbel root: policy 0, choice -1.
+__global__ void __launch_bounds__(128)
+mcts_gumbel_result_kernel(const MctsGame *__restrict__ games, const MctsHot *__restrict__ hot_all, const MctsCold *__restrict__ cold_all,
+                          int64_t G, int64_t max_nodes, float *__restrict__ policy, int16_t *__restrict__ choice) {
+    const int lane = threadIdx.x & 31;
+    const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (g >= G) return;
+    const MctsHot *hot = hot_all + g * max_nodes;
+    const MctsCold *cold = cold_all + g * max_nodes;
+    const MctsGame &gm = games[g];
+    float *row = policy + g * AQ_MAX_LEGAL;
+    if (gm.pad[2] <= 0) {
+        for (int c = lane; c < AQ_MAX_LEGAL; c += 32) row[c] = 0.f;
+        if (lane == 0) choice[g] = -1;
+        return;
+    }
+    const int first = cold[0].first_child, nc = cold[0].n_children;
+    const GumbelQ r = gumbel_q(gm, hot, first, nc, hot[0].n - 1, lane);
+    const int pick = gumbel_pick(r, hot, cold, first, nc, r.max_n, lane);
+    double z[kChildSlots];
+    double mx = -INFINITY;
+#pragma unroll
+    for (int s = 0; s < kChildSlots; ++s) {
+        const int c = lane + 32 * s;
+        z[s] = -INFINITY;
+        if (c < nc) {
+            const MctsHot ch = hot[first + c];
+            z[s] = __dadd_rn(log((double)ch.prior), gumbel_sigma(r, ch));
+        }
+        mx = fmax(mx, z[s]);
+    }
+#pragma unroll
+    for (int m = 16; m; m >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, m));
+    double sum = 0.0;
+#pragma unroll
+    for (int s = 0; s < kChildSlots; ++s) {
+        z[s] = lane + 32 * s < nc ? exp(__dsub_rn(z[s], mx)) : 0.0;
+        sum = __dadd_rn(sum, z[s]);
+    }
+    sum = warp_sum(sum);
+#pragma unroll
+    for (int s = 0; s < kChildSlots; ++s) {
+        const int c = lane + 32 * s;
+        if (c < AQ_MAX_LEGAL) row[c] = c < nc ? (float)__ddiv_rn(z[s], sum) : 0.f;
+    }
+    if (lane == 0) choice[g] = (int16_t)pick;
+}
+
+// ------------------------------------------------------------------------------------------
 extern "C" int64_t aq_mcts_ws_bytes(int64_t G, int64_t max_nodes) {
     return (int64_t)(mcts_nodes_offset(G) + (size_t)G * (size_t)max_nodes * kNodeBytes);
 }
@@ -637,6 +905,13 @@ extern "C" int aq_mcts_select(void *ws, int64_t G, int64_t max_nodes, float c_pu
                      games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, c_puct, leaf_states, leaf_kind);
 }
 
+extern "C" int aq_mcts_select_gumbel(void *ws, int64_t G, int64_t max_nodes, float c_puct, AqState *leaf_states,
+                                     int32_t *leaf_kind, void *stream) {
+    if (G <= 0 || !ws || !leaf_states || !leaf_kind) return aq_set_error(AQ_ERR_ARG, "aq_mcts_select_gumbel");
+    return aq_launch("aq_mcts_select_gumbel", mcts_select_gumbel_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream),
+                     false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, c_puct, leaf_states, leaf_kind);
+}
+
 extern "C" int aq_mcts_expand_backup(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values,
                                      const uint32_t *mask, const uint8_t *pawn, void *stream) {
     if (G <= 0 || !ws || !priors || !values || !mask || !pawn) return aq_set_error(AQ_ERR_ARG, "aq_mcts_expand_backup");
@@ -650,6 +925,16 @@ extern "C" int aq_mcts_expand_select(void *ws, int64_t G, int64_t max_nodes, con
     return aq_launch("aq_mcts_expand_select", mcts_expand_select_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream),
                      false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, priors, values, mask, pawn, c_puct, leaf_states,
                      leaf_kind);
+}
+
+extern "C" int aq_mcts_expand_select_gumbel(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values,
+                                            const uint32_t *mask, const uint8_t *pawn, float c_puct, AqState *leaf_states, int32_t *leaf_kind,
+                                            void *stream) {
+    if (G <= 0 || !ws || !priors || !values || !mask || !pawn || !leaf_states || !leaf_kind)
+        return aq_set_error(AQ_ERR_ARG, "aq_mcts_expand_select_gumbel");
+    return aq_launch("aq_mcts_expand_select_gumbel", mcts_expand_select_gumbel_kernel, (unsigned)((G + 3) / 4), 128, 0,
+                     reinterpret_cast<cudaStream_t>(stream), false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, priors,
+                     values, mask, pawn, c_puct, leaf_states, leaf_kind);
 }
 
 extern "C" int aq_mcts_root_counts(void *ws, int64_t G, int64_t max_nodes, int32_t *counts, int16_t *actions,
@@ -673,8 +958,47 @@ extern "C" int aq_mcts_root_noise(void *ws, int64_t G, int64_t max_nodes, const 
                      (double)fraction, root_priors);
 }
 
+extern "C" int aq_mcts_gumbel_root(void *ws, int64_t G, int64_t max_nodes, const int64_t *game_id, uint64_t seed, int32_t ply,
+                                   int32_t considered, float gumbel_scale, int32_t sims, float *root_scores, void *stream) {
+    if (G < 1 || max_nodes < 1 || !ws || considered < 1 || sims < 1 || !(gumbel_scale >= 0.f) || !isfinite(gumbel_scale))
+        return aq_set_error(AQ_ERR_ARG, "aq_mcts_gumbel_root");
+    return aq_launch("aq_mcts_gumbel_root", mcts_gumbel_root_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream), false,
+                     games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, game_id, seed, (int)ply, (int)considered,
+                     (double)gumbel_scale, (int)sims, root_scores);
+}
+
+extern "C" int aq_mcts_gumbel_result(void *ws, int64_t G, int64_t max_nodes, float *policy, int16_t *choice, void *stream) {
+    if (G < 1 || max_nodes < 1 || !ws || !policy || !choice) return aq_set_error(AQ_ERR_ARG, "aq_mcts_gumbel_result");
+    return aq_launch("aq_mcts_gumbel_result", mcts_gumbel_result_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream),
+                     false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, policy, choice);
+}
+
 extern "C" int64_t aq_selfplay_ws_bytes(int64_t G) {
     return (int64_t)(((size_t)(G > 0 ? G : 0) * sizeof(AqState) + 255) & ~(size_t)255) + (G > 0 ? G : 0);
+}
+
+// The move kernel of kChosen, then the compaction of the games still running.
+template <bool kChosen>
+static int selfplay_advance(const char *what, const AqState *states, const int32_t *counts, const float *child_policy, const int16_t *choice,
+                            const int16_t *actions, const int16_t *n_children, const int64_t *game_id, int64_t G, double temperature,
+                            uint64_t seed, int32_t ply, void *policy, int policy_f64, int16_t *chosen, AqState *next_states,
+                            int64_t *next_game_id, uint8_t *final_flags, int64_t *final_plies, int32_t *alive_count, void *workspace,
+                            cudaStream_t st) {
+    AqState *moved = reinterpret_cast<AqState *>(workspace);
+    uint8_t *term = reinterpret_cast<uint8_t *>(workspace) + (((size_t)G * sizeof(AqState) + 255) & ~(size_t)255);
+    const int greedy = temperature == 0.0;
+    const double inv_t = greedy ? 1.0 : 1.0 / temperature;
+    const unsigned grid = (unsigned)((G + 3) / 4);
+    int rc;
+    if (policy_f64)
+        rc = aq_launch(what, selfplay_move_kernel<double, kChosen>, grid, 128, 0, st, false, states, counts, actions, n_children, game_id, G,
+                       inv_t, greedy, seed, ply, child_policy, choice, reinterpret_cast<double *>(policy), chosen, moved, term);
+    else
+        rc = aq_launch(what, selfplay_move_kernel<float, kChosen>, grid, 128, 0, st, false, states, counts, actions, n_children, game_id, G,
+                       inv_t, greedy, seed, ply, child_policy, choice, reinterpret_cast<float *>(policy), chosen, moved, term);
+    if (rc) return rc;
+    return aq_launch(kChosen ? "aq_selfplay_advance_chosen(compact)" : "aq_selfplay_advance(compact)", selfplay_compact_kernel, 1, 1024, 0,
+                     st, false, moved, term, game_id, G, ply, next_states, next_game_id, final_flags, final_plies, alive_count);
 }
 
 extern "C" int aq_selfplay_advance(const AqState *states, const int32_t *counts, const int16_t *actions, const int16_t *n_children,
@@ -684,20 +1008,19 @@ extern "C" int aq_selfplay_advance(const AqState *states, const int32_t *counts,
     if (G <= 0 || !states || !counts || !actions || !n_children || !game_id || !policy || !next_states || !next_game_id || !final_flags ||
         !final_plies || !alive_count || !workspace || !(temperature >= 0.0))
         return aq_set_error(AQ_ERR_ARG, "aq_selfplay_advance");
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    AqState *moved = reinterpret_cast<AqState *>(workspace);
-    uint8_t *term = reinterpret_cast<uint8_t *>(workspace) + (((size_t)G * sizeof(AqState) + 255) & ~(size_t)255);
-    const int greedy = temperature == 0.0;
-    const double inv_t = greedy ? 1.0 : 1.0 / temperature;
-    const unsigned grid = (unsigned)((G + 3) / 4);
-    int rc;
-    if (policy_f64)
-        rc = aq_launch("aq_selfplay_advance(move)", selfplay_move_kernel<double>, grid, 128, 0, st, false, states, counts, actions, n_children,
-                       game_id, G, inv_t, greedy, seed, ply, reinterpret_cast<double *>(policy), chosen, moved, term);
-    else
-        rc = aq_launch("aq_selfplay_advance(move)", selfplay_move_kernel<float>, grid, 128, 0, st, false, states, counts, actions, n_children,
-                       game_id, G, inv_t, greedy, seed, ply, reinterpret_cast<float *>(policy), chosen, moved, term);
-    if (rc) return rc;
-    return aq_launch("aq_selfplay_advance(compact)", selfplay_compact_kernel, 1, 1024, 0, st, false, moved, term, game_id, G, ply, next_states,
-                     next_game_id, final_flags, final_plies, alive_count);
+    return selfplay_advance<false>("aq_selfplay_advance(move)", states, counts, nullptr, nullptr, actions, n_children, game_id, G, temperature,
+                                   seed, ply, policy, policy_f64, chosen, next_states, next_game_id, final_flags, final_plies, alive_count,
+                                   workspace, reinterpret_cast<cudaStream_t>(stream));
+}
+
+extern "C" int aq_selfplay_advance_chosen(const AqState *states, const float *child_policy, const int16_t *choice, const int16_t *actions,
+                                          const int16_t *n_children, const int64_t *game_id, int64_t G, int32_t ply, void *policy,
+                                          int policy_f64, int16_t *chosen, AqState *next_states, int64_t *next_game_id, uint8_t *final_flags,
+                                          int64_t *final_plies, int32_t *alive_count, void *workspace, void *stream) {
+    if (G <= 0 || !states || !child_policy || !choice || !actions || !n_children || !game_id || !policy || !next_states || !next_game_id ||
+        !final_flags || !final_plies || !alive_count || !workspace)
+        return aq_set_error(AQ_ERR_ARG, "aq_selfplay_advance_chosen");
+    return selfplay_advance<true>("aq_selfplay_advance_chosen(move)", states, nullptr, child_policy, choice, actions, n_children, game_id, G,
+                                  1.0, 0, ply, policy, policy_f64, chosen, next_states, next_game_id, final_flags, final_plies, alive_count,
+                                  workspace, reinterpret_cast<cudaStream_t>(stream));
 }

@@ -9,6 +9,8 @@ Tree reuse between moves (AlphaGo Zero: the child of the played move becomes the
 statistics) is opt-in, BatchedMCTS(..., tree_reuse=True); the default keeps the reference's fresh root.
 Dirichlet noise on the root priors (AlphaZero self-play exploration) is opt-in too,
 BatchedMCTS(..., dirichlet_alpha=0.3); the default searches with the network's priors.
+So is the Gumbel root of Gumbel AlphaZero, BatchedMCTS(..., gumbel_considered=16): sequential halving over Gumbel-top-k sampled
+root children and a completed-Q improved policy; the default keeps PUCT at the root.
 """
 import math
 from copy import deepcopy
@@ -47,16 +49,34 @@ class BatchedMCTS:
     dirichlet_alpha (AlphaZero; the reference has none): each search mixes eta ~ Dirichlet(dirichlet_alpha) into its root's child
     priors, p' = (1 - noise_fraction) * p + noise_fraction * eta (aq_mcts_root_noise), once, before the first descent that reads
     them: a carried root right after it is carried, a fresh root right after simulation 1 expands it.  The draw is keyed by
-    search(..., noise_seed, game_id, ply).  None (the default) runs exactly the search without noise."""
+    search(..., noise_seed, game_id, ply).  None (the default) runs exactly the search without noise.
+
+    gumbel_considered (Gumbel AlphaZero, Danihelka et al. 2022, as mctx's gumbel_muzero_policy; the reference has none): the root
+    samples min(gumbel_considered, K) of its K children without replacement (Gumbel-top-k, Gumbel noise scaled by gumbel_scale) and
+    spreads the search's sims - 1 root-child visits over them by sequential halving; every node below the root keeps PUCT.  After
+    the search, last_policy f32[G,136] holds the improved policy softmax(logits + sigma(completed Q)) over the root's children and
+    last_choice int16[G] the child to play (aq_mcts_gumbel_root / _result, csrc/mcts.cu).  The draw is keyed by search(...,
+    noise_seed, game_id, ply).  It cannot be combined with tree_reuse (the schedule starts from a root without child visits) or with
+    dirichlet_alpha (the Gumbel draw is the root's exploration).  None (the default) runs exactly the PUCT search."""
 
     def __init__(self, evaluator, sims=None, c_puct=C_PUCT, device=None, use_graph=True, tree_reuse=False, dirichlet_alpha=None,
-                 noise_fraction=0.25):
+                 noise_fraction=0.25, gumbel_considered=None, gumbel_scale=1.0):
         if tree_reuse and not sims:
             raise ValueError("BatchedMCTS(tree_reuse=True) needs `sims` at construction: it sizes the node arena")
         if dirichlet_alpha is not None and not (math.isfinite(dirichlet_alpha) and dirichlet_alpha > 0):
             raise ValueError(f"dirichlet_alpha must be a finite number > 0 (or None), not {dirichlet_alpha!r}")
         if not 0.0 <= noise_fraction <= 1.0:
             raise ValueError(f"noise_fraction must be in [0, 1], not {noise_fraction!r}")
+        if gumbel_considered is not None:
+            if isinstance(gumbel_considered, bool) or int(gumbel_considered) != gumbel_considered or gumbel_considered < 1:
+                raise ValueError(f"gumbel_considered must be an integer >= 1 (or None), not {gumbel_considered!r}")
+            if not (math.isfinite(gumbel_scale) and gumbel_scale >= 0):
+                raise ValueError(f"gumbel_scale must be a finite number >= 0, not {gumbel_scale!r}")
+            if tree_reuse:
+                raise ValueError("gumbel_considered cannot be combined with tree_reuse: the Gumbel schedule starts from a root without "
+                                 "child visits")
+            if dirichlet_alpha is not None:
+                raise ValueError("gumbel_considered cannot be combined with dirichlet_alpha: the Gumbel draw is the root's exploration")
         self.model = evaluator if hasattr(evaluator, "flat_parameters") else None
         self.evaluator = network_evaluator(evaluator) if hasattr(evaluator, "predict_batch") else evaluator
         self.sims = sims
@@ -66,12 +86,16 @@ class BatchedMCTS:
         self.tree_reuse = bool(tree_reuse)
         self.dirichlet_alpha = None if dirichlet_alpha is None else float(dirichlet_alpha)
         self.noise_fraction = float(noise_fraction)
+        self.gumbel_considered = None if gumbel_considered is None else int(gumbel_considered)
+        self.gumbel_scale = float(gumbel_scale)
+        self.last_policy = None  # gumbel_considered: f32[G,136] improved policy of the last search, else None
+        self.last_choice = None  # gumbel_considered: int16[G] child chosen by the last search, else None
         self._ws = [None, None] if self.tree_reuse else [None]
         self._last = None     # tree_reuse: (workspace slot, G) of the previous search, the source a next search can continue
         self.last_kept = None  # tree_reuse: int32[G] nodes carried into each row by the last search (0 = fresh root), else None
         self._buf = {}
         self._graphs = {}
-        self._warm = False   # one eager simulation step has run (lazy initialisation is done)
+        self._warm = set()   # step modes (the last item of a graph key: Gumbel or not) whose lazy initialisation an eager step has done
 
     def _workspace(self, G, max_nodes, slot=0):
         L = _lib.load()
@@ -98,16 +122,19 @@ class BatchedMCTS:
             }
         return self._buf[G]
 
-    def _step(self, ws, G, max_nodes, buf, evaluate, st, steps=1):
+    def _step(self, ws, G, max_nodes, buf, evaluate, st, steps=1, gumbel=False):
         """`steps` simulations for all games: select, then `steps` leaf evaluations out = evaluate(stream) (terminal leaves are
-        evaluated too and ignored by the backup) joined by the fused expand + backup + next select, then the last expand + backup."""
+        evaluated too and ignored by the backup) joined by the fused expand + backup + next select, then the last expand + backup.
+        gumbel: the selects leave a Gumbel root by the Gumbel rule."""
         L, P = _lib.load(), _lib.ptr
-        _lib.check(L.aq_mcts_select(P(ws), G, max_nodes, self.c_puct, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_select")
+        select, expand_select = ((L.aq_mcts_select_gumbel, L.aq_mcts_expand_select_gumbel) if gumbel else
+                                 (L.aq_mcts_select, L.aq_mcts_expand_select))
+        _lib.check(select(P(ws), G, max_nodes, self.c_puct, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_select")
         for i in range(steps):
             out = evaluate(st)
             leaves = (P(ws), G, max_nodes, P(out["priors"]), P(out["value"]), P(out["mask"]), P(out["pawn"]))
             if i + 1 < steps:
-                _lib.check(L.aq_mcts_expand_select(*leaves, self.c_puct, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_expand_select")
+                _lib.check(expand_select(*leaves, self.c_puct, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_expand_select")
             else:
                 _lib.check(L.aq_mcts_expand_backup(*leaves, st), "aq_mcts_expand_backup")
 
@@ -115,11 +142,12 @@ class BatchedMCTS:
         """n simulations; step(stream, k) enqueues k of them.  With a graph key (network evaluator) and use_graph, they are replays of
         CUDA graphs captured for the key; else one eager step per simulation."""
         if self.use_graph and key is not None:
-            if not self._warm and n:
-                # the searcher's first step runs outside capture: lazy initialisation (module load, function attributes) must not
-                # happen inside one; a failure here is a real error and propagates
+            if key[-1] not in self._warm and n:
+                # the searcher's first step of a mode runs outside capture: lazy initialisation (module load, function attributes)
+                # must not happen inside one; a failure here is a real error and propagates
                 step(st, 1)
-                n, self._warm = n - 1, True
+                n = n - 1
+                self._warm.add(key[-1])
                 torch.cuda.synchronize(self.device)
             graphs = self._graphs.get(key)
             if graphs is None:
@@ -164,7 +192,7 @@ class BatchedMCTS:
         if self.tree_reuse and sims > self.sims:
             raise ValueError(f"this searcher's node arena holds {self.sims} simulations per search, not {sims}")
         if G_real == 0:
-            self.last_kept = None
+            self.last_kept = self.last_policy = self.last_choice = None
             return (torch.empty((0, gl.MAX_LEGAL), dtype=torch.int32, device=dev), torch.empty((0, gl.MAX_LEGAL), dtype=torch.int16, device=dev),
                     torch.empty((0,), dtype=torch.int16, device=dev), torch.zeros((3,), dtype=torch.int32, device=dev))
         # Self-play and the arena drop finished games, so the number of roots shrinks by a few almost every ply.  Batches above 256
@@ -205,7 +233,7 @@ class BatchedMCTS:
                 prec = PRECISIONS[self.model.precision]
                 # bf16 operand tiles, refreshed in place if the parameters changed since the last search
                 prep = self.model.prepared_weights() if prec == 1 else None
-                key = (G, max_nodes, ws.data_ptr(), flat.data_ptr(), prep.data_ptr() if prep is not None else 0, prec)
+                key = (G, max_nodes, ws.data_ptr(), flat.data_ptr(), prep.data_ptr() if prep is not None else 0, prec, False)
 
                 def evaluate(s):
                     _lib.check(L.aq_leaf_eval(P(flat), P(prep), P(buf["leaf"]), G, P(buf["priors"]), P(buf["value"]), P(buf["mask"]),
@@ -214,11 +242,24 @@ class BatchedMCTS:
             else:
                 key, evaluate = None, lambda s: self.evaluator(buf["leaf"])
             step = lambda s, k: self._step(ws, G, max_nodes, buf, evaluate, s, k)
-            if self.dirichlet_alpha is None:
-                self._simulate(sims, step, key, st)
-            else:
+            if self.dirichlet_alpha is not None or self.gumbel_considered is not None:
                 seed = (int(torch.randint(0, 2 ** 63 - 1, (1,)).item()) if noise_seed is None else int(noise_seed)) & (2 ** 64 - 1)
                 gid = None if game_id is None else pad(game_id.to(device=dev, dtype=torch.int64).reshape(G_real), 0)
+            self.last_policy = self.last_choice = None
+            if self.gumbel_considered is not None:
+                # simulation 1 expands the root, aq_mcts_gumbel_root draws its Gumbel state, the other sims - 1 descend by its rule
+                self._simulate(1, step, key, st)
+                _lib.check(L.aq_mcts_gumbel_root(P(ws), G, max_nodes, P(gid), seed, int(ply), self.gumbel_considered, self.gumbel_scale,
+                                                 sims, None, st), "aq_mcts_gumbel_root")
+                gstep = lambda s, k: self._step(ws, G, max_nodes, buf, evaluate, s, k, gumbel=True)
+                self._simulate(sims - 1, gstep, None if key is None else key[:-1] + (True,), st)
+                policy = torch.empty((G, gl.MAX_LEGAL), dtype=torch.float32, device=dev)
+                choice = torch.empty((G,), dtype=torch.int16, device=dev)
+                _lib.check(L.aq_mcts_gumbel_result(P(ws), G, max_nodes, P(policy), P(choice), st), "aq_mcts_gumbel_result")
+                self.last_policy, self.last_choice = policy[:G_real], choice[:G_real]
+            elif self.dirichlet_alpha is None:
+                self._simulate(sims, step, key, st)
+            else:
                 # aq_mcts_root_noise skips a root that is unexpanded or noised already, so noising before and after simulation 1 is the
                 # whole rule: the first call noises a carried root, the second a fresh root, which simulation 1 expanded
                 for n in (1, sims - 1):
@@ -274,17 +315,20 @@ class _SearcherCache(dict):
         return (_SearcherCache, ())
 
 
-def searcher_for(evaluator, sims, device=None, tree_reuse=False, dirichlet_alpha=None, noise_fraction=0.25):
+def searcher_for(evaluator, sims, device=None, tree_reuse=False, dirichlet_alpha=None, noise_fraction=0.25, gumbel_considered=None,
+                 gumbel_scale=1.0):
     """The BatchedMCTS of a network for `sims` simulations, kept on the network object: its node arenas (3.5 GB at 4,096 games x
     200 simulations), leaf buffers and captured graphs are reused by every later self-play / arena / policy call on that network
     instead of being allocated and captured again.  Evaluators that are plain callables get a fresh searcher."""
     dev = gl._dev(device)
-    opts = dict(tree_reuse=tree_reuse, dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction)
+    opts = dict(tree_reuse=tree_reuse, dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction, gumbel_considered=gumbel_considered,
+                gumbel_scale=gumbel_scale)
     if not hasattr(evaluator, "flat_parameters"):
         return BatchedMCTS(evaluator, sims, device=dev, **opts)
     cache = evaluator.__dict__.setdefault("_searchers", _SearcherCache())
     key = (int(sims), str(dev), bool(tree_reuse), None if dirichlet_alpha is None else float(dirichlet_alpha),
-           None if dirichlet_alpha is None else float(noise_fraction))
+           None if dirichlet_alpha is None else float(noise_fraction), None if gumbel_considered is None else int(gumbel_considered),
+           None if gumbel_considered is None else float(gumbel_scale))
     if key not in cache:
         if len(cache) >= 4:
             cache.clear()

@@ -42,7 +42,8 @@ def write_data(history, directory='./data/'):
 
 @torch.no_grad()
 def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_TEMPERATURE, seed=None, max_plies=None,
-                      policy_dtype=torch.float64, tree_reuse=False, dirichlet_alpha=None, noise_fraction=0.25):
+                      policy_dtype=torch.float64, tree_reuse=False, dirichlet_alpha=None, noise_fraction=0.25, gumbel_considered=None,
+                      gumbel_scale=1.0):
     """Execute `num_games` self-play games in lock-step (self_play.py:40-68 per game) and keep the record on the device:
     dict(states uint8[T,32] packed, policy [T,209] search policies over all actions (self_play.py:51-54), value f32[T]
     back-filled game results seen from the player to move (self_play.py:63-66), game int64[T], ply int64[T],
@@ -59,14 +60,20 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
 
     dirichlet_alpha (AlphaZero; the reference has none): every search mixes Dirichlet(dirichlet_alpha) noise into its root priors
     with weight noise_fraction (BatchedMCTS), drawn from (seed, game, ply) like the moves, so a game still does not depend on the
-    other games of the batch and a seed reproduces the run.  The record is the same as without noise."""
+    other games of the batch and a seed reproduces the run.  The record is the same as without noise.
+
+    gumbel_considered (Gumbel AlphaZero; the reference has none): every search uses the Gumbel root of BatchedMCTS, its draw keyed
+    by (seed, game, ply), and the ply calls aq_selfplay_advance_chosen: the recorded policy is the search's improved policy
+    softmax(logits + sigma(completed Q)) and the move is the search's choice.  `temperature` is not used then.  The record format
+    and the value targets are the same."""
     if policy_dtype not in (torch.float64, torch.float32):
         raise ValueError("policy_dtype must be torch.float64 or torch.float32")
     dev = gl._dev(device)
     L, P = _lib.load(), _lib.ptr
     seed = (int(seed) if seed is not None else int(torch.seed())) & (2 ** 64 - 1)
     sims = sims or pv_mcts.PV_EVALUATE_COUNT
-    mcts = pv_mcts.searcher_for(model, sims, dev, tree_reuse=tree_reuse, dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction)
+    mcts = pv_mcts.searcher_for(model, sims, dev, tree_reuse=tree_reuse, dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction,
+                                gumbel_considered=gumbel_considered, gumbel_scale=gumbel_scale)
     states = start_states(num_games, dev)
     game_id = torch.arange(num_games, device=dev)
     rec_state, rec_policy, rec_game, sizes = [], [], [], []
@@ -85,9 +92,15 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
             nxt = torch.empty_like(states)
             nxt_id = torch.empty_like(game_id)
             chosen = torch.empty((G,), dtype=torch.int16, device=dev) if tree_reuse else None
-            _lib.check(L.aq_selfplay_advance(P(states), P(counts), P(actions), P(n), P(game_id), G, float(temperature), seed, ply,
-                                             P(dense), int(policy_dtype == torch.float64), P(chosen), P(nxt), P(nxt_id), P(final_flags),
-                                             P(final_plies), P(alive), P(ws), _lib.stream_ptr(dev)), "aq_selfplay_advance")
+            if gumbel_considered is None:
+                _lib.check(L.aq_selfplay_advance(P(states), P(counts), P(actions), P(n), P(game_id), G, float(temperature), seed, ply,
+                                                 P(dense), int(policy_dtype == torch.float64), P(chosen), P(nxt), P(nxt_id), P(final_flags),
+                                                 P(final_plies), P(alive), P(ws), _lib.stream_ptr(dev)), "aq_selfplay_advance")
+            else:
+                _lib.check(L.aq_selfplay_advance_chosen(P(states), P(mcts.last_policy), P(mcts.last_choice), P(actions), P(n), P(game_id), G,
+                                                        ply, P(dense), int(policy_dtype == torch.float64), P(chosen), P(nxt), P(nxt_id),
+                                                        P(final_flags), P(final_plies), P(alive), P(ws), _lib.stream_ptr(dev)),
+                           "aq_selfplay_advance_chosen")
             parts = [status, alive]
             if mcts.last_kept is not None:
                 parts.append((mcts.last_kept > 0).sum(dtype=torch.int32).reshape(1))
@@ -122,11 +135,12 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
 
 
 def play_batch(model, num_games, device=None, sims=None, temperature=SP_TEMPERATURE, seed=None, max_plies=None, tree_reuse=False,
-               dirichlet_alpha=None, noise_fraction=0.25):
+               dirichlet_alpha=None, noise_fraction=0.25, gumbel_considered=None, gumbel_scale=1.0):
     """play_batch_device + conversion to the reference's history: a list of [[player, enemy, walls], policy (209 floats), value]
     (self_play.py:51-54, 63-66), games in order, plies in order within a game.  Returns (history, dict with per-game results)."""
     rec = play_batch_device(model, num_games, device, sims, temperature, seed, max_plies, tree_reuse=tree_reuse,
-                            dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction)
+                            dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction, gumbel_considered=gumbel_considered,
+                            gumbel_scale=gumbel_scale)
     rows, _ = gl.unpack_rows(rec["states"])
     rows = rows.cpu().numpy()
     pols = rec["policy"].cpu().numpy()
@@ -147,17 +161,18 @@ def play(model, device=None):
 
 
 def self_play(game_count=None, model_path=None, data_dir='./data/', rank=0, world_size=1, sims=None, seed=None, tree_reuse=False,
-              dirichlet_alpha=None, noise_fraction=0.25):
+              dirichlet_alpha=None, noise_fraction=0.25, gumbel_considered=None, gumbel_scale=1.0):
     """Perform self-play games and save the training data (self_play.py:71-98).  With
     world_size > 1 each rank plays its share of the games on its own GPU and rank 0 writes the file.
-    tree_reuse=True keeps each game's search tree between moves; dirichlet_alpha adds AlphaZero root noise to every search
-    (see play_batch_device)."""
+    tree_reuse=True keeps each game's search tree between moves; dirichlet_alpha adds AlphaZero root noise to every search;
+    gumbel_considered searches with the Gumbel AlphaZero root and records its improved policy (see play_batch_device)."""
     game_count = SP_GAME_COUNT if game_count is None else game_count
     model = GNNNetwork()
     model.prep_for_inference(model_path=model_path or (PV_NETWORK_PATH + 'best.pth'))
     mine = game_count // world_size + (1 if rank < game_count % world_size else 0)
     history, _ = play_batch(model, mine, sims=sims, seed=None if seed is None else seed + rank, tree_reuse=tree_reuse,
-                            dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction) if mine else ([], None)
+                            dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction, gumbel_considered=gumbel_considered,
+                            gumbel_scale=gumbel_scale) if mine else ([], None)
     if world_size > 1:
         import torch.distributed as dist
         gathered = [None] * world_size if rank == 0 else None

@@ -53,7 +53,7 @@ typedef struct AqState {
     uint64_t reserved; /* reserved, 0 */
 } AqState;
 
-#define AQ_VERSION 207 /* bumped with every change of a signature below; the ctypes loader refuses a library of another version */
+#define AQ_VERSION 208 /* bumped with every change of a signature below; the ctypes loader refuses a library of another version */
 int aq_version(void);
 const char *aq_last_error_string(void);
 /* Number of kernels this library has launched in the process so far (monotonic; kernels replayed through a CUDA graph the caller
@@ -278,6 +278,31 @@ int aq_mcts_expand_backup(void *ws, int64_t G, int64_t max_nodes, const float *p
  * descent depends only on that game's own backup). */
 int aq_mcts_expand_select(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values, const uint32_t *mask,
                           const uint8_t *pawn, float c_puct, AqState *leaf_states, int32_t *leaf_kind, void *stream);
+/* Gumbel root (Gumbel AlphaZero, Danihelka et al. 2022, as DeepMind's mctx gumbel_muzero_policy; the reference has none): the
+ * root's children are sampled without replacement by Gumbel-top-k and the simulations spread over them by sequential halving; every
+ * node below the root keeps PUCT.  A Gumbel search runs aq_mcts_reset, simulation 1, aq_mcts_gumbel_root, sims - 1 simulations with
+ * aq_mcts_select_gumbel / aq_mcts_expand_select_gumbel in place of aq_mcts_select / aq_mcts_expand_select, then
+ * aq_mcts_gumbel_result.
+ * aq_mcts_gumbel_root gives every root that simulation 1 has expanded and nothing has visited since (root n == 1) and that has
+ * no Gumbel state yet its state: per child c of the K children, base_c = float32(g_c + (log p_c - max log p)) with
+ * g_c = gumbel_scale * (-log(-log U_c)), U_c in (0, 1) a counter-based draw (splitmix64, keyed by (seed, game_id[g], ply) with its
+ * own domain constant: independent of the batch, the row and padding rows); v_hat = the root's value; m = min(considered, K);
+ * n = sims - 1 root-child visits.  Calling it again is a no-op for a root that has its state.
+ *   game_id [G] int64 (NULL: the row index); root_scores [G,136] f32 (may be NULL): base_c after the call, 0 beyond n_children.
+ *   AQ_ERR_ARG for G < 1, a null ws, considered < 1, sims < 1, gumbel_scale < 0 or not finite.
+ * The _gumbel select / expand-select leave a root with Gumbel state by the child with the largest max(-1e9, base_c + sigma_c)
+ * among those with n_c == considered_visit(m, n, sum of the children's n): mctx's sequential-halving table; sigma_c is mctx's
+ * completed-Q transform (mixed value of v_hat and the visited children's Q, min-max rescaled, times (50 + max n) * 0.1).
+ * csrc/mcts.cu states the rule and its float64 rounding exactly.  Roots without Gumbel state, and all other nodes, use PUCT.
+ * aq_mcts_gumbel_result: policy [G,136] f32 = softmax(log p_c + sigma_c) over the root's children (legal_actions() order, 0 beyond);
+ * choice [G] int16 = the child with the largest score among the most visited ones.  Roots without Gumbel state: 0 and -1. */
+int aq_mcts_gumbel_root(void *ws, int64_t G, int64_t max_nodes, const int64_t *game_id, uint64_t seed, int32_t ply, int32_t considered,
+                        float gumbel_scale, int32_t sims, float *root_scores, void *stream);
+int aq_mcts_select_gumbel(void *ws, int64_t G, int64_t max_nodes, float c_puct, AqState *leaf_states, int32_t *leaf_kind,
+                          void *stream);
+int aq_mcts_expand_select_gumbel(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values, const uint32_t *mask,
+                                 const uint8_t *pawn, float c_puct, AqState *leaf_states, int32_t *leaf_kind, void *stream);
+int aq_mcts_gumbel_result(void *ws, int64_t G, int64_t max_nodes, float *policy /*[G,136]*/, int16_t *choice /*[G]*/, void *stream);
 int aq_mcts_root_counts(void *ws, int64_t G, int64_t max_nodes, int32_t *counts /*[G,136]*/,
                         int16_t *actions /*[G,136]*/, int16_t *n_children /*[G]*/, int32_t *overflow, void *stream);
 /* Dirichlet noise on the priors of every expanded, not yet noised root (AlphaZero; the reference has none).
@@ -313,6 +338,13 @@ int aq_selfplay_advance(const AqState *states, const int32_t *counts, const int1
                         const int64_t *game_id, int64_t G, double temperature, uint64_t seed, int32_t ply, void *policy,
                         int policy_f64, int16_t *chosen, AqState *next_states, int64_t *next_game_id, uint8_t *final_flags,
                         int64_t *final_plies, int32_t *alive_count, void *workspace, void *stream);
+/* aq_selfplay_advance with the policy and the move from the search (a Gumbel root: aq_mcts_gumbel_result) instead of counts,
+ * temperature and a draw: policy[g, actions[g, c]] = child_policy[g, c] for c < n_children[g], 0 for the other actions; the move is
+ * child choice[g] (out of range: the game cannot move and ends as a draw).  Everything else as aq_selfplay_advance. */
+int aq_selfplay_advance_chosen(const AqState *states, const float *child_policy /*[G,136]*/, const int16_t *choice /*[G]*/,
+                               const int16_t *actions, const int16_t *n_children, const int64_t *game_id, int64_t G, int32_t ply,
+                               void *policy, int policy_f64, int16_t *chosen, AqState *next_states, int64_t *next_game_id,
+                               uint8_t *final_flags, int64_t *final_plies, int32_t *alive_count, void *workspace, void *stream);
 
 /* agents.heuristic_eval (agents.py:22-54) for B states: shortest pawn-path lengths to the goal row for the mover
  * and for the enemy (shortest_path_bfs, agents.py:27-41, with the jump rules of legal_actions_pos; -1 = no path).
