@@ -9,7 +9,7 @@ import torch
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG, "libaqgnn.so")
-ABI_VERSION = 208 # AQ_VERSION of include/aqgnn.h this table of signatures was written for
+ABI_VERSION = 209 # AQ_VERSION of include/aqgnn.h this table of signatures was written for
 
 # name -> (restype, argtypes); must list every symbol declared in include/aqgnn.h
 _vp, _i64, _i32, _f32 = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_float
@@ -70,10 +70,13 @@ SYMBOLS = {
     "aq_mcts_expand_select_gumbel": (_i32, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _f32, _vp, _vp, _vp]),
     "aq_mcts_gumbel_result": (_i32, [_vp, _i64, _i64, _vp, _vp, _vp]),
     "aq_mcts_root_counts": (_i32, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "aq_mcts_root_values": (_i32, [_vp, _i64, _i64, _vp, _vp, _vp, _vp]),
     "aq_mcts_root_noise": (_i32, [_vp, _i64, _i64, _vp, _u64, _i32, _f32, _f32, _vp, _vp]),
     "aq_selfplay_ws_bytes": (_i64, [_i64]),
     "aq_selfplay_advance": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _f64, _u64, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "aq_selfplay_advance_chosen": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "aq_selfplay_advance_resign": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _f64, _u64, _i32, _vp, _i32, _vp, _vp, _vp, _f64, _f64,
+                                          _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "aq_shortest_paths": (_i32, [_vp, _i64, _vp, _vp, _vp, _vp]),
     "aq_negamax_backup": (_i32, [_vp, _vp, _i64, _vp, _vp, _vp, _vp]),
 }

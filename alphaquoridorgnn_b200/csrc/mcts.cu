@@ -508,6 +508,38 @@ __global__ void mcts_root_counts_kernel(const MctsGame *__restrict__ games, cons
     }
 }
 
+// One warp per game, child c in lane c % 32 (as mcts_root_counts_kernel), every value in double as written:
+//   root_value = w_root / n_root (the root mover's view; NaN if n_root == 0)
+//   best_child = the child with the largest n, the first in legal_actions() order on ties (policy_from_counts(counts, 0)); -1 if none
+//   best_q     = -(w_b / n_b) (the root mover's view); -inf if there is no child or n_b == 0
+__global__ void __launch_bounds__(128)
+mcts_root_values_kernel(const MctsHot *__restrict__ hot_all, const MctsCold *__restrict__ cold_all, int64_t G, int64_t max_nodes,
+                        double *__restrict__ root_value, double *__restrict__ best_q, int16_t *__restrict__ best_child) {
+    const int lane = threadIdx.x & 31;
+    const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (g >= G) return;
+    const MctsHot *hot = hot_all + g * max_nodes;
+    const MctsCold *cold = cold_all + g * max_nodes;
+    const int first = cold[0].first_child;
+    const int nc = first < 0 ? 0 : cold[0].n_children;
+    long long best = -1;
+    for (int c = lane; c < nc; c += 32) best = max(best, ((long long)hot[first + c].n << 8) | (long long)(255 - c));   // largest n, then smallest c
+#pragma unroll
+    for (int d = 16; d; d >>= 1) best = max(best, __shfl_xor_sync(0xffffffffu, best, d));
+    if (lane == 0) {
+        const MctsHot r = hot[0];
+        root_value[g] = r.n > 0 ? __ddiv_rn(r.w, (double)r.n) : (double)NAN;
+        const int b = best < 0 ? -1 : 255 - (int)(best & 255);
+        double q = -INFINITY;
+        if (b >= 0) {
+            const MctsHot ch = hot[first + b];
+            if (ch.n > 0) q = -__ddiv_rn(ch.w, (double)ch.n);
+        }
+        best_q[g] = q;
+        best_child[g] = (int16_t)b;
+    }
+}
+
 // ------------------------------------------------------------------------------------------
 // One ply of G lock-step self-play games after their searches (reference self_play.py:47-60): for every game
 //   scores = counts ** (1 / temperature) / sum  (pv_mcts.py:88-95; temperature 0 = one-hot on the FIRST maximum, np.argmax)
@@ -528,14 +560,29 @@ __device__ __forceinline__ uint64_t mix64(uint64_t z) {  // splitmix64 finaliser
     return z ^ (z >> 31);
 }
 
-template <typename T, bool kChosen>
-__global__ void __launch_bounds__(128)
-selfplay_move_kernel(const AqState *__restrict__ states, const int32_t *__restrict__ counts, const int16_t *__restrict__ actions,
-                     const int16_t *__restrict__ n_children, const int64_t *__restrict__ game_id, int64_t G, double inv_t, int greedy,
-                     uint64_t seed, int ply, const float *__restrict__ child_policy, const int16_t *__restrict__ choice,
-                     T *__restrict__ policy, int16_t *__restrict__ chosen, AqState *__restrict__ moved, uint8_t *__restrict__ term) {
+// kResign (aq_selfplay_advance_resign): s = max(root_value[g], best_q[g]) (NaN if either is); resign_min[game_id, ply & 1] takes
+// min(., s) for every game (a NaN s leaves it); a game that is not a calibration game (resign_draw(seed, game_id) < calibration)
+// and has s < v_resign resigns: its policy row is written as ever, no move is played and its term flags are 1 | 4.
+// is_calibration[game_id] records the calibration bit the kernel used, so callers need not restate the draw.
+constexpr uint64_t kResignDomain = 0xA4093822299F31D0ull;   // the fractional digits of pi after kGumbelDomain's
+
+// u in [0, 1) of game `id`: the same for every ply of the game, so a game is a calibration game for its whole length
+__device__ __forceinline__ double resign_draw(uint64_t seed, int64_t id) {
+    return (double)(mix64(mix64((seed ^ kResignDomain) + 0x9E3779B97F4A7C15ull * (uint64_t)(id + 1))) >> 11) * 0x1p-53;
+}
+
+// The move kernels share this body; selfplay_move_kernel<T, kChosen> instantiates it without kResign, so its code is what it was
+// before resignation existed.  tid is the kernel's threadIdx.x: read there, the compiler knows its range from __launch_bounds__.
+template <typename T, bool kChosen, bool kResign>
+__device__ __forceinline__ void
+selfplay_move(unsigned tid, const AqState *__restrict__ states, const int32_t *__restrict__ counts, const int16_t *__restrict__ actions,
+              const int16_t *__restrict__ n_children, const int64_t *__restrict__ game_id, int64_t G, double inv_t, int greedy,
+              uint64_t seed, int ply, const float *__restrict__ child_policy, const int16_t *__restrict__ choice,
+              T *__restrict__ policy, int16_t *__restrict__ chosen, AqState *__restrict__ moved, uint8_t *__restrict__ term,
+              const double *__restrict__ root_value, const double *__restrict__ best_q, double v_resign, double calibration,
+              double *__restrict__ resign_min, uint8_t *__restrict__ is_calibration) {
     __shared__ T rows[4][AQ_ACTIONS];
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int lane = tid & 31, w = tid >> 5;
     const int64_t g = (int64_t)blockIdx.x * 4 + w;
     if (g >= G) return;
     const int n = n_children[g];
@@ -613,7 +660,21 @@ selfplay_move_kernel(const AqState *__restrict__ states, const int32_t *__restri
     if (lane == 0) {
         AqState t = load_state(states + g);
         int flags = 2;   // a root without children cannot move: reported as a draw (does not happen for non-terminal roots)
-        if (pick >= 0) {
+        bool resigned = false;
+        if constexpr (kResign) {
+            const int64_t id = game_id[g];
+            const double rv = root_value[g], bq = best_q[g];
+            const double s = (isnan(rv) || isnan(bq)) ? (double)NAN : fmax(rv, bq);
+            double *m = resign_min + 2 * id + (ply & 1);
+            *m = fmin(*m, s);
+            const bool cal = resign_draw(seed, id) < calibration;
+            is_calibration[id] = (uint8_t)cal;
+            resigned = !cal && s < v_resign;
+        }
+        if (resigned) {
+            flags = 1 | 4;
+            a = -1;
+        } else if (pick >= 0) {
             t = state_after(t, a);
             flags = terminal_flags(t);
         }
@@ -623,12 +684,37 @@ selfplay_move_kernel(const AqState *__restrict__ states, const int32_t *__restri
     }
 }
 
+template <typename T, bool kChosen>
+__global__ void __launch_bounds__(128)
+selfplay_move_kernel(const AqState *__restrict__ states, const int32_t *__restrict__ counts, const int16_t *__restrict__ actions,
+                     const int16_t *__restrict__ n_children, const int64_t *__restrict__ game_id, int64_t G, double inv_t, int greedy,
+                     uint64_t seed, int ply, const float *__restrict__ child_policy, const int16_t *__restrict__ choice,
+                     T *__restrict__ policy, int16_t *__restrict__ chosen, AqState *__restrict__ moved, uint8_t *__restrict__ term) {
+    selfplay_move<T, kChosen, false>(threadIdx.x, states, counts, actions, n_children, game_id, G, inv_t, greedy, seed, ply, child_policy, choice, policy,
+                                     chosen, moved, term, nullptr, nullptr, 0.0, 0.0, nullptr, nullptr);
+}
+
+template <typename T, bool kChosen>
+__global__ void __launch_bounds__(128)
+selfplay_move_resign_kernel(const AqState *__restrict__ states, const int32_t *__restrict__ counts, const int16_t *__restrict__ actions,
+                            const int16_t *__restrict__ n_children, const int64_t *__restrict__ game_id, int64_t G, double inv_t, int greedy,
+                            uint64_t seed, int ply, const float *__restrict__ child_policy, const int16_t *__restrict__ choice,
+                            T *__restrict__ policy, int16_t *__restrict__ chosen, AqState *__restrict__ moved, uint8_t *__restrict__ term,
+                            const double *__restrict__ root_value, const double *__restrict__ best_q, double v_resign, double calibration,
+                            double *__restrict__ resign_min, uint8_t *__restrict__ is_calibration) {
+    selfplay_move<T, kChosen, true>(threadIdx.x, states, counts, actions, n_children, game_id, G, inv_t, greedy, seed, ply, child_policy, choice, policy,
+                                    chosen, moved, term, root_value, best_q, v_resign, calibration, resign_min,
+                                    is_calibration);
+}
+
 // Survivors keep their order (games that ended leave; self_play.py:45 `while not state.is_done()`); one CTA, a block scan per
-// 1,024 games.  For a game that ended: final_flags[game] = terminal flags of its last state, final_plies[game] = its length.
-__global__ void __launch_bounds__(1024)
-selfplay_compact_kernel(const AqState *__restrict__ moved, const uint8_t *__restrict__ term, const int64_t *__restrict__ game_id,
-                        int64_t G, int ply, AqState *__restrict__ next_states, int64_t *__restrict__ next_game_id,
-                        uint8_t *__restrict__ final_flags, int64_t *__restrict__ final_plies, int32_t *__restrict__ alive_count) {
+// 1,024 games.  For a game that ended: final_flags[game] = terminal flags of its last state, final_plies[game] = its length
+// (kResign: a resigned game, term bit 2, played `ply` moves).
+template <bool kResign>
+__device__ __forceinline__ void
+selfplay_compact(const AqState *__restrict__ moved, const uint8_t *__restrict__ term, const int64_t *__restrict__ game_id,
+                 int64_t G, int ply, AqState *__restrict__ next_states, int64_t *__restrict__ next_game_id,
+                 uint8_t *__restrict__ final_flags, int64_t *__restrict__ final_plies, int32_t *__restrict__ alive_count) {
     __shared__ int warp_total[32];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     int base = 0;
@@ -653,13 +739,27 @@ selfplay_compact_kernel(const AqState *__restrict__ moved, const uint8_t *__rest
                 next_game_id[o] = id;
             } else {
                 final_flags[id] = (uint8_t)flags;
-                final_plies[id] = ply + 1;
+                final_plies[id] = (kResign && (flags & 4)) ? ply : ply + 1;
             }
         }
         base += all;
         __syncthreads();
     }
     if (threadIdx.x == 0) *alive_count = base;
+}
+
+__global__ void __launch_bounds__(1024)
+selfplay_compact_kernel(const AqState *__restrict__ moved, const uint8_t *__restrict__ term, const int64_t *__restrict__ game_id,
+                        int64_t G, int ply, AqState *__restrict__ next_states, int64_t *__restrict__ next_game_id,
+                        uint8_t *__restrict__ final_flags, int64_t *__restrict__ final_plies, int32_t *__restrict__ alive_count) {
+    selfplay_compact<false>(moved, term, game_id, G, ply, next_states, next_game_id, final_flags, final_plies, alive_count);
+}
+
+__global__ void __launch_bounds__(1024)
+selfplay_compact_resign_kernel(const AqState *__restrict__ moved, const uint8_t *__restrict__ term, const int64_t *__restrict__ game_id,
+                               int64_t G, int ply, AqState *__restrict__ next_states, int64_t *__restrict__ next_game_id,
+                               uint8_t *__restrict__ final_flags, int64_t *__restrict__ final_plies, int32_t *__restrict__ alive_count) {
+    selfplay_compact<true>(moved, term, game_id, G, ply, next_states, next_game_id, final_flags, final_plies, alive_count);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -949,6 +1049,13 @@ extern "C" int aq_mcts_root_counts(void *ws, int64_t G, int64_t max_nodes, int32
                      cold_of(ws, G, max_nodes), G, max_nodes, counts, actions, n_children, overflow);
 }
 
+extern "C" int aq_mcts_root_values(void *ws, int64_t G, int64_t max_nodes, double *root_value, double *best_q, int16_t *best_child,
+                                   void *stream) {
+    if (G <= 0 || max_nodes < 1 || !ws || !root_value || !best_q || !best_child) return aq_set_error(AQ_ERR_ARG, "aq_mcts_root_values");
+    return aq_launch("aq_mcts_root_values", mcts_root_values_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream),
+                     false, hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, root_value, best_q, best_child);
+}
+
 extern "C" int aq_mcts_root_noise(void *ws, int64_t G, int64_t max_nodes, const int64_t *game_id, uint64_t seed, int32_t ply, float alpha,
                                   float fraction, float *root_priors, void *stream) {
     if (G < 1 || max_nodes < 1 || !ws || !(alpha > 0.f) || !isfinite(alpha) || !(fraction >= 0.f && fraction <= 1.f))
@@ -977,28 +1084,46 @@ extern "C" int64_t aq_selfplay_ws_bytes(int64_t G) {
     return (int64_t)(((size_t)(G > 0 ? G : 0) * sizeof(AqState) + 255) & ~(size_t)255) + (G > 0 ? G : 0);
 }
 
-// The move kernel of kChosen, then the compaction of the games still running.
-template <bool kChosen>
-static int selfplay_advance(const char *what, const AqState *states, const int32_t *counts, const float *child_policy, const int16_t *choice,
-                            const int16_t *actions, const int16_t *n_children, const int64_t *game_id, int64_t G, double temperature,
-                            uint64_t seed, int32_t ply, void *policy, int policy_f64, int16_t *chosen, AqState *next_states,
-                            int64_t *next_game_id, uint8_t *final_flags, int64_t *final_plies, int32_t *alive_count, void *workspace,
-                            cudaStream_t st) {
+// What the resigning ply reads and writes besides the move (aq_selfplay_advance_resign).
+struct ResignArgs {
+    const double *root_value, *best_q;
+    double v_resign, calibration;
+    double *resign_min;
+    uint8_t *is_calibration;
+};
+
+template <typename T, bool kChosen, bool kResign>
+static int launch_move(const char *what, unsigned grid, cudaStream_t st, const AqState *states, const int32_t *counts, const int16_t *actions,
+                       const int16_t *n_children, const int64_t *game_id, int64_t G, double inv_t, int greedy, uint64_t seed, int32_t ply,
+                       const float *child_policy, const int16_t *choice, void *policy, int16_t *chosen, AqState *moved, uint8_t *term,
+                       const ResignArgs &r) {
+    if constexpr (kResign)
+        return aq_launch(what, selfplay_move_resign_kernel<T, kChosen>, grid, 128, 0, st, false, states, counts, actions, n_children, game_id,
+                         G, inv_t, greedy, seed, (int)ply, child_policy, choice, reinterpret_cast<T *>(policy), chosen, moved, term, r.root_value,
+                         r.best_q, r.v_resign, r.calibration, r.resign_min, r.is_calibration);
+    else
+        return aq_launch(what, selfplay_move_kernel<T, kChosen>, grid, 128, 0, st, false, states, counts, actions, n_children, game_id, G,
+                         inv_t, greedy, seed, (int)ply, child_policy, choice, reinterpret_cast<T *>(policy), chosen, moved, term);
+}
+
+// The move kernel of kChosen (and kResign), then the compaction of the games still running.
+template <bool kChosen, bool kResign>
+static int selfplay_advance(const char *what, const char *compact_what, const AqState *states, const int32_t *counts, const float *child_policy,
+                            const int16_t *choice, const int16_t *actions, const int16_t *n_children, const int64_t *game_id, int64_t G,
+                            double temperature, uint64_t seed, int32_t ply, void *policy, int policy_f64, int16_t *chosen, const ResignArgs &r,
+                            AqState *next_states, int64_t *next_game_id, uint8_t *final_flags, int64_t *final_plies, int32_t *alive_count,
+                            void *workspace, cudaStream_t st) {
     AqState *moved = reinterpret_cast<AqState *>(workspace);
     uint8_t *term = reinterpret_cast<uint8_t *>(workspace) + (((size_t)G * sizeof(AqState) + 255) & ~(size_t)255);
     const int greedy = temperature == 0.0;
     const double inv_t = greedy ? 1.0 : 1.0 / temperature;
     const unsigned grid = (unsigned)((G + 3) / 4);
-    int rc;
-    if (policy_f64)
-        rc = aq_launch(what, selfplay_move_kernel<double, kChosen>, grid, 128, 0, st, false, states, counts, actions, n_children, game_id, G,
-                       inv_t, greedy, seed, ply, child_policy, choice, reinterpret_cast<double *>(policy), chosen, moved, term);
-    else
-        rc = aq_launch(what, selfplay_move_kernel<float, kChosen>, grid, 128, 0, st, false, states, counts, actions, n_children, game_id, G,
-                       inv_t, greedy, seed, ply, child_policy, choice, reinterpret_cast<float *>(policy), chosen, moved, term);
+    const int rc = (policy_f64 ? launch_move<double, kChosen, kResign> : launch_move<float, kChosen, kResign>)(
+        what, grid, st, states, counts, actions, n_children, game_id, G, inv_t, greedy, seed, ply, child_policy, choice, policy, chosen, moved,
+        term, r);
     if (rc) return rc;
-    return aq_launch(kChosen ? "aq_selfplay_advance_chosen(compact)" : "aq_selfplay_advance(compact)", selfplay_compact_kernel, 1, 1024, 0,
-                     st, false, moved, term, game_id, G, ply, next_states, next_game_id, final_flags, final_plies, alive_count);
+    return aq_launch(compact_what, kResign ? selfplay_compact_resign_kernel : selfplay_compact_kernel, 1, 1024, 0, st, false, moved, term,
+                     game_id, G, (int)ply, next_states, next_game_id, final_flags, final_plies, alive_count);
 }
 
 extern "C" int aq_selfplay_advance(const AqState *states, const int32_t *counts, const int16_t *actions, const int16_t *n_children,
@@ -1008,9 +1133,10 @@ extern "C" int aq_selfplay_advance(const AqState *states, const int32_t *counts,
     if (G <= 0 || !states || !counts || !actions || !n_children || !game_id || !policy || !next_states || !next_game_id || !final_flags ||
         !final_plies || !alive_count || !workspace || !(temperature >= 0.0))
         return aq_set_error(AQ_ERR_ARG, "aq_selfplay_advance");
-    return selfplay_advance<false>("aq_selfplay_advance(move)", states, counts, nullptr, nullptr, actions, n_children, game_id, G, temperature,
-                                   seed, ply, policy, policy_f64, chosen, next_states, next_game_id, final_flags, final_plies, alive_count,
-                                   workspace, reinterpret_cast<cudaStream_t>(stream));
+    return selfplay_advance<false, false>("aq_selfplay_advance(move)", "aq_selfplay_advance(compact)", states, counts, nullptr, nullptr,
+                                          actions, n_children, game_id, G, temperature, seed, ply, policy, policy_f64, chosen, ResignArgs{},
+                                          next_states, next_game_id, final_flags, final_plies, alive_count, workspace,
+                                          reinterpret_cast<cudaStream_t>(stream));
 }
 
 extern "C" int aq_selfplay_advance_chosen(const AqState *states, const float *child_policy, const int16_t *choice, const int16_t *actions,
@@ -1020,7 +1146,32 @@ extern "C" int aq_selfplay_advance_chosen(const AqState *states, const float *ch
     if (G <= 0 || !states || !child_policy || !choice || !actions || !n_children || !game_id || !policy || !next_states || !next_game_id ||
         !final_flags || !final_plies || !alive_count || !workspace)
         return aq_set_error(AQ_ERR_ARG, "aq_selfplay_advance_chosen");
-    return selfplay_advance<true>("aq_selfplay_advance_chosen(move)", states, nullptr, child_policy, choice, actions, n_children, game_id, G,
-                                  1.0, 0, ply, policy, policy_f64, chosen, next_states, next_game_id, final_flags, final_plies, alive_count,
-                                  workspace, reinterpret_cast<cudaStream_t>(stream));
+    return selfplay_advance<true, false>("aq_selfplay_advance_chosen(move)", "aq_selfplay_advance_chosen(compact)", states, nullptr,
+                                         child_policy, choice, actions, n_children, game_id, G, 1.0, 0, ply, policy, policy_f64, chosen,
+                                         ResignArgs{}, next_states, next_game_id, final_flags, final_plies, alive_count, workspace,
+                                         reinterpret_cast<cudaStream_t>(stream));
+}
+
+extern "C" int aq_selfplay_advance_resign(const AqState *states, const int32_t *counts, const float *child_policy, const int16_t *choice,
+                                          const int16_t *actions, const int16_t *n_children, const int64_t *game_id, int64_t G, double temperature,
+                                          uint64_t seed, int32_t ply, void *policy, int policy_f64, int16_t *chosen, const double *root_value,
+                                          const double *best_q, double v_resign, double calibration, double *resign_min, uint8_t *is_calibration,
+                                          AqState *next_states,
+                                          int64_t *next_game_id, uint8_t *final_flags, int64_t *final_plies, int32_t *alive_count, void *workspace,
+                                          void *stream) {
+    const bool by_counts = counts != nullptr, by_choice = child_policy != nullptr || choice != nullptr;
+    if (G <= 0 || !states || by_counts == by_choice || (by_choice && (!child_policy || !choice)) || (by_counts && !(temperature >= 0.0)) ||
+        !actions || !n_children || !game_id || !policy || !next_states || !next_game_id || !final_flags || !final_plies || !alive_count ||
+        !workspace || isnan(v_resign) || !(calibration >= 0.0 && calibration <= 1.0) || !root_value || !best_q || !resign_min ||
+        !is_calibration)
+        return aq_set_error(AQ_ERR_ARG, "aq_selfplay_advance_resign");
+    const ResignArgs r{root_value, best_q, v_resign, calibration, resign_min, is_calibration};
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    if (by_counts)
+        return selfplay_advance<false, true>("aq_selfplay_advance_resign(move)", "aq_selfplay_advance_resign(compact)", states, counts, nullptr,
+                                             nullptr, actions, n_children, game_id, G, temperature, seed, ply, policy, policy_f64, chosen, r,
+                                             next_states, next_game_id, final_flags, final_plies, alive_count, workspace, st);
+    return selfplay_advance<true, true>("aq_selfplay_advance_resign(move)", "aq_selfplay_advance_resign(compact)", states, nullptr, child_policy,
+                                        choice, actions, n_children, game_id, G, 1.0, seed, ply, policy, policy_f64, chosen, r, next_states,
+                                        next_game_id, final_flags, final_plies, alive_count, workspace, st);
 }

@@ -93,6 +93,7 @@ class BatchedMCTS:
         self._ws = [None, None] if self.tree_reuse else [None]
         self._last = None     # tree_reuse: (workspace slot, G) of the previous search, the source a next search can continue
         self.last_kept = None  # tree_reuse: int32[G] nodes carried into each row by the last search (0 = fresh root), else None
+        self._root = None      # (workspace, G, real rows, max_nodes) of the last search: what root_values() reads
         self._buf = {}
         self._graphs = {}
         self._warm = set()   # step modes (the last item of a graph key: Gumbel or not) whose lazy initialisation an eager step has done
@@ -193,6 +194,7 @@ class BatchedMCTS:
             raise ValueError(f"this searcher's node arena holds {self.sims} simulations per search, not {sims}")
         if G_real == 0:
             self.last_kept = self.last_policy = self.last_choice = None
+            self._root = (None, 0, 0, 0)
             return (torch.empty((0, gl.MAX_LEGAL), dtype=torch.int32, device=dev), torch.empty((0, gl.MAX_LEGAL), dtype=torch.int16, device=dev),
                     torch.empty((0,), dtype=torch.int16, device=dev), torch.zeros((3,), dtype=torch.int32, device=dev))
         # Self-play and the arena drop finished games, so the number of roots shrinks by a few almost every ply.  Batches above 256
@@ -273,7 +275,28 @@ class BatchedMCTS:
                        "aq_mcts_root_counts")
             if self.model is not None:
                 status[1:2].copy_(torch.isnan(buf["value"]).any().reshape(1))
+        self._root = (ws, G, G_real, max_nodes)
         return counts[:G_real], actions[:G_real], n[:G_real], status
+
+    @torch.no_grad()
+    def root_values(self):
+        """The search's evaluation of each root of the last search, on the device and without a synchronisation (aq_mcts_root_values):
+        (root_value float64[G], best_q float64[G]), both from the player to move at the root.  root_value = w / n of the root (NaN
+        if it has no visit); best_q = -(w / n) of its most visited child, the first in legal_actions() order on ties (the move
+        temperature 0 plays), -inf if that child has no visit or the root no children.  With tree_reuse the carried visits count."""
+        if self._root is None:
+            raise ValueError("root_values() reads the last search of this searcher: run a search first")
+        ws, G, G_real, max_nodes = self._root
+        dev = self.device
+        root_value = torch.empty((G,), dtype=torch.float64, device=dev)
+        best_q = torch.empty((G,), dtype=torch.float64, device=dev)
+        if G:
+            best_child = torch.empty((G,), dtype=torch.int16, device=dev)
+            P = _lib.ptr
+            with torch.cuda.device(dev):
+                _lib.check(_lib.load().aq_mcts_root_values(P(ws), G, max_nodes, P(root_value), P(best_q), P(best_child), _lib.stream_ptr(dev)),
+                           "aq_mcts_root_values")
+        return root_value[:G_real], best_q[:G_real]
 
     @staticmethod
     def check_status(status):

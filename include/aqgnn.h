@@ -53,7 +53,7 @@ typedef struct AqState {
     uint64_t reserved; /* reserved, 0 */
 } AqState;
 
-#define AQ_VERSION 208 /* bumped with every change of a signature below; the ctypes loader refuses a library of another version */
+#define AQ_VERSION 209 /* bumped with every change of a signature below; the ctypes loader refuses a library of another version */
 int aq_version(void);
 const char *aq_last_error_string(void);
 /* Number of kernels this library has launched in the process so far (monotonic; kernels replayed through a CUDA graph the caller
@@ -305,6 +305,14 @@ int aq_mcts_expand_select_gumbel(void *ws, int64_t G, int64_t max_nodes, const f
 int aq_mcts_gumbel_result(void *ws, int64_t G, int64_t max_nodes, float *policy /*[G,136]*/, int16_t *choice /*[G]*/, void *stream);
 int aq_mcts_root_counts(void *ws, int64_t G, int64_t max_nodes, int32_t *counts /*[G,136]*/,
                         int16_t *actions /*[G,136]*/, int16_t *n_children /*[G]*/, int32_t *overflow, void *stream);
+/* Root values of the last search of every game (fresh, carried, noised or Gumbel roots alike), all in double, one warp per game:
+ *   root_value [G] = w_root / n_root, from the player to move at the root; NaN if n_root == 0
+ *   best_child [G] = the root child with the largest visit count, the first in legal_actions() order on ties (the child that
+ *                    temperature 0 plays); -1 without children
+ *   best_q     [G] = -(w_b / n_b) of that child b, from the player to move at the root; -inf if n_b == 0 or there are no children
+ * AQ_ERR_ARG for G < 1, max_nodes < 1 or a NULL pointer. */
+int aq_mcts_root_values(void *ws, int64_t G, int64_t max_nodes, double *root_value /*[G]*/, double *best_q /*[G]*/, int16_t *best_child /*[G]*/,
+                        void *stream);
 /* Dirichlet noise on the priors of every expanded, not yet noised root (AlphaZero; the reference has none).
  *   game_id [G] int64 (NULL: the row index), seed / ply: the key of the draw; alpha > 0, 0 <= fraction <= 1
  *   root_priors [G,136] f32 (may be NULL): the root's child priors after the call, legal_actions() order, 0 beyond n_children
@@ -345,6 +353,30 @@ int aq_selfplay_advance_chosen(const AqState *states, const float *child_policy 
                                const int16_t *actions, const int16_t *n_children, const int64_t *game_id, int64_t G, int32_t ply,
                                void *policy, int policy_f64, int16_t *chosen, AqState *next_states, int64_t *next_game_id,
                                uint8_t *final_flags, int64_t *final_plies, int32_t *alive_count, void *workspace, void *stream);
+/* Resignation (AlphaGo Zero, Silver et al. 2017; the reference has none): one ply as aq_selfplay_advance when counts is given (then
+ * child_policy and choice are NULL), or as aq_selfplay_advance_chosen when child_policy and choice are (then counts is NULL), in which
+ * a game may resign.  For game g, with s = max(root_value[g], best_q[g]) as aq_mcts_root_values returns them (NaN if either is):
+ *   resign_min [num_games, 2] f64, indexed by game_id: resign_min[game_id[g], ply & 1] = min(itself, s) for every game at every
+ *              ply (a NaN s leaves it); column 0 belongs to the first player, column 1 to the second.  The caller initialises it
+ *              (+inf).
+ *   calibration game: u < calibration with u = (mix64(mix64((seed ^ kResignDomain) + 0x9E3779B97F4A7C15 * (game_id + 1))) >> 11)
+ *              * 2^-53 (splitmix64 finaliser, csrc/mcts.cu): a function of (seed, game id) alone, the same at every ply and
+ *              independent of the move, noise and Gumbel draws.  Calibration games never resign; they are played to the end.
+ *   is_calibration [num_games] u8, indexed by game_id: 1 for a calibration game, 0 otherwise, written for every game at every ply
+ *              (the bit the kernel used).
+ *   A game that is not a calibration game and has s < v_resign resigns: its policy row is written as without resignation, no
+ *   move is played (chosen[g] = -1), and it leaves the batch with final_flags = 1 | 4 (bit 0: the player to move has lost, bit 2:
+ *   resigned) and final_plies = ply, the moves played.  A resigned game therefore has final_plies + 1 recorded positions, a game
+ *   that ends on the board final_plies; the value targets of both follow from bit 0 and final_plies alike.
+ * Every other game gets exactly what aq_selfplay_advance / aq_selfplay_advance_chosen give it.  Two launches.
+ * AQ_ERR_ARG as those entries, and for neither or both modes given, a NaN v_resign, calibration outside [0, 1] or a NULL
+ * root_value, best_q, resign_min or is_calibration. */
+int aq_selfplay_advance_resign(const AqState *states, const int32_t *counts, const float *child_policy, const int16_t *choice,
+                               const int16_t *actions, const int16_t *n_children, const int64_t *game_id, int64_t G, double temperature,
+                               uint64_t seed, int32_t ply, void *policy, int policy_f64, int16_t *chosen, const double *root_value,
+                               const double *best_q, double v_resign, double calibration, double *resign_min /*[num_games,2]*/,
+                               uint8_t *is_calibration /*[num_games]*/, AqState *next_states, int64_t *next_game_id, uint8_t *final_flags, int64_t *final_plies,
+                               int32_t *alive_count, void *workspace, void *stream);
 
 /* agents.heuristic_eval (agents.py:22-54) for B states: shortest pawn-path lengths to the goal row for the mover
  * and for the enemy (shortest_path_bfs, agents.py:27-41, with the jump rules of legal_actions_pos; -1 = no path).
