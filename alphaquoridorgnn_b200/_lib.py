@@ -9,7 +9,7 @@ import torch
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG, "libaqgnn.so")
-ABI_VERSION = 209 # AQ_VERSION of include/aqgnn.h this table of signatures was written for
+ABI_VERSION = 210 # AQ_VERSION of include/aqgnn.h this table of signatures was written for
 
 # name -> (restype, argtypes); must list every symbol declared in include/aqgnn.h
 _vp, _i64, _i32, _f32 = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_float
@@ -70,6 +70,9 @@ SYMBOLS = {
     "aq_mcts_expand_select_gumbel": (_i32, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _f32, _vp, _vp, _vp]),
     "aq_mcts_gumbel_result": (_i32, [_vp, _i64, _i64, _vp, _vp, _vp]),
     "aq_mcts_root_counts": (_i32, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "aq_mcts_select_forced": (_i32, [_vp, _i64, _i64, _f32, _f32, _vp, _vp, _vp]),
+    "aq_mcts_expand_select_forced": (_i32, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp]),
+    "aq_mcts_root_counts_pruned": (_i32, [_vp, _i64, _i64, _f32, _f32, _vp, _vp, _vp, _vp, _vp]),
     "aq_mcts_root_values": (_i32, [_vp, _i64, _i64, _vp, _vp, _vp, _vp]),
     "aq_mcts_root_noise": (_i32, [_vp, _i64, _i64, _vp, _u64, _i32, _f32, _f32, _vp, _vp]),
     "aq_selfplay_ws_bytes": (_i64, [_i64]),

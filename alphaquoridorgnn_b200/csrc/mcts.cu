@@ -8,7 +8,8 @@
 // The reference has no virtual loss, no Dirichlet noise and no tree reuse, so batching ACROSS games
 // leaves every game's search unchanged.  Tree reuse between moves (aq_mcts_advance, AlphaGo Zero) and
 // Dirichlet noise on the root priors (aq_mcts_root_noise, AlphaZero) are opt-in additions the reference
-// does not have; without them every search starts from aq_mcts_reset with the network's priors.
+// does not have; without them every search starts from aq_mcts_reset with the network's priors.  So are the Gumbel root and KataGo's
+// forced playouts with policy target pruning (aq_mcts_select_forced, aq_mcts_root_counts_pruned).
 //
 // Arithmetic is kept as the reference computes it under NumPy >= 2 (requirements.txt pins
 // numpy~=2.0.2, NEP 50 promotion): w accumulates in float64; the PUCT score is
@@ -285,17 +286,40 @@ __device__ __forceinline__ int gumbel_pick(const GumbelQ &r, const MctsHot *hot,
     return best_c == 0x7fffffff ? 0 : best_c;
 }
 
+// ------------------------------------------------------------------------------------------
+// Forced playouts and policy target pruning (KataGo: David J. Wu, "Accelerating Self-Play Learning in Go", 2019; the reference has
+// none).  At a root with n_root visits, t = n_root - 1 (the sum of the children's n, as the PUCT scan takes it), child c with
+// stored prior P_c (noised if the root was noised), visits n_c and value sum w_c, and k = forced_k widened to double:
+//   n_forced(c) = sqrt((double)k * (double)P_c * (double)t)                                    (float64, rounded as written)
+//   PUCT(c, m)  = float32(-w_c / n_c) + ((c_puct * P_c) * float32(sqrt(t))) / float32(1 + m)  (the select score, float32, with
+//                 the visit count of U replaced by m)
+// Root rule (aq_mcts_select_forced): the root's descent takes the first child in legal_actions() order with n_c >= 1 and
+// (double)n_c < n_forced(c), else the PUCT arg-max; every other node uses PUCT.  Unvisited children are never forced.
+// Pruning (aq_mcts_root_counts_pruned): c* = the first child with the largest n keeps n_c*.  Every other child with n_c >= 1 starts
+// from m = n_c; while m >= 1, (double)(m - 1) >= (double)n_c - n_forced(c) and PUCT(c, m - 1) < PUCT(c*, n_c*): m -= 1.  A child
+// that was reduced and ends with m <= 1 gets 0.  k = 0 is the plain search and the plain counts.
+// ------------------------------------------------------------------------------------------
+enum class RootRule { kPuct, kGumbel, kForced };
+
+__device__ __forceinline__ float puct_score(const MctsHot &ch, float c_puct, float sq, int m) {
+    const float q = ch.n ? (float)(-ch.w / (double)ch.n) : 0.0f;
+    return __fadd_rn(q, __fdiv_rn(__fmul_rn(__fmul_rn(c_puct, ch.prior), sq), (float)(1 + m)));
+}
+
+__device__ __forceinline__ double forced_visits(double k, float prior, int t) { return sqrt(__dmul_rn(__dmul_rn(k, (double)prior), (double)t)); }
+
 // Descent of game g by its warp (pv_mcts.py:69-78).  The node arrays are read through plain pointers: in the fused kernel the same
 // warp has just written them (expansion + backup), so the loads must be coherent ones.  kGumbel: the root of a game with a Gumbel
-// root (MctsGame.pad[2] > 0) is left by the Gumbel rule, every other node by PUCT.
-template <bool kGumbel>
+// root (MctsGame.pad[2] > 0) is left by the Gumbel rule; kForced: the root is left by the forced-playout rule (forced_k) when a
+// child qualifies; every other node by PUCT.
+template <RootRule kRule>
 __device__ __forceinline__ void select_game(MctsGame *games, const MctsHot *hot, const MctsCold *cold, int64_t g, int lane, float c_puct,
-                                            AqState *leaf_states, int32_t *leaf_kind) {
+                                            double forced_k, AqState *leaf_states, int32_t *leaf_kind) {
     AqState s = games[g].root;
     int node = 0, kind = 0;
     // what the descent needs from a node: first_child, n_children (cold half) and n (hot half, known from the scan of its parent)
     int first = cold[0].first_child, nc = cold[0].n_children, nn = hot[0].n;
-    if (kGumbel && games[g].pad[2] > 0 && first >= 0 && nc > 0 && !terminal_flags(s)) {   // the Gumbel root's step; PUCT below it
+    if (kRule == RootRule::kGumbel && games[g].pad[2] > 0 && first >= 0 && nc > 0 && !terminal_flags(s)) {   // the Gumbel root's step
         const MctsGame &gm = games[g];
         const GumbelQ r = gumbel_q(gm, hot, first, nc, nn - 1, lane);
         node = first + gumbel_pick(r, hot, cold, first, nc, considered_visit(gm.pad[2], gm.pad[3], nn - 1), lane);
@@ -304,6 +328,28 @@ __device__ __forceinline__ void select_game(MctsGame *games, const MctsHot *hot,
         first = cc.first_child;
         nc = cc.n_children;
         s = state_after(s, cc.action);
+    }
+    if (kRule == RootRule::kForced && first >= 0 && nc > 0 && !terminal_flags(s)) {   // a forced root child, if any; else PUCT
+        int forced = -1;
+#pragma unroll 1
+        for (int c0 = 0; c0 < nc && forced < 0; c0 += 32) {
+            const int c = c0 + lane;
+            bool below = false;
+            if (c < nc) {
+                const MctsHot ch = hot[first + c];
+                below = ch.n >= 1 && (double)ch.n < forced_visits(forced_k, ch.prior, nn - 1);
+            }
+            const unsigned hit = __ballot_sync(0xffffffffu, below);
+            if (hit) forced = c0 + __ffs(hit) - 1;
+        }
+        if (forced >= 0) {
+            node = first + forced;
+            nn = hot[node].n;
+            const MctsCold cc = cold[node];
+            first = cc.first_child;
+            nc = cc.n_children;
+            s = state_after(s, cc.action);
+        }
     }
     while (true) {
         const int tf = terminal_flags(s);  // pv_mcts.py:35-42: terminal test comes first
@@ -318,9 +364,7 @@ __device__ __forceinline__ void select_game(MctsGame *games, const MctsHot *hot,
         int b_n = 0;  // visit count of this lane's best child
         for (int c = lane; c < nc; c += 32) {
             const MctsHot ch = hot[first + c];
-            const float q = ch.n ? (float)(-ch.w / (double)ch.n) : 0.0f;
-            const float u = __fdiv_rn(__fmul_rn(__fmul_rn(c_puct, ch.prior), sq), (float)(1 + ch.n));
-            const float sc = __fadd_rn(q, u);
+            const float sc = puct_score(ch, c_puct, sq, ch.n);
             if (sc > best || (sc == best && c < best_c) || best_c == 0x7fffffff) {
                 best = sc; best_c = c;
                 b_n = ch.n;
@@ -357,7 +401,7 @@ mcts_select_kernel(MctsGame *games, const MctsHot *hot_all, const MctsCold *cold
     const int lane = threadIdx.x & 31;
     const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (g >= G) return;
-    select_game<false>(games, hot_all + g * max_nodes, cold_all + g * max_nodes, g, lane, c_puct, leaf_states, leaf_kind);
+    select_game<RootRule::kPuct>(games, hot_all + g * max_nodes, cold_all + g * max_nodes, g, lane, c_puct, 0.0, leaf_states, leaf_kind);
 }
 
 // mcts_select_kernel with the Gumbel rule at the roots of games that have one
@@ -367,7 +411,18 @@ mcts_select_gumbel_kernel(MctsGame *games, const MctsHot *hot_all, const MctsCol
     const int lane = threadIdx.x & 31;
     const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (g >= G) return;
-    select_game<true>(games, hot_all + g * max_nodes, cold_all + g * max_nodes, g, lane, c_puct, leaf_states, leaf_kind);
+    select_game<RootRule::kGumbel>(games, hot_all + g * max_nodes, cold_all + g * max_nodes, g, lane, c_puct, 0.0, leaf_states, leaf_kind);
+}
+
+// mcts_select_kernel with the forced-playout rule at the roots
+__global__ void __launch_bounds__(128)
+mcts_select_forced_kernel(MctsGame *games, const MctsHot *hot_all, const MctsCold *cold_all, int64_t G, int64_t max_nodes, float c_puct,
+                          double forced_k, AqState *leaf_states, int32_t *leaf_kind) {
+    const int lane = threadIdx.x & 31;
+    const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (g >= G) return;
+    select_game<RootRule::kForced>(games, hot_all + g * max_nodes, cold_all + g * max_nodes, g, lane, c_puct, forced_k, leaf_states,
+                                   leaf_kind);
 }
 
 // Expansion of the selected leaf of game g with the evaluated priors (pv_mcts.py:47-56) and the backup of its value (:60-66).
@@ -469,7 +524,7 @@ mcts_expand_select_kernel(MctsGame *games, MctsHot *hot_all, MctsCold *cold_all,
     MctsCold *cold = cold_all + g * max_nodes;
     expand_backup_game(games, hot, cold, g, lane, max_nodes, priors, values, mask, pawn);
     __syncwarp();   // orders the warp's node writes (children by all lanes, the backup by lane 0) before the descent's reads
-    select_game<false>(games, hot, cold, g, lane, c_puct, leaf_states, leaf_kind);
+    select_game<RootRule::kPuct>(games, hot, cold, g, lane, c_puct, 0.0, leaf_states, leaf_kind);
 }
 
 // mcts_expand_select_kernel with the Gumbel rule at the roots of games that have one
@@ -484,7 +539,22 @@ mcts_expand_select_gumbel_kernel(MctsGame *games, MctsHot *hot_all, MctsCold *co
     MctsCold *cold = cold_all + g * max_nodes;
     expand_backup_game(games, hot, cold, g, lane, max_nodes, priors, values, mask, pawn);
     __syncwarp();
-    select_game<true>(games, hot, cold, g, lane, c_puct, leaf_states, leaf_kind);
+    select_game<RootRule::kGumbel>(games, hot, cold, g, lane, c_puct, 0.0, leaf_states, leaf_kind);
+}
+
+// mcts_expand_select_kernel with the forced-playout rule at the roots
+__global__ void __launch_bounds__(128)
+mcts_expand_select_forced_kernel(MctsGame *games, MctsHot *hot_all, MctsCold *cold_all, int64_t G, int64_t max_nodes,
+                                 const float *__restrict__ priors, const float *__restrict__ values, const uint32_t *__restrict__ mask,
+                                 const uint8_t *__restrict__ pawn, float c_puct, double forced_k, AqState *leaf_states, int32_t *leaf_kind) {
+    const int lane = threadIdx.x & 31;
+    const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (g >= G) return;
+    MctsHot *hot = hot_all + g * max_nodes;
+    MctsCold *cold = cold_all + g * max_nodes;
+    expand_backup_game(games, hot, cold, g, lane, max_nodes, priors, values, mask, pawn);
+    __syncwarp();
+    select_game<RootRule::kForced>(games, hot, cold, g, lane, c_puct, forced_k, leaf_states, leaf_kind);
 }
 
 __global__ void mcts_root_counts_kernel(const MctsGame *__restrict__ games, const MctsHot *__restrict__ hot_all,
@@ -500,6 +570,48 @@ __global__ void mcts_root_counts_kernel(const MctsGame *__restrict__ games, cons
     const int nc = first < 0 ? 0 : cold[0].n_children;
     for (int c = lane; c < AQ_MAX_LEGAL; c += 32) {
         counts[g * AQ_MAX_LEGAL + c] = c < nc ? hot[first + c].n : 0;
+        actions[g * AQ_MAX_LEGAL + c] = c < nc ? cold[first + c].action : (int16_t)-1;
+    }
+    if (lane == 0) {
+        n_out[g] = (int16_t)nc;
+        if (overflow && games[g].overflow) atomicExch(overflow, 1);
+    }
+}
+
+// mcts_root_counts_kernel with the counts pruned (the rule is stated above RootRule): one warp per game, child c in lane c % 32,
+// slot c / 32.  c* is found as mcts_root_values_kernel finds its best child.
+__global__ void __launch_bounds__(128)
+mcts_root_counts_pruned_kernel(const MctsGame *__restrict__ games, const MctsHot *__restrict__ hot_all, const MctsCold *__restrict__ cold_all,
+                               int64_t G, int64_t max_nodes, float c_puct, double forced_k, int32_t *__restrict__ counts,
+                               int16_t *__restrict__ actions, int16_t *__restrict__ n_out, int32_t *__restrict__ overflow) {
+    const int lane = threadIdx.x & 31;
+    const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (g >= G) return;
+    const MctsHot *hot = hot_all + g * max_nodes;
+    const MctsCold *cold = cold_all + g * max_nodes;
+    const int first = cold[0].first_child;
+    const int nc = first < 0 ? 0 : cold[0].n_children;
+    const int t = hot[0].n - 1;
+    const float sq = (float)sqrt((double)t);
+    long long best = -1;
+    for (int c = lane; c < nc; c += 32) best = max(best, ((long long)hot[first + c].n << 8) | (long long)(255 - c));   // largest n, then smallest c
+#pragma unroll
+    for (int d = 16; d; d >>= 1) best = max(best, __shfl_xor_sync(0xffffffffu, best, d));
+    const int b = best < 0 ? -1 : 255 - (int)(best & 255);
+    const float best_score = b >= 0 ? puct_score(hot[first + b], c_puct, sq, hot[first + b].n) : 0.f;
+    for (int c = lane; c < AQ_MAX_LEGAL; c += 32) {
+        int m = 0;
+        if (c < nc) {
+            const MctsHot ch = hot[first + c];
+            m = ch.n;
+            if (c != b && ch.n >= 1) {
+                const double floor_n = __dsub_rn((double)ch.n, forced_visits(forced_k, ch.prior, t));
+#pragma unroll 1
+                while (m >= 1 && (double)(m - 1) >= floor_n && puct_score(ch, c_puct, sq, m - 1) < best_score) --m;
+                if (m < ch.n && m <= 1) m = 0;   // reduced to a single playout: pruned entirely
+            }
+        }
+        counts[g * AQ_MAX_LEGAL + c] = m;
         actions[g * AQ_MAX_LEGAL + c] = c < nc ? cold[first + c].action : (int16_t)-1;
     }
     if (lane == 0) {
@@ -1012,6 +1124,16 @@ extern "C" int aq_mcts_select_gumbel(void *ws, int64_t G, int64_t max_nodes, flo
                      false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, c_puct, leaf_states, leaf_kind);
 }
 
+static inline bool forced_k_ok(float forced_k) { return forced_k >= 0.f && isfinite(forced_k); }
+
+extern "C" int aq_mcts_select_forced(void *ws, int64_t G, int64_t max_nodes, float c_puct, float forced_k, AqState *leaf_states,
+                                     int32_t *leaf_kind, void *stream) {
+    if (G <= 0 || !ws || !leaf_states || !leaf_kind || !forced_k_ok(forced_k)) return aq_set_error(AQ_ERR_ARG, "aq_mcts_select_forced");
+    return aq_launch("aq_mcts_select_forced", mcts_select_forced_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream),
+                     false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, c_puct, (double)forced_k, leaf_states,
+                     leaf_kind);
+}
+
 extern "C" int aq_mcts_expand_backup(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values,
                                      const uint32_t *mask, const uint8_t *pawn, void *stream) {
     if (G <= 0 || !ws || !priors || !values || !mask || !pawn) return aq_set_error(AQ_ERR_ARG, "aq_mcts_expand_backup");
@@ -1035,6 +1157,29 @@ extern "C" int aq_mcts_expand_select_gumbel(void *ws, int64_t G, int64_t max_nod
     return aq_launch("aq_mcts_expand_select_gumbel", mcts_expand_select_gumbel_kernel, (unsigned)((G + 3) / 4), 128, 0,
                      reinterpret_cast<cudaStream_t>(stream), false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, priors,
                      values, mask, pawn, c_puct, leaf_states, leaf_kind);
+}
+
+extern "C" int aq_mcts_expand_select_forced(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values,
+                                            const uint32_t *mask, const uint8_t *pawn, float c_puct, float forced_k, AqState *leaf_states,
+                                            int32_t *leaf_kind, void *stream) {
+    if (G <= 0 || !ws || !priors || !values || !mask || !pawn || !leaf_states || !leaf_kind || !forced_k_ok(forced_k))
+        return aq_set_error(AQ_ERR_ARG, "aq_mcts_expand_select_forced");
+    return aq_launch("aq_mcts_expand_select_forced", mcts_expand_select_forced_kernel, (unsigned)((G + 3) / 4), 128, 0,
+                     reinterpret_cast<cudaStream_t>(stream), false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, priors,
+                     values, mask, pawn, c_puct, (double)forced_k, leaf_states, leaf_kind);
+}
+
+extern "C" int aq_mcts_root_counts_pruned(void *ws, int64_t G, int64_t max_nodes, float c_puct, float forced_k, int32_t *counts,
+                                          int16_t *actions, int16_t *n_children, int32_t *overflow, void *stream) {
+    if (G <= 0 || !ws || !counts || !actions || !n_children || !forced_k_ok(forced_k))
+        return aq_set_error(AQ_ERR_ARG, "aq_mcts_root_counts_pruned");
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    if (overflow) {
+        cudaError_t e = cudaMemsetAsync(overflow, 0, sizeof(int32_t), st);
+        if (e != cudaSuccess) return aq_set_error((int)e, "aq_mcts_root_counts_pruned");
+    }
+    return aq_launch("aq_mcts_root_counts_pruned", mcts_root_counts_pruned_kernel, (unsigned)((G + 3) / 4), 128, 0, st, false, games_of(ws),
+                     hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, c_puct, (double)forced_k, counts, actions, n_children, overflow);
 }
 
 extern "C" int aq_mcts_root_counts(void *ws, int64_t G, int64_t max_nodes, int32_t *counts, int16_t *actions,

@@ -11,6 +11,8 @@ Dirichlet noise on the root priors (AlphaZero self-play exploration) is opt-in t
 BatchedMCTS(..., dirichlet_alpha=0.3); the default searches with the network's priors.
 So is the Gumbel root of Gumbel AlphaZero, BatchedMCTS(..., gumbel_considered=16): sequential halving over Gumbel-top-k sampled
 root children and a completed-Q improved policy; the default keeps PUCT at the root.
+Forced playouts with policy target pruning (KataGo), BatchedMCTS(..., forced_k=2.0), give every visited root child at least
+sqrt(k * P * sum N) visits and take the surplus back out of the counts the search returns; the default returns the plain counts.
 """
 import math
 from copy import deepcopy
@@ -57,10 +59,19 @@ class BatchedMCTS:
     the search, last_policy f32[G,136] holds the improved policy softmax(logits + sigma(completed Q)) over the root's children and
     last_choice int16[G] the child to play (aq_mcts_gumbel_root / _result, csrc/mcts.cu).  The draw is keyed by search(...,
     noise_seed, game_id, ply).  It cannot be combined with tree_reuse (the schedule starts from a root without child visits) or with
-    dirichlet_alpha (the Gumbel draw is the root's exploration).  None (the default) runs exactly the PUCT search."""
+    dirichlet_alpha (the Gumbel draw is the root's exploration).  None (the default) runs exactly the PUCT search.
+
+    forced_k (forced playouts and policy target pruning, KataGo: Wu 2019; the reference has none): the root's descent takes the
+    first child in legal_actions() order that has been visited but has fewer than n_forced = sqrt(forced_k * P * t) visits (P its
+    prior, noised if the root was, t the sum of the root children's visits), else the PUCT arg-max; every node below the root keeps
+    PUCT (aq_mcts_select_forced).  The counts a search returns are then pruned (aq_mcts_root_counts_pruned): every child but the
+    most visited one loses the visits, up to n_forced, that PUCT would not have given it against that child, and a child left with
+    one visit goes to 0.  The most visited child keeps its count, so temperature 0 and root_values() see the same move.  It pairs
+    with dirichlet_alpha (the forced visits then explore the noise without training on it) and tree_reuse (carried visits count in
+    t), not with gumbel_considered.  forced_k=0 is the plain search; None (the default) runs exactly it."""
 
     def __init__(self, evaluator, sims=None, c_puct=C_PUCT, device=None, use_graph=True, tree_reuse=False, dirichlet_alpha=None,
-                 noise_fraction=0.25, gumbel_considered=None, gumbel_scale=1.0):
+                 noise_fraction=0.25, gumbel_considered=None, gumbel_scale=1.0, forced_k=None):
         if tree_reuse and not sims:
             raise ValueError("BatchedMCTS(tree_reuse=True) needs `sims` at construction: it sizes the node arena")
         if dirichlet_alpha is not None and not (math.isfinite(dirichlet_alpha) and dirichlet_alpha > 0):
@@ -77,6 +88,10 @@ class BatchedMCTS:
                                  "child visits")
             if dirichlet_alpha is not None:
                 raise ValueError("gumbel_considered cannot be combined with dirichlet_alpha: the Gumbel draw is the root's exploration")
+            if forced_k is not None:
+                raise ValueError("gumbel_considered cannot be combined with forced_k: the Gumbel schedule sets the root's visits")
+        if forced_k is not None and (isinstance(forced_k, bool) or not (math.isfinite(forced_k) and forced_k >= 0)):
+            raise ValueError(f"forced_k must be a finite number >= 0 (or None), not {forced_k!r}")
         self.model = evaluator if hasattr(evaluator, "flat_parameters") else None
         self.evaluator = network_evaluator(evaluator) if hasattr(evaluator, "predict_batch") else evaluator
         self.sims = sims
@@ -88,6 +103,8 @@ class BatchedMCTS:
         self.noise_fraction = float(noise_fraction)
         self.gumbel_considered = None if gumbel_considered is None else int(gumbel_considered)
         self.gumbel_scale = float(gumbel_scale)
+        self.forced_k = None if forced_k is None else float(forced_k)
+        self._mode = "puct" if self.forced_k is None else "forced"   # step mode of the simulations (a Gumbel search: of its first)
         self.last_policy = None  # gumbel_considered: f32[G,136] improved policy of the last search, else None
         self.last_choice = None  # gumbel_considered: int16[G] child chosen by the last search, else None
         self._ws = [None, None] if self.tree_reuse else [None]
@@ -96,7 +113,8 @@ class BatchedMCTS:
         self._root = None      # (workspace, G, real rows, max_nodes) of the last search: what root_values() reads
         self._buf = {}
         self._graphs = {}
-        self._warm = set()   # step modes (the last item of a graph key: Gumbel or not) whose lazy initialisation an eager step has done
+        self._warm = set()   # step modes (the last item of a graph key: "puct", "gumbel" or "forced") whose lazy initialisation an
+                             # eager step has done
 
     def _workspace(self, G, max_nodes, slot=0):
         L = _lib.load()
@@ -123,19 +141,24 @@ class BatchedMCTS:
             }
         return self._buf[G]
 
-    def _step(self, ws, G, max_nodes, buf, evaluate, st, steps=1, gumbel=False):
+    def _step(self, ws, G, max_nodes, buf, evaluate, st, steps=1, gumbel=False, forced=False):
         """`steps` simulations for all games: select, then `steps` leaf evaluations out = evaluate(stream) (terminal leaves are
         evaluated too and ignored by the backup) joined by the fused expand + backup + next select, then the last expand + backup.
-        gumbel: the selects leave a Gumbel root by the Gumbel rule."""
+        gumbel: the selects leave a Gumbel root by the Gumbel rule; forced: the root by the forced-playout rule (forced_k)."""
         L, P = _lib.load(), _lib.ptr
-        select, expand_select = ((L.aq_mcts_select_gumbel, L.aq_mcts_expand_select_gumbel) if gumbel else
-                                 (L.aq_mcts_select, L.aq_mcts_expand_select))
-        _lib.check(select(P(ws), G, max_nodes, self.c_puct, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_select")
+        if forced:
+            k = (self.forced_k,)
+            select, expand_select = L.aq_mcts_select_forced, L.aq_mcts_expand_select_forced
+        else:
+            k = ()
+            select, expand_select = ((L.aq_mcts_select_gumbel, L.aq_mcts_expand_select_gumbel) if gumbel else
+                                     (L.aq_mcts_select, L.aq_mcts_expand_select))
+        _lib.check(select(P(ws), G, max_nodes, self.c_puct, *k, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_select")
         for i in range(steps):
             out = evaluate(st)
             leaves = (P(ws), G, max_nodes, P(out["priors"]), P(out["value"]), P(out["mask"]), P(out["pawn"]))
             if i + 1 < steps:
-                _lib.check(expand_select(*leaves, self.c_puct, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_expand_select")
+                _lib.check(expand_select(*leaves, self.c_puct, *k, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_expand_select")
             else:
                 _lib.check(L.aq_mcts_expand_backup(*leaves, st), "aq_mcts_expand_backup")
 
@@ -235,7 +258,7 @@ class BatchedMCTS:
                 prec = PRECISIONS[self.model.precision]
                 # bf16 operand tiles, refreshed in place if the parameters changed since the last search
                 prep = self.model.prepared_weights() if prec == 1 else None
-                key = (G, max_nodes, ws.data_ptr(), flat.data_ptr(), prep.data_ptr() if prep is not None else 0, prec, False)
+                key = (G, max_nodes, ws.data_ptr(), flat.data_ptr(), prep.data_ptr() if prep is not None else 0, prec, self._mode)
 
                 def evaluate(s):
                     _lib.check(L.aq_leaf_eval(P(flat), P(prep), P(buf["leaf"]), G, P(buf["priors"]), P(buf["value"]), P(buf["mask"]),
@@ -243,7 +266,7 @@ class BatchedMCTS:
                     return buf
             else:
                 key, evaluate = None, lambda s: self.evaluator(buf["leaf"])
-            step = lambda s, k: self._step(ws, G, max_nodes, buf, evaluate, s, k)
+            step = lambda s, k: self._step(ws, G, max_nodes, buf, evaluate, s, k, forced=self.forced_k is not None)
             if self.dirichlet_alpha is not None or self.gumbel_considered is not None:
                 seed = (int(torch.randint(0, 2 ** 63 - 1, (1,)).item()) if noise_seed is None else int(noise_seed)) & (2 ** 64 - 1)
                 gid = None if game_id is None else pad(game_id.to(device=dev, dtype=torch.int64).reshape(G_real), 0)
@@ -254,7 +277,7 @@ class BatchedMCTS:
                 _lib.check(L.aq_mcts_gumbel_root(P(ws), G, max_nodes, P(gid), seed, int(ply), self.gumbel_considered, self.gumbel_scale,
                                                  sims, None, st), "aq_mcts_gumbel_root")
                 gstep = lambda s, k: self._step(ws, G, max_nodes, buf, evaluate, s, k, gumbel=True)
-                self._simulate(sims - 1, gstep, None if key is None else key[:-1] + (True,), st)
+                self._simulate(sims - 1, gstep, None if key is None else key[:-1] + ("gumbel",), st)
                 policy = torch.empty((G, gl.MAX_LEGAL), dtype=torch.float32, device=dev)
                 choice = torch.empty((G,), dtype=torch.int16, device=dev)
                 _lib.check(L.aq_mcts_gumbel_result(P(ws), G, max_nodes, P(policy), P(choice), st), "aq_mcts_gumbel_result")
@@ -271,8 +294,12 @@ class BatchedMCTS:
             counts = torch.empty((G, gl.MAX_LEGAL), dtype=torch.int32, device=dev)
             actions = torch.empty((G, gl.MAX_LEGAL), dtype=torch.int16, device=dev)
             n = torch.empty((G,), dtype=torch.int16, device=dev)
-            _lib.check(L.aq_mcts_root_counts(P(ws), G, max_nodes, P(counts), P(actions), P(n), P(status[:1]), st),
-                       "aq_mcts_root_counts")
+            if self.forced_k is None:
+                _lib.check(L.aq_mcts_root_counts(P(ws), G, max_nodes, P(counts), P(actions), P(n), P(status[:1]), st),
+                           "aq_mcts_root_counts")
+            else:
+                _lib.check(L.aq_mcts_root_counts_pruned(P(ws), G, max_nodes, self.c_puct, self.forced_k, P(counts), P(actions), P(n),
+                                                        P(status[:1]), st), "aq_mcts_root_counts_pruned")
             if self.model is not None:
                 status[1:2].copy_(torch.isnan(buf["value"]).any().reshape(1))
         self._root = (ws, G, G_real, max_nodes)
@@ -321,7 +348,9 @@ class BatchedMCTS:
         The counts then include the carried visits; last_kept gives the nodes carried per row.
 
         With dirichlet_alpha, the root noise of row g is drawn from (noise_seed, game_id[g], ply): game_id int64[G] (None = the row
-        index) names the game, so a game's noise does not depend on the other rows; noise_seed None draws one from torch's generator."""
+        index) names the game, so a game's noise does not depend on the other rows; noise_seed None draws one from torch's generator.
+
+        With forced_k, the counts are the pruned counts (aq_mcts_root_counts_pruned); the tree keeps the visits it made."""
         counts, actions, n, status = self.search_async(roots, sims, src_row, path, noise_seed, game_id, ply)
         self.check_status(status.tolist())   # one synchronisation for both flags
         return counts, actions, n
@@ -339,19 +368,19 @@ class _SearcherCache(dict):
 
 
 def searcher_for(evaluator, sims, device=None, tree_reuse=False, dirichlet_alpha=None, noise_fraction=0.25, gumbel_considered=None,
-                 gumbel_scale=1.0):
+                 gumbel_scale=1.0, forced_k=None):
     """The BatchedMCTS of a network for `sims` simulations, kept on the network object: its node arenas (3.5 GB at 4,096 games x
     200 simulations), leaf buffers and captured graphs are reused by every later self-play / arena / policy call on that network
     instead of being allocated and captured again.  Evaluators that are plain callables get a fresh searcher."""
     dev = gl._dev(device)
     opts = dict(tree_reuse=tree_reuse, dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction, gumbel_considered=gumbel_considered,
-                gumbel_scale=gumbel_scale)
+                gumbel_scale=gumbel_scale, forced_k=forced_k)
     if not hasattr(evaluator, "flat_parameters"):
         return BatchedMCTS(evaluator, sims, device=dev, **opts)
     cache = evaluator.__dict__.setdefault("_searchers", _SearcherCache())
     key = (int(sims), str(dev), bool(tree_reuse), None if dirichlet_alpha is None else float(dirichlet_alpha),
            None if dirichlet_alpha is None else float(noise_fraction), None if gumbel_considered is None else int(gumbel_considered),
-           None if gumbel_considered is None else float(gumbel_scale))
+           None if gumbel_considered is None else float(gumbel_scale), None if forced_k is None else float(forced_k))
     if key not in cache:
         if len(cache) >= 4:
             cache.clear()

@@ -44,7 +44,7 @@ def write_data(history, directory='./data/'):
 @torch.no_grad()
 def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_TEMPERATURE, seed=None, max_plies=None,
                       policy_dtype=torch.float64, tree_reuse=False, dirichlet_alpha=None, noise_fraction=0.25, gumbel_considered=None,
-                      gumbel_scale=1.0, resign_threshold=None, resign_calibration=0.1):
+                      gumbel_scale=1.0, resign_threshold=None, resign_calibration=0.1, forced_k=None):
     """Execute `num_games` self-play games in lock-step (self_play.py:40-68 per game) and keep the record on the device:
     dict(states uint8[T,32] packed, policy [T,209] search policies over all actions (self_play.py:51-54), value f32[T]
     back-filled game results seen from the player to move (self_play.py:63-66), game int64[T], ply int64[T],
@@ -75,7 +75,12 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
     records its last searched position too and ends lost for the player to move (flags bit 0 and bit 2, plies = the moves played;
     the value targets follow as for any loss).  The record gains resign_min f64[num_games, 2], the smallest s each side saw
     (column 0 the first player, +inf where a side never searched), and calibration bool[num_games]; resign_threshold_for picks a
-    threshold from them.  None (the default) plays every game to its end, as the reference does."""
+    threshold from them.  None (the default) plays every game to its end, as the reference does.
+
+    forced_k (KataGo's forced playouts and policy target pruning; the reference has none): every search forces visits to its
+    visited root children (BatchedMCTS) and returns pruned counts, and the ply records and draws its move from those.  It is meant
+    to pair with dirichlet_alpha: the noise still explores, but the visits it forced are taken out of the policy target.  The
+    record format, the value targets and resignation are the same (the most visited child is never pruned)."""
     if policy_dtype not in (torch.float64, torch.float32):
         raise ValueError("policy_dtype must be torch.float64 or torch.float32")
     if resign_threshold is not None:
@@ -88,7 +93,7 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
     seed = (int(seed) if seed is not None else int(torch.seed())) & (2 ** 64 - 1)
     sims = sims or pv_mcts.PV_EVALUATE_COUNT
     mcts = pv_mcts.searcher_for(model, sims, dev, tree_reuse=tree_reuse, dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction,
-                                gumbel_considered=gumbel_considered, gumbel_scale=gumbel_scale)
+                                gumbel_considered=gumbel_considered, gumbel_scale=gumbel_scale, forced_k=forced_k)
     states = start_states(num_games, dev)
     game_id = torch.arange(num_games, device=dev)
     rec_state, rec_policy, rec_game, sizes = [], [], [], []
@@ -188,13 +193,14 @@ def resign_threshold_for(rec, max_false_positive=0.05):
 
 def play_batch(model, num_games, device=None, sims=None, temperature=SP_TEMPERATURE, seed=None, max_plies=None, tree_reuse=False,
                dirichlet_alpha=None, noise_fraction=0.25, gumbel_considered=None, gumbel_scale=1.0, resign_threshold=None,
-               resign_calibration=0.1):
+               resign_calibration=0.1, forced_k=None):
     """play_batch_device + conversion to the reference's history: a list of [[player, enemy, walls], policy (209 floats), value]
     (self_play.py:51-54, 63-66), games in order, plies in order within a game.  Returns (history, dict with per-game results:
     flags, plies, and with resign_threshold also resign_min and calibration)."""
     rec = play_batch_device(model, num_games, device, sims, temperature, seed, max_plies, tree_reuse=tree_reuse,
                             dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction, gumbel_considered=gumbel_considered,
-                            gumbel_scale=gumbel_scale, resign_threshold=resign_threshold, resign_calibration=resign_calibration)
+                            gumbel_scale=gumbel_scale, resign_threshold=resign_threshold, resign_calibration=resign_calibration,
+                            forced_k=forced_k)
     rows, _ = gl.unpack_rows(rec["states"])
     rows = rows.cpu().numpy()
     pols = rec["policy"].cpu().numpy()
@@ -219,12 +225,13 @@ def play(model, device=None):
 
 def self_play(game_count=None, model_path=None, data_dir='./data/', rank=0, world_size=1, sims=None, seed=None, tree_reuse=False,
               dirichlet_alpha=None, noise_fraction=0.25, gumbel_considered=None, gumbel_scale=1.0, resign_threshold=None,
-              resign_calibration=0.1):
+              resign_calibration=0.1, forced_k=None):
     """Perform self-play games and save the training data (self_play.py:71-98).  With
     world_size > 1 each rank plays its share of the games on its own GPU and rank 0 writes the file.
     tree_reuse=True keeps each game's search tree between moves; dirichlet_alpha adds AlphaZero root noise to every search;
     gumbel_considered searches with the Gumbel AlphaZero root and records its improved policy; resign_threshold lets games resign,
-    resign_calibration of them excepted (see play_batch_device)."""
+    resign_calibration of them excepted; forced_k forces root playouts and prunes them from the policy targets (see
+    play_batch_device)."""
     game_count = SP_GAME_COUNT if game_count is None else game_count
     model = GNNNetwork()
     model.prep_for_inference(model_path=model_path or (PV_NETWORK_PATH + 'best.pth'))
@@ -232,7 +239,7 @@ def self_play(game_count=None, model_path=None, data_dir='./data/', rank=0, worl
     history, _ = play_batch(model, mine, sims=sims, seed=None if seed is None else seed + rank, tree_reuse=tree_reuse,
                             dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction, gumbel_considered=gumbel_considered,
                             gumbel_scale=gumbel_scale, resign_threshold=resign_threshold,
-                            resign_calibration=resign_calibration) if mine else ([], None)
+                            resign_calibration=resign_calibration, forced_k=forced_k) if mine else ([], None)
     if world_size > 1:
         import torch.distributed as dist
         gathered = [None] * world_size if rank == 0 else None

@@ -53,7 +53,7 @@ typedef struct AqState {
     uint64_t reserved; /* reserved, 0 */
 } AqState;
 
-#define AQ_VERSION 209 /* bumped with every change of a signature below; the ctypes loader refuses a library of another version */
+#define AQ_VERSION 210 /* bumped with every change of a signature below; the ctypes loader refuses a library of another version */
 int aq_version(void);
 const char *aq_last_error_string(void);
 /* Number of kernels this library has launched in the process so far (monotonic; kernels replayed through a CUDA graph the caller
@@ -313,6 +313,23 @@ int aq_mcts_root_counts(void *ws, int64_t G, int64_t max_nodes, int32_t *counts 
  * AQ_ERR_ARG for G < 1, max_nodes < 1 or a NULL pointer. */
 int aq_mcts_root_values(void *ws, int64_t G, int64_t max_nodes, double *root_value /*[G]*/, double *best_q /*[G]*/, int16_t *best_child /*[G]*/,
                         void *stream);
+/* Forced playouts and policy target pruning (KataGo: Wu 2019; the reference has neither).  A forced search runs
+ * aq_mcts_select_forced / aq_mcts_expand_select_forced in place of aq_mcts_select / aq_mcts_expand_select and reads its counts with
+ * aq_mcts_root_counts_pruned in place of aq_mcts_root_counts; both take forced_k >= 0 after c_puct.  With t = n_root - 1 (the sum of
+ * the root children's n), P_c the stored prior (noised if the root was noised) and k = (double)forced_k:
+ *   n_forced(c) = sqrt(k * P_c * t) in float64;  PUCT(c, m) = the select score with the visit count of U replaced by m
+ * The forced select leaves the root (expanded, not terminal) by the first child in legal_actions() order with n_c >= 1 and
+ * (double)n_c < n_forced(c), else by PUCT; every other node uses PUCT.  aq_mcts_root_counts_pruned writes what aq_mcts_root_counts
+ * writes, except the counts: c* (the first child with the largest n) keeps n_c*; every other child with n_c >= 1 starts from
+ * m = n_c and, while m >= 1, (double)(m - 1) >= (double)n_c - n_forced(c) and PUCT(c, m - 1) < PUCT(c*, n_c*), loses one; a child
+ * that was reduced and ends with m <= 1 gets 0.  k = 0 is the plain search and the plain counts; the most visited child never
+ * changes.  csrc/mcts.cu states the rounding exactly.  AQ_ERR_ARG as the plain entry points, and for forced_k < 0 or not finite. */
+int aq_mcts_select_forced(void *ws, int64_t G, int64_t max_nodes, float c_puct, float forced_k, AqState *leaf_states, int32_t *leaf_kind,
+                          void *stream);
+int aq_mcts_expand_select_forced(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values, const uint32_t *mask,
+                                 const uint8_t *pawn, float c_puct, float forced_k, AqState *leaf_states, int32_t *leaf_kind, void *stream);
+int aq_mcts_root_counts_pruned(void *ws, int64_t G, int64_t max_nodes, float c_puct, float forced_k, int32_t *counts /*[G,136]*/,
+                               int16_t *actions /*[G,136]*/, int16_t *n_children /*[G]*/, int32_t *overflow, void *stream);
 /* Dirichlet noise on the priors of every expanded, not yet noised root (AlphaZero; the reference has none).
  *   game_id [G] int64 (NULL: the row index), seed / ply: the key of the draw; alpha > 0, 0 <= fraction <= 1
  *   root_priors [G,136] f32 (may be NULL): the root's child priors after the call, legal_actions() order, 0 beyond n_children
