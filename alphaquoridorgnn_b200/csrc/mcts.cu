@@ -8,8 +8,9 @@
 // The reference has no virtual loss, no Dirichlet noise and no tree reuse, so batching ACROSS games
 // leaves every game's search unchanged.  Tree reuse between moves (aq_mcts_advance, AlphaGo Zero) and
 // Dirichlet noise on the root priors (aq_mcts_root_noise, AlphaZero) are opt-in additions the reference
-// does not have; without them every search starts from aq_mcts_reset with the network's priors.  So are the Gumbel root and KataGo's
-// forced playouts with policy target pruning (aq_mcts_select_forced, aq_mcts_root_counts_pruned).
+// does not have; without them every search starts from aq_mcts_reset with the network's priors.  So are the Gumbel root, KataGo's
+// forced playouts with policy target pruning (aq_mcts_select_forced, aq_mcts_root_counts_pruned) and KataGo's playout cap
+// randomization (aq_selfplay_partition, and the aq_mcts_*_rows entry points that search a prefix of the games).
 //
 // Arithmetic is kept as the reference computes it under NumPy >= 2 (requirements.txt pins
 // numpy~=2.0.2, NEP 50 promotion): w accumulates in float64; the PUCT score is
@@ -875,6 +876,60 @@ selfplay_compact_resign_kernel(const AqState *__restrict__ moved, const uint8_t 
 }
 
 // ------------------------------------------------------------------------------------------
+// Playout cap randomization (KataGo: David J. Wu, "Accelerating Self-Play Learning in Go", 2019, section 3.1; the reference has none).
+// The move of game `id` at `ply` gets a full search with probability full_prob, else a fast one:
+//   full iff u < full_prob,  u = (mix64(mix64((seed ^ kPcrDomain) + 0x9E3779B97F4A7C15 * (id + 1)) + 0xD1B54A32D192ED03 * (ply + 1))
+//                                 >> 11) * 2^-53
+// (the key of the noise and Gumbel draws with its own domain constant), so the draw depends on (seed, game, ply) alone.
+// ------------------------------------------------------------------------------------------
+constexpr uint64_t kPcrDomain = 0x082EFA98EC4E6C89ull;   // the fractional digits of pi after kResignDomain's
+
+__device__ __forceinline__ bool pcr_full(uint64_t seed, int64_t id, int ply, double full_prob) {
+    const uint64_t bits = mix64(mix64((seed ^ kPcrDomain) + 0x9E3779B97F4A7C15ull * (uint64_t)(id + 1)) + 0xD1B54A32D192ED03ull * (uint64_t)(ply + 1));
+    return (double)(bits >> 11) * 0x1p-53 < full_prob;
+}
+
+// Stable partition of rows [0, n) into full rows, then fast rows; one CTA, a block scan per 1,024 rows as selfplay_compact.  The
+// first pass counts the full rows, the second places full rows from 0 and fast rows from that count, each kind in input order.
+__global__ void __launch_bounds__(1024)
+selfplay_partition_kernel(const AqState *__restrict__ states, const int64_t *__restrict__ game_id, int64_t G, const int32_t *__restrict__ count,
+                          uint64_t seed, int ply, double full_prob, AqState *__restrict__ out_states, int64_t *__restrict__ out_game_id,
+                          int64_t *__restrict__ out_row, int32_t *__restrict__ full_count) {
+    __shared__ int warp_total[32];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int64_t n = count ? min((int64_t)max(*count, 0), G) : G;
+    int64_t full_total = 0;
+    for (int pass = 0; pass < 2; ++pass) {
+        int64_t base_full = 0, base_fast = full_total;
+        for (int64_t start = 0; start < n; start += 1024) {
+            const int64_t i = start + threadIdx.x;
+            const bool full = i < n && pcr_full(seed, game_id[i], ply, full_prob);
+            const unsigned m = __ballot_sync(0xffffffffu, full);
+            if (lane == 0) warp_total[w] = __popc(m);
+            __syncthreads();
+            int before = 0, all = 0;
+            for (int v = 0; v < 32; ++v) {
+                const int t = warp_total[v];
+                before += v < w ? t : 0;
+                all += t;
+            }
+            if (pass == 1 && i < n) {
+                const int full_before = before + __popc(m & ((1u << lane) - 1u));   // full rows of this chunk before row i
+                const int64_t o = full ? base_full + full_before : base_fast + (int)threadIdx.x - full_before;
+                store_state(out_states + o, load_state(states + i));
+                out_game_id[o] = game_id[i];
+                out_row[o] = i;
+            }
+            base_full += all;
+            base_fast += min(n - start, (int64_t)1024) - all;
+            __syncthreads();
+        }
+        full_total = base_full;
+    }
+    if (threadIdx.x == 0) *full_count = (int32_t)full_total;
+}
+
+// ------------------------------------------------------------------------------------------
 // Dirichlet noise on the root priors (AlphaZero; the reference has none).  For game g with K = n_children root children:
 //   eta ~ Dirichlet(alpha, ..., alpha),  p'_c = float32((1 - fraction) * (double)p_c + fraction * eta_c)  (double, rounded once)
 // eta is a pure function of (seed, game_id, ply, K, alpha).  Counter layout (tests/mcts_noise_oracle.py restates it):
@@ -1110,11 +1165,25 @@ extern "C" int aq_mcts_advance(const void *src_ws, int64_t G_src, void *dst_ws, 
                      max_nodes, roots, src_game, path, path_len, reserve_nodes, kept, status);
 }
 
+// The prefix entry points (_rows) run a kernel over the first `rows` games of a workspace laid out for G: the node pointers come from
+// G, the kernel's bound is `rows`.  The plain entry points are the same helpers with rows = G.
+static inline bool rows_ok(int64_t G, int64_t rows) { return G > 0 && rows >= 1 && rows <= G; }
+
+static int select_rows(const char *what, void *ws, int64_t G, int64_t rows, int64_t max_nodes, float c_puct, AqState *leaf_states,
+                       int32_t *leaf_kind, void *stream) {
+    if (!rows_ok(G, rows) || !ws || !leaf_states || !leaf_kind) return aq_set_error(AQ_ERR_ARG, what);
+    return aq_launch(what, mcts_select_kernel, (unsigned)((rows + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream), false,
+                     games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), rows, max_nodes, c_puct, leaf_states, leaf_kind);
+}
+
 extern "C" int aq_mcts_select(void *ws, int64_t G, int64_t max_nodes, float c_puct, AqState *leaf_states,
                               int32_t *leaf_kind, void *stream) {
-    if (G <= 0 || !ws || !leaf_states || !leaf_kind) return aq_set_error(AQ_ERR_ARG, "aq_mcts_select");
-    return aq_launch("aq_mcts_select", mcts_select_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream), false,
-                     games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, c_puct, leaf_states, leaf_kind);
+    return select_rows("aq_mcts_select", ws, G, G, max_nodes, c_puct, leaf_states, leaf_kind, stream);
+}
+
+extern "C" int aq_mcts_select_rows(void *ws, int64_t G, int64_t rows, int64_t max_nodes, float c_puct, AqState *leaf_states,
+                                   int32_t *leaf_kind, void *stream) {
+    return select_rows("aq_mcts_select_rows", ws, G, rows, max_nodes, c_puct, leaf_states, leaf_kind, stream);
 }
 
 extern "C" int aq_mcts_select_gumbel(void *ws, int64_t G, int64_t max_nodes, float c_puct, AqState *leaf_states,
@@ -1126,27 +1195,59 @@ extern "C" int aq_mcts_select_gumbel(void *ws, int64_t G, int64_t max_nodes, flo
 
 static inline bool forced_k_ok(float forced_k) { return forced_k >= 0.f && isfinite(forced_k); }
 
+static int select_forced_rows(const char *what, void *ws, int64_t G, int64_t rows, int64_t max_nodes, float c_puct, float forced_k,
+                              AqState *leaf_states, int32_t *leaf_kind, void *stream) {
+    if (!rows_ok(G, rows) || !ws || !leaf_states || !leaf_kind || !forced_k_ok(forced_k)) return aq_set_error(AQ_ERR_ARG, what);
+    return aq_launch(what, mcts_select_forced_kernel, (unsigned)((rows + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream), false,
+                     games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), rows, max_nodes, c_puct, (double)forced_k, leaf_states, leaf_kind);
+}
+
 extern "C" int aq_mcts_select_forced(void *ws, int64_t G, int64_t max_nodes, float c_puct, float forced_k, AqState *leaf_states,
                                      int32_t *leaf_kind, void *stream) {
-    if (G <= 0 || !ws || !leaf_states || !leaf_kind || !forced_k_ok(forced_k)) return aq_set_error(AQ_ERR_ARG, "aq_mcts_select_forced");
-    return aq_launch("aq_mcts_select_forced", mcts_select_forced_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream),
-                     false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, c_puct, (double)forced_k, leaf_states,
-                     leaf_kind);
+    return select_forced_rows("aq_mcts_select_forced", ws, G, G, max_nodes, c_puct, forced_k, leaf_states, leaf_kind, stream);
+}
+
+extern "C" int aq_mcts_select_forced_rows(void *ws, int64_t G, int64_t rows, int64_t max_nodes, float c_puct, float forced_k,
+                                          AqState *leaf_states, int32_t *leaf_kind, void *stream) {
+    return select_forced_rows("aq_mcts_select_forced_rows", ws, G, rows, max_nodes, c_puct, forced_k, leaf_states, leaf_kind, stream);
+}
+
+static int expand_backup_rows(const char *what, void *ws, int64_t G, int64_t rows, int64_t max_nodes, const float *priors,
+                              const float *values, const uint32_t *mask, const uint8_t *pawn, void *stream) {
+    if (!rows_ok(G, rows) || !ws || !priors || !values || !mask || !pawn) return aq_set_error(AQ_ERR_ARG, what);
+    return aq_launch(what, mcts_expand_backup_kernel, (unsigned)((rows + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream), false,
+                     games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), rows, max_nodes, priors, values, mask, pawn);
 }
 
 extern "C" int aq_mcts_expand_backup(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values,
                                      const uint32_t *mask, const uint8_t *pawn, void *stream) {
-    if (G <= 0 || !ws || !priors || !values || !mask || !pawn) return aq_set_error(AQ_ERR_ARG, "aq_mcts_expand_backup");
-    return aq_launch("aq_mcts_expand_backup", mcts_expand_backup_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream),
-                     false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, priors, values, mask, pawn);
+    return expand_backup_rows("aq_mcts_expand_backup", ws, G, G, max_nodes, priors, values, mask, pawn, stream);
+}
+
+extern "C" int aq_mcts_expand_backup_rows(void *ws, int64_t G, int64_t rows, int64_t max_nodes, const float *priors, const float *values,
+                                          const uint32_t *mask, const uint8_t *pawn, void *stream) {
+    return expand_backup_rows("aq_mcts_expand_backup_rows", ws, G, rows, max_nodes, priors, values, mask, pawn, stream);
+}
+
+static int expand_select_rows(const char *what, void *ws, int64_t G, int64_t rows, int64_t max_nodes, const float *priors,
+                              const float *values, const uint32_t *mask, const uint8_t *pawn, float c_puct, AqState *leaf_states,
+                              int32_t *leaf_kind, void *stream) {
+    if (!rows_ok(G, rows) || !ws || !priors || !values || !mask || !pawn || !leaf_states || !leaf_kind) return aq_set_error(AQ_ERR_ARG, what);
+    return aq_launch(what, mcts_expand_select_kernel, (unsigned)((rows + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream), false,
+                     games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), rows, max_nodes, priors, values, mask, pawn, c_puct, leaf_states,
+                     leaf_kind);
 }
 
 extern "C" int aq_mcts_expand_select(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values, const uint32_t *mask,
                                      const uint8_t *pawn, float c_puct, AqState *leaf_states, int32_t *leaf_kind, void *stream) {
-    if (G <= 0 || !ws || !priors || !values || !mask || !pawn || !leaf_states || !leaf_kind) return aq_set_error(AQ_ERR_ARG, "aq_mcts_expand_select");
-    return aq_launch("aq_mcts_expand_select", mcts_expand_select_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream),
-                     false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, priors, values, mask, pawn, c_puct, leaf_states,
-                     leaf_kind);
+    return expand_select_rows("aq_mcts_expand_select", ws, G, G, max_nodes, priors, values, mask, pawn, c_puct, leaf_states, leaf_kind, stream);
+}
+
+extern "C" int aq_mcts_expand_select_rows(void *ws, int64_t G, int64_t rows, int64_t max_nodes, const float *priors, const float *values,
+                                          const uint32_t *mask, const uint8_t *pawn, float c_puct, AqState *leaf_states, int32_t *leaf_kind,
+                                          void *stream) {
+    return expand_select_rows("aq_mcts_expand_select_rows", ws, G, rows, max_nodes, priors, values, mask, pawn, c_puct, leaf_states, leaf_kind,
+                              stream);
 }
 
 extern "C" int aq_mcts_expand_select_gumbel(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values,
@@ -1159,14 +1260,28 @@ extern "C" int aq_mcts_expand_select_gumbel(void *ws, int64_t G, int64_t max_nod
                      values, mask, pawn, c_puct, leaf_states, leaf_kind);
 }
 
+static int expand_select_forced_rows(const char *what, void *ws, int64_t G, int64_t rows, int64_t max_nodes, const float *priors,
+                                     const float *values, const uint32_t *mask, const uint8_t *pawn, float c_puct, float forced_k,
+                                     AqState *leaf_states, int32_t *leaf_kind, void *stream) {
+    if (!rows_ok(G, rows) || !ws || !priors || !values || !mask || !pawn || !leaf_states || !leaf_kind || !forced_k_ok(forced_k))
+        return aq_set_error(AQ_ERR_ARG, what);
+    return aq_launch(what, mcts_expand_select_forced_kernel, (unsigned)((rows + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream), false,
+                     games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), rows, max_nodes, priors, values, mask, pawn, c_puct,
+                     (double)forced_k, leaf_states, leaf_kind);
+}
+
 extern "C" int aq_mcts_expand_select_forced(void *ws, int64_t G, int64_t max_nodes, const float *priors, const float *values,
                                             const uint32_t *mask, const uint8_t *pawn, float c_puct, float forced_k, AqState *leaf_states,
                                             int32_t *leaf_kind, void *stream) {
-    if (G <= 0 || !ws || !priors || !values || !mask || !pawn || !leaf_states || !leaf_kind || !forced_k_ok(forced_k))
-        return aq_set_error(AQ_ERR_ARG, "aq_mcts_expand_select_forced");
-    return aq_launch("aq_mcts_expand_select_forced", mcts_expand_select_forced_kernel, (unsigned)((G + 3) / 4), 128, 0,
-                     reinterpret_cast<cudaStream_t>(stream), false, games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, priors,
-                     values, mask, pawn, c_puct, (double)forced_k, leaf_states, leaf_kind);
+    return expand_select_forced_rows("aq_mcts_expand_select_forced", ws, G, G, max_nodes, priors, values, mask, pawn, c_puct, forced_k,
+                                     leaf_states, leaf_kind, stream);
+}
+
+extern "C" int aq_mcts_expand_select_forced_rows(void *ws, int64_t G, int64_t rows, int64_t max_nodes, const float *priors,
+                                                 const float *values, const uint32_t *mask, const uint8_t *pawn, float c_puct, float forced_k,
+                                                 AqState *leaf_states, int32_t *leaf_kind, void *stream) {
+    return expand_select_forced_rows("aq_mcts_expand_select_forced_rows", ws, G, rows, max_nodes, priors, values, mask, pawn, c_puct, forced_k,
+                                     leaf_states, leaf_kind, stream);
 }
 
 extern "C" int aq_mcts_root_counts_pruned(void *ws, int64_t G, int64_t max_nodes, float c_puct, float forced_k, int32_t *counts,
@@ -1201,13 +1316,23 @@ extern "C" int aq_mcts_root_values(void *ws, int64_t G, int64_t max_nodes, doubl
                      false, hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, root_value, best_q, best_child);
 }
 
+static int root_noise_rows(const char *what, void *ws, int64_t G, int64_t rows, int64_t max_nodes, const int64_t *game_id, uint64_t seed,
+                           int32_t ply, float alpha, float fraction, float *root_priors, void *stream) {
+    if (!rows_ok(G, rows) || max_nodes < 1 || !ws || !(alpha > 0.f) || !isfinite(alpha) || !(fraction >= 0.f && fraction <= 1.f))
+        return aq_set_error(AQ_ERR_ARG, what);
+    return aq_launch(what, mcts_root_noise_kernel, (unsigned)((rows + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream), false,
+                     games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), rows, max_nodes, game_id, seed, (int)ply, (double)alpha,
+                     (double)fraction, root_priors);
+}
+
 extern "C" int aq_mcts_root_noise(void *ws, int64_t G, int64_t max_nodes, const int64_t *game_id, uint64_t seed, int32_t ply, float alpha,
                                   float fraction, float *root_priors, void *stream) {
-    if (G < 1 || max_nodes < 1 || !ws || !(alpha > 0.f) || !isfinite(alpha) || !(fraction >= 0.f && fraction <= 1.f))
-        return aq_set_error(AQ_ERR_ARG, "aq_mcts_root_noise");
-    return aq_launch("aq_mcts_root_noise", mcts_root_noise_kernel, (unsigned)((G + 3) / 4), 128, 0, reinterpret_cast<cudaStream_t>(stream), false,
-                     games_of(ws), hot_of(ws, G), cold_of(ws, G, max_nodes), G, max_nodes, game_id, seed, (int)ply, (double)alpha,
-                     (double)fraction, root_priors);
+    return root_noise_rows("aq_mcts_root_noise", ws, G, G, max_nodes, game_id, seed, ply, alpha, fraction, root_priors, stream);
+}
+
+extern "C" int aq_mcts_root_noise_rows(void *ws, int64_t G, int64_t rows, int64_t max_nodes, const int64_t *game_id, uint64_t seed,
+                                       int32_t ply, float alpha, float fraction, float *root_priors, void *stream) {
+    return root_noise_rows("aq_mcts_root_noise_rows", ws, G, rows, max_nodes, game_id, seed, ply, alpha, fraction, root_priors, stream);
 }
 
 extern "C" int aq_mcts_gumbel_root(void *ws, int64_t G, int64_t max_nodes, const int64_t *game_id, uint64_t seed, int32_t ply,
@@ -1319,4 +1444,14 @@ extern "C" int aq_selfplay_advance_resign(const AqState *states, const int32_t *
     return selfplay_advance<true, true>("aq_selfplay_advance_resign(move)", "aq_selfplay_advance_resign(compact)", states, nullptr, child_policy,
                                         choice, actions, n_children, game_id, G, 1.0, seed, ply, policy, policy_f64, chosen, r, next_states,
                                         next_game_id, final_flags, final_plies, alive_count, workspace, st);
+}
+
+extern "C" int aq_selfplay_partition(const AqState *states, const int64_t *game_id, int64_t G, const int32_t *count, uint64_t seed, int32_t ply,
+                                     double full_prob, AqState *out_states, int64_t *out_game_id, int64_t *out_row, int32_t *full_count,
+                                     void *stream) {
+    if (G < 1 || G > INT32_MAX || !states || !game_id || !(full_prob >= 0.0 && full_prob <= 1.0) || !out_states || !out_game_id || !out_row ||
+        !full_count)
+        return aq_set_error(AQ_ERR_ARG, "aq_selfplay_partition");
+    return aq_launch("aq_selfplay_partition", selfplay_partition_kernel, 1, 1024, 0, reinterpret_cast<cudaStream_t>(stream), false, states,
+                     game_id, G, count, seed, (int)ply, full_prob, out_states, out_game_id, out_row, full_count);
 }

@@ -13,6 +13,8 @@ So is the Gumbel root of Gumbel AlphaZero, BatchedMCTS(..., gumbel_considered=16
 root children and a completed-Q improved policy; the default keeps PUCT at the root.
 Forced playouts with policy target pruning (KataGo), BatchedMCTS(..., forced_k=2.0), give every visited root child at least
 sqrt(k * P * sum N) visits and take the surplus back out of the counts the search returns; the default returns the plain counts.
+Playout cap randomization (KataGo), search(..., fast_sims=50, full_rows=F), gives rows [0, F) the full search and the others a
+cheap one of fast_sims simulations without root noise; the default gives every row the full search.
 """
 import math
 from copy import deepcopy
@@ -28,6 +30,11 @@ PV_EVALUATE_COUNT = 50  # Number of simulations per inference (pv_mcts.py:18)
 C_PUCT = 1.25           # pv_mcts.py:71
 MAX_CHILDREN = 133      # 5 pawn moves + 128 wall placements
 GRAPH_CHUNK = 25        # simulations per launch of the chunk graph (BatchedMCTS.search)
+
+
+def _padded(n):
+    """Batch size a search of n rows runs at when it pads (network evaluator, graphs on, n > 256): the next multiple of 256."""
+    return n if n <= 256 or n % 256 == 0 else n + 256 - n % 256
 
 
 def network_evaluator(model):
@@ -68,7 +75,20 @@ class BatchedMCTS:
     most visited one loses the visits, up to n_forced, that PUCT would not have given it against that child, and a child left with
     one visit goes to 0.  The most visited child keeps its count, so temperature 0 and root_values() see the same move.  It pairs
     with dirichlet_alpha (the forced visits then explore the noise without training on it) and tree_reuse (carried visits count in
-    t), not with gumbel_considered.  forced_k=0 is the plain search; None (the default) runs exactly it."""
+    t), not with gumbel_considered.  forced_k=0 is the plain search; None (the default) runs exactly it.
+
+    search(..., fast_sims, full_rows) (playout cap randomization, KataGo: Wu 2019, section 3.1; the reference has none): rows
+    [0, full_rows) get the full search of `sims` new simulations with the configured root noise, and the other rows a fast search of
+    fast_sims new simulations without root noise; a fast row's result is exactly that of this searcher's search with
+    dirichlet_alpha=None and fast_sims simulations.  Fast rows keep the select rule and the counts of the searcher: with forced_k they
+    force root playouts and return pruned counts too (KataGo turns forced playouts off for its cheap searches; here one select rule
+    serves every row of a launch, and without noise the rule finds little to force).  Every tree is started (reset or advance), the
+    full rows' roots are noised before and after simulation 1, then phase A runs fast_sims simulations on every row and phase B the
+    other sims - fast_sims on the full rows alone, through the prefix entry points (aq_mcts_*_rows); the counts are read for every
+    row.  When the search pads (network evaluator, graphs, more than 256 rows), its rows are laid out as [full rows | copies of the
+    last full root up to the padded size of the full-row count | fast rows | padding], so that phase B is replayed from graphs
+    captured for a few sizes; outputs, last_kept and root_values() are in the caller's order all the same.  It cannot be combined
+    with gumbel_considered, whose schedule depends on the budget."""
 
     def __init__(self, evaluator, sims=None, c_puct=C_PUCT, device=None, use_graph=True, tree_reuse=False, dirichlet_alpha=None,
                  noise_fraction=0.25, gumbel_considered=None, gumbel_scale=1.0, forced_k=None):
@@ -109,8 +129,10 @@ class BatchedMCTS:
         self.last_choice = None  # gumbel_considered: int16[G] child chosen by the last search, else None
         self._ws = [None, None] if self.tree_reuse else [None]
         self._last = None     # tree_reuse: (workspace slot, G) of the previous search, the source a next search can continue
+        self._last_rows = None  # tree_reuse: the workspace row of each caller row of the previous search when it is not that row
         self.last_kept = None  # tree_reuse: int32[G] nodes carried into each row by the last search (0 = fresh root), else None
         self._root = None      # (workspace, G, real rows, max_nodes) of the last search: what root_values() reads
+        self._root_rows = None  # the workspace row of each caller row of the last search when it is not that row (None: row r is row r)
         self._buf = {}
         self._graphs = {}
         self._warm = set()   # step modes (the last item of a graph key: "puct", "gumbel" or "forced") whose lazy initialisation an
@@ -141,26 +163,31 @@ class BatchedMCTS:
             }
         return self._buf[G]
 
-    def _step(self, ws, G, max_nodes, buf, evaluate, st, steps=1, gumbel=False, forced=False):
+    def _step(self, ws, G, max_nodes, buf, evaluate, st, steps=1, gumbel=False, forced=False, rows=None):
         """`steps` simulations for all games: select, then `steps` leaf evaluations out = evaluate(stream) (terminal leaves are
         evaluated too and ignored by the backup) joined by the fused expand + backup + next select, then the last expand + backup.
-        gumbel: the selects leave a Gumbel root by the Gumbel rule; forced: the root by the forced-playout rule (forced_k)."""
+        gumbel: the selects leave a Gumbel root by the Gumbel rule; forced: the root by the forced-playout rule (forced_k).
+        rows: the simulations run for games [0, rows) only, through the prefix entry points (aq_mcts_*_rows)."""
         L, P = _lib.load(), _lib.ptr
         if forced:
             k = (self.forced_k,)
-            select, expand_select = L.aq_mcts_select_forced, L.aq_mcts_expand_select_forced
+            select, expand_select = ((L.aq_mcts_select_forced, L.aq_mcts_expand_select_forced) if rows is None else
+                                     (L.aq_mcts_select_forced_rows, L.aq_mcts_expand_select_forced_rows))
         else:
             k = ()
             select, expand_select = ((L.aq_mcts_select_gumbel, L.aq_mcts_expand_select_gumbel) if gumbel else
-                                     (L.aq_mcts_select, L.aq_mcts_expand_select))
-        _lib.check(select(P(ws), G, max_nodes, self.c_puct, *k, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_select")
+                                     (L.aq_mcts_select, L.aq_mcts_expand_select) if rows is None else
+                                     (L.aq_mcts_select_rows, L.aq_mcts_expand_select_rows))
+        expand_backup = L.aq_mcts_expand_backup if rows is None else L.aq_mcts_expand_backup_rows
+        dims = (G,) if rows is None else (G, rows)
+        _lib.check(select(P(ws), *dims, max_nodes, self.c_puct, *k, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_select")
         for i in range(steps):
             out = evaluate(st)
-            leaves = (P(ws), G, max_nodes, P(out["priors"]), P(out["value"]), P(out["mask"]), P(out["pawn"]))
+            leaves = (P(ws), *dims, max_nodes, P(out["priors"]), P(out["value"]), P(out["mask"]), P(out["pawn"]))
             if i + 1 < steps:
                 _lib.check(expand_select(*leaves, self.c_puct, *k, P(buf["leaf"]), P(buf["kind"]), st), "aq_mcts_expand_select")
             else:
-                _lib.check(L.aq_mcts_expand_backup(*leaves, st), "aq_mcts_expand_backup")
+                _lib.check(expand_backup(*leaves, st), "aq_mcts_expand_backup")
 
     def _simulate(self, n, step, key, st):
         """n simulations; step(stream, k) enqueues k of them.  With a graph key (network evaluator) and use_graph, they are replays of
@@ -198,7 +225,7 @@ class BatchedMCTS:
             step(st, 1)
 
     @torch.no_grad()
-    def search_async(self, roots, sims=None, src_row=None, path=None, noise_seed=None, game_id=None, ply=0):
+    def search_async(self, roots, sims=None, src_row=None, path=None, noise_seed=None, game_id=None, ply=0, fast_sims=None, full_rows=None):
         """search() without the synchronisation: returns (counts, actions, n_children, status int32[3] on the device); the caller
         passes status.tolist() to check_status() when it synchronises anyway."""
         sims = sims or self.sims or PV_EVALUATE_COUNT
@@ -215,21 +242,54 @@ class BatchedMCTS:
                 raise ValueError("search(src_row=...) needs the path of actions from each source root")
         if self.tree_reuse and sims > self.sims:
             raise ValueError(f"this searcher's node arena holds {self.sims} simulations per search, not {sims}")
+        pcr = fast_sims is not None
+        if pcr:
+            if isinstance(fast_sims, bool) or int(fast_sims) != fast_sims or not 1 <= fast_sims <= sims:
+                raise ValueError(f"fast_sims must be an integer in [1, sims = {sims}] (or None), not {fast_sims!r}")
+            if self.gumbel_considered is not None:
+                raise ValueError("fast_sims cannot be combined with gumbel_considered: the Gumbel schedule depends on the budget")
+            full = G_real if full_rows is None else full_rows
+            if isinstance(full, bool) or int(full) != full or not 0 <= full <= G_real:
+                raise ValueError(f"full_rows must be an integer in [0, {G_real}] (or None), not {full_rows!r}")
+            fast_sims, full = int(fast_sims), int(full)
+        elif full_rows is not None:
+            raise ValueError("search(full_rows=...) splits full and fast searches: it needs fast_sims")
         if G_real == 0:
             self.last_kept = self.last_policy = self.last_choice = None
-            self._root = (None, 0, 0, 0)
+            self._root, self._root_rows = (None, 0, 0, 0), None
             return (torch.empty((0, gl.MAX_LEGAL), dtype=torch.int32, device=dev), torch.empty((0, gl.MAX_LEGAL), dtype=torch.int16, device=dev),
                     torch.empty((0,), dtype=torch.int16, device=dev), torch.zeros((3,), dtype=torch.int32, device=dev))
         # Self-play and the arena drop finished games, so the number of roots shrinks by a few almost every ply.  Batches above 256
         # are padded to the next multiple of 256 with copies of the last root (searched and discarded; games are independent, so the
         # real ones are unaffected): workspaces, buffers and the captured CUDA graph of the simulation step are then reused across
         # plies instead of being rebuilt for every distinct size.
-        if self.model is not None and self.use_graph and G_real > 256 and G_real % 256:
+        rows = None   # the workspace row of each caller row, when it is not that row
+        pads = self.model is not None and self.use_graph and G_real > 256
+        if pcr and pads:
+            # [full rows | copies of the last full root up to _padded(full) | fast rows | copies of the last root up to a multiple of
+            # 256]: the full-row prefix that phase B searches has a padded size too, so its graphs are reused across plies as well
+            full_pad = _padded(full)
+            G = _padded(full_pad + G_real - full)
+            if G > G_real:
+                rows = torch.cat([torch.arange(full, device=dev), torch.arange(full_pad, full_pad + G_real - full, device=dev)])
+                src = torch.full((G,), G_real - 1, dtype=torch.int64, device=dev)
+                src[:full_pad] = full - 1
+                src[rows] = torch.arange(G_real, device=dev)
+                roots = roots[src].contiguous()
+            full = full_pad
+        elif pads and G_real % 256:
             roots = torch.cat([roots, roots[-1:].expand(256 - G_real % 256, -1)]).contiguous()
         G = roots.shape[0]
 
         def pad(t, fill):   # a per-game argument for the padded rows: they start fresh (src_row -1) and draw the noise of game 0
+            if rows is not None:
+                out = t.new_full((G,) + t.shape[1:], fill)
+                out[rows] = t
+                return out
             return (torch.cat([t, t.new_full((G - G_real,) + t.shape[1:], fill)]) if G > G_real else t).contiguous()
+
+        def real(t):        # the caller's rows of a per-game output
+            return t[:G_real] if rows is None else t[rows]
 
         max_nodes = 1 + (2 * self.sims if self.tree_reuse else sims) * MAX_CHILDREN
         slot = 0 if self._last is None else 1 - self._last[0]
@@ -241,17 +301,21 @@ class BatchedMCTS:
             st = _lib.stream_ptr(dev)
             if src_row is not None:
                 src_slot, G_src = self._last
-                src = pad(src_row.to(device=dev, dtype=torch.int64).reshape(G_real), -1)
+                src = src_row.to(device=dev, dtype=torch.int64).reshape(G_real)
+                if self._last_rows is not None:   # caller rows of the previous search -> its workspace rows (out of range stays so)
+                    n_prev = self._last_rows.shape[0]
+                    src = torch.where(src < 0, src, torch.where(src < n_prev, self._last_rows[src.clamp(0, n_prev - 1)], src - n_prev + G_src))
+                src = pad(src, -1)
                 path = pad(path.to(device=dev, dtype=torch.int16).reshape(G_real, -1), 0)
                 kept = torch.empty((G,), dtype=torch.int32, device=dev)
                 _lib.check(L.aq_mcts_advance(P(self._ws[src_slot]), G_src, P(ws), G, max_nodes, P(roots), P(src), P(path), path.shape[1],
                                              sims * MAX_CHILDREN, P(kept), P(status[2:]), st), "aq_mcts_advance")
-                self.last_kept = kept[:G_real]
+                self.last_kept = real(kept)
             else:
                 _lib.check(L.aq_mcts_reset(P(ws), P(roots), G, max_nodes, st), "aq_mcts_reset")
                 self.last_kept = None
             if self.tree_reuse:
-                self._last = (slot, G)
+                self._last, self._last_rows = (slot, G), rows
             if self.model is not None:
                 from .pv_network_gnn import PRECISIONS
                 flat = self.model.flat_parameters()
@@ -260,10 +324,13 @@ class BatchedMCTS:
                 prep = self.model.prepared_weights() if prec == 1 else None
                 key = (G, max_nodes, ws.data_ptr(), flat.data_ptr(), prep.data_ptr() if prep is not None else 0, prec, self._mode)
 
-                def evaluate(s):
-                    _lib.check(L.aq_leaf_eval(P(flat), P(prep), P(buf["leaf"]), G, P(buf["priors"]), P(buf["value"]), P(buf["mask"]),
-                                              P(buf["pawn"]), P(buf["pooled"]), prec, s), "aq_leaf_eval")
-                    return buf
+                def evaluate_rows(n):
+                    def evaluate(s):
+                        _lib.check(L.aq_leaf_eval(P(flat), P(prep), P(buf["leaf"]), n, P(buf["priors"]), P(buf["value"]), P(buf["mask"]),
+                                                  P(buf["pawn"]), P(buf["pooled"]), prec, s), "aq_leaf_eval")
+                        return buf
+                    return evaluate
+                evaluate = evaluate_rows(G)
             else:
                 key, evaluate = None, lambda s: self.evaluator(buf["leaf"])
             step = lambda s, k: self._step(ws, G, max_nodes, buf, evaluate, s, k, forced=self.forced_k is not None)
@@ -271,7 +338,19 @@ class BatchedMCTS:
                 seed = (int(torch.randint(0, 2 ** 63 - 1, (1,)).item()) if noise_seed is None else int(noise_seed)) & (2 ** 64 - 1)
                 gid = None if game_id is None else pad(game_id.to(device=dev, dtype=torch.int64).reshape(G_real), 0)
             self.last_policy = self.last_choice = None
-            if self.gumbel_considered is not None:
+            if pcr:
+                # Phase A: fast_sims simulations of every row; phase B: sims - fast_sims more of the full rows [0, full) alone.  Only the
+                # full rows are noised, at the same two points as a search without playout cap randomization.
+                for n in ((1, fast_sims - 1) if self.dirichlet_alpha is not None else (fast_sims,)):
+                    if self.dirichlet_alpha is not None and full:
+                        _lib.check(L.aq_mcts_root_noise_rows(P(ws), G, full, max_nodes, P(gid), seed, int(ply), self.dirichlet_alpha,
+                                                             self.noise_fraction, None, st), "aq_mcts_root_noise_rows")
+                    self._simulate(n, step, key, st)
+                if full and sims > fast_sims:
+                    evaluate_b = evaluate_rows(full) if self.model is not None else lambda s: self.evaluator(buf["leaf"][:full])
+                    step_b = lambda s, k: self._step(ws, G, max_nodes, buf, evaluate_b, s, k, forced=self.forced_k is not None, rows=full)
+                    self._simulate(sims - fast_sims, step_b, None if key is None else key[:-1] + (full, self._mode + "-rows"), st)
+            elif self.gumbel_considered is not None:
                 # simulation 1 expands the root, aq_mcts_gumbel_root draws its Gumbel state, the other sims - 1 descend by its rule
                 self._simulate(1, step, key, st)
                 _lib.check(L.aq_mcts_gumbel_root(P(ws), G, max_nodes, P(gid), seed, int(ply), self.gumbel_considered, self.gumbel_scale,
@@ -302,8 +381,8 @@ class BatchedMCTS:
                                                         P(status[:1]), st), "aq_mcts_root_counts_pruned")
             if self.model is not None:
                 status[1:2].copy_(torch.isnan(buf["value"]).any().reshape(1))
-        self._root = (ws, G, G_real, max_nodes)
-        return counts[:G_real], actions[:G_real], n[:G_real], status
+        self._root, self._root_rows = (ws, G, G_real, max_nodes), rows
+        return real(counts), real(actions), real(n), status
 
     @torch.no_grad()
     def root_values(self):
@@ -323,6 +402,8 @@ class BatchedMCTS:
             with torch.cuda.device(dev):
                 _lib.check(_lib.load().aq_mcts_root_values(P(ws), G, max_nodes, P(root_value), P(best_q), P(best_child), _lib.stream_ptr(dev)),
                            "aq_mcts_root_values")
+        if self._root_rows is not None:
+            return root_value[self._root_rows], best_q[self._root_rows]
         return root_value[:G_real], best_q[:G_real]
 
     @staticmethod
@@ -337,7 +418,7 @@ class BatchedMCTS:
             raise _lib.AqError("the network returned NaN for a leaf: with precision 'bf16' that is how an activation beyond the fp16 range of the "
                                "aggregation operand is reported (gnn_tc2.cu); evaluate this network with precision 'fp32'")
 
-    def search(self, roots, sims=None, src_row=None, path=None, noise_seed=None, game_id=None, ply=0):
+    def search(self, roots, sims=None, src_row=None, path=None, noise_seed=None, game_id=None, ply=0, fast_sims=None, full_rows=None):
         """roots: packed uint8[G,32] (non-terminal states).  Runs `sims` simulations per game
         (pv_mcts.py:84) and returns (counts int32[G,136], actions int16[G,136], n_children int16[G]):
         visit counts of the root's children in State.legal_actions() order (pv_mcts.py:88).
@@ -350,8 +431,11 @@ class BatchedMCTS:
         With dirichlet_alpha, the root noise of row g is drawn from (noise_seed, game_id[g], ply): game_id int64[G] (None = the row
         index) names the game, so a game's noise does not depend on the other rows; noise_seed None draws one from torch's generator.
 
-        With forced_k, the counts are the pruned counts (aq_mcts_root_counts_pruned); the tree keeps the visits it made."""
-        counts, actions, n, status = self.search_async(roots, sims, src_row, path, noise_seed, game_id, ply)
+        With forced_k, the counts are the pruned counts (aq_mcts_root_counts_pruned); the tree keeps the visits it made.
+
+        With fast_sims (playout cap randomization), rows [0, full_rows) (None: all) get the full search above and the other rows a
+        fast one: exactly the search of this searcher with dirichlet_alpha=None and fast_sims simulations.  See the class docstring."""
+        counts, actions, n, status = self.search_async(roots, sims, src_row, path, noise_seed, game_id, ply, fast_sims, full_rows)
         self.check_status(status.tolist())   # one synchronisation for both flags
         return counts, actions, n
 

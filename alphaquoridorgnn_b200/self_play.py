@@ -44,12 +44,13 @@ def write_data(history, directory='./data/'):
 @torch.no_grad()
 def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_TEMPERATURE, seed=None, max_plies=None,
                       policy_dtype=torch.float64, tree_reuse=False, dirichlet_alpha=None, noise_fraction=0.25, gumbel_considered=None,
-                      gumbel_scale=1.0, resign_threshold=None, resign_calibration=0.1, forced_k=None):
+                      gumbel_scale=1.0, resign_threshold=None, resign_calibration=0.1, forced_k=None, fast_sims=None, full_search_prob=0.25):
     """Execute `num_games` self-play games in lock-step (self_play.py:40-68 per game) and keep the record on the device:
     dict(states uint8[T,32] packed, policy [T,209] search policies over all actions (self_play.py:51-54), value f32[T]
     back-filled game results seen from the player to move (self_play.py:63-66), game int64[T], ply int64[T],
     flags uint8[G] (bit 0 = the player to move at the end has lost, bit 1 = draw), plies int64[G], sims int = new simulations
-    run, reused int = searches that continued a carried tree).
+    run, reused int = searches that continued a carried tree, full_searches / fast_searches int = searches with `sims` / fast_sims
+    new simulations).
 
     Per ply: one search (200 graph-replayed simulation steps in a handful of launches) and ONE library call,
     aq_selfplay_advance -- search policy, its dense 209-wide record, the sampled move, the next states and the compaction of the
@@ -80,7 +81,18 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
     forced_k (KataGo's forced playouts and policy target pruning; the reference has none): every search forces visits to its
     visited root children (BatchedMCTS) and returns pruned counts, and the ply records and draws its move from those.  It is meant
     to pair with dirichlet_alpha: the noise still explores, but the visits it forced are taken out of the policy target.  The
-    record format, the value targets and resignation are the same (the most visited child is never pruned)."""
+    record format, the value targets and resignation are the same (the most visited child is never pruned).
+
+    fast_sims (KataGo's playout cap randomization; the reference has none): each move of each game is full with probability
+    full_search_prob, drawn from (seed, game, ply) alone (aq_selfplay_partition), else fast.  A full move searches with `sims` new
+    simulations and the configured root noise and forced playouts, and its position is recorded; a fast move searches with
+    fast_sims new simulations without root noise (BatchedMCTS.search(fast_sims=...); with forced_k it still forces and prunes, unlike
+    KataGo's cheap searches), plays its move as any other and is not recorded: neither a policy nor a value target.  Per ply: the
+    partition of the games into full and fast rows (at ply 0 on the start states, which costs one synchronisation before the first
+    ply; later at the end of the previous ply), the search, the move, and the one synchronisation, which also reads the number of full
+    rows.  The record holds only the full positions, with their real ply; the value targets follow from the game results as ever.
+    It combines with tree_reuse, dirichlet_alpha, forced_k and resignation (every game may resign after a full or a fast search),
+    not with gumbel_considered.  None (the default) searches every move in full."""
     if policy_dtype not in (torch.float64, torch.float32):
         raise ValueError("policy_dtype must be torch.float64 or torch.float32")
     if resign_threshold is not None:
@@ -88,15 +100,24 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
             raise ValueError("resign_threshold must be a number (or None), not NaN")
         if not 0.0 <= resign_calibration <= 1.0:
             raise ValueError(f"resign_calibration must be in [0, 1], not {resign_calibration!r}")
+    sims = sims or pv_mcts.PV_EVALUATE_COUNT
+    pcr = fast_sims is not None
+    if pcr:
+        if isinstance(fast_sims, bool) or int(fast_sims) != fast_sims or not 1 <= fast_sims <= sims:
+            raise ValueError(f"fast_sims must be an integer in [1, sims = {sims}] (or None), not {fast_sims!r}")
+        if not 0.0 <= full_search_prob <= 1.0:
+            raise ValueError(f"full_search_prob must be in [0, 1], not {full_search_prob!r}")
+        if gumbel_considered is not None:
+            raise ValueError("fast_sims cannot be combined with gumbel_considered: the Gumbel schedule depends on the budget")
+        fast_sims = int(fast_sims)
     dev = gl._dev(device)
     L, P = _lib.load(), _lib.ptr
     seed = (int(seed) if seed is not None else int(torch.seed())) & (2 ** 64 - 1)
-    sims = sims or pv_mcts.PV_EVALUATE_COUNT
     mcts = pv_mcts.searcher_for(model, sims, dev, tree_reuse=tree_reuse, dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction,
                                 gumbel_considered=gumbel_considered, gumbel_scale=gumbel_scale, forced_k=forced_k)
     states = start_states(num_games, dev)
     game_id = torch.arange(num_games, device=dev)
-    rec_state, rec_policy, rec_game, sizes = [], [], [], []
+    rec_state, rec_policy, rec_game, sizes, searched = [], [], [], [], []
     final_flags = torch.zeros(max(num_games, 1), dtype=torch.uint8, device=dev)
     final_plies = torch.zeros(max(num_games, 1), dtype=torch.int64, device=dev)
     ws = torch.empty((max(1, L.aq_selfplay_ws_bytes(num_games)),), dtype=torch.uint8, device=dev)
@@ -105,13 +126,29 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
     if resign:
         resign_min = torch.full((max(num_games, 1), 2), math.inf, dtype=torch.float64, device=dev)
         calibration = torch.zeros(max(num_games, 1), dtype=torch.uint8, device=dev)   # written by the kernel for every game it plays
-    ply, sims_run, reused = 0, 0, 0
+    ply, sims_run, reused, full_searches = 0, 0, 0, 0
     src_row = path = None
+    full = None   # pcr: the number of full rows of the ply, which come first
+    if pcr:
+        full_count = torch.zeros((1,), dtype=torch.int32, device=dev)
+        row_of = torch.empty(max(num_games, 1), dtype=torch.int64, device=dev)   # tree_reuse: a game's row in the last search
+
+        def partition(st, gid, G, count, at_ply):   # -> the rows reordered full first, their input rows; full_count is written
+            out, out_id, out_row = torch.empty_like(st), torch.empty_like(gid), torch.empty_like(gid)
+            _lib.check(L.aq_selfplay_partition(P(st), P(gid), G, P(count), seed, at_ply, float(full_search_prob), P(out), P(out_id),
+                                               P(out_row), P(full_count), _lib.stream_ptr(dev)), "aq_selfplay_partition")
+            return out, out_id, out_row
+        if num_games:
+            with torch.cuda.device(dev):
+                states, game_id, _ = partition(states, game_id, num_games, None, 0)
+            full = int(full_count.item())
     with torch.cuda.device(dev):
         while states.shape[0] > 0 and (max_plies is None or ply < max_plies):
             G = states.shape[0]
-            counts, actions, n, status = mcts.search_async(states, src_row=src_row, path=path, noise_seed=seed, game_id=game_id, ply=ply)
-            sims_run += G * sims
+            counts, actions, n, status = mcts.search_async(states, src_row=src_row, path=path, noise_seed=seed, game_id=game_id, ply=ply,
+                                                           fast_sims=fast_sims, full_rows=full)
+            sims_run += G * sims if full is None else full * sims + (G - full) * fast_sims
+            full_searches += G if full is None else full
             dense = torch.empty((G, POLICY_OUTPUT_SIZE), dtype=policy_dtype, device=dev)
             nxt = torch.empty_like(states)
             nxt_id = torch.empty_like(game_id)
@@ -137,19 +174,31 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
             parts = [status, alive]
             if mcts.last_kept is not None:
                 parts.append((mcts.last_kept > 0).sum(dtype=torch.int32).reshape(1))
+            if pcr:   # the next ply's partition, on the survivors
+                nxt, nxt_id, _ = partition(nxt, nxt_id, G, alive, ply + 1)
+                parts.append(full_count)
             flags = torch.cat(parts).tolist()      # the ply's only synchronisation
             mcts.check_status(flags[:3])
-            reused += flags[4] if len(flags) > 4 else 0
-            rec_state.append(states)
-            rec_policy.append(dense)
-            rec_game.append(game_id)
-            sizes.append(G)
+            reused += flags[4] if mcts.last_kept is not None else 0
+            keep = G if full is None else full     # pcr: only the full rows are recorded
+            rec_state.append(states[:keep])
+            rec_policy.append(dense[:keep])
+            rec_game.append(game_id[:keep])
+            sizes.append(keep)
+            searched.append(G)
             ply += 1
             if tree_reuse:
-                # the compaction keeps game_id ascending, so a survivor's previous row is found by binary search
-                src_row = torch.searchsorted(game_id, nxt_id[:flags[3]])
+                if pcr:
+                    # the partition reorders the games, so a survivor's previous row is looked up by its game id
+                    row_of[game_id] = torch.arange(G, device=dev)
+                    src_row = row_of[nxt_id[:flags[3]]]
+                else:
+                    # the compaction keeps game_id ascending, so a survivor's previous row is found by binary search
+                    src_row = torch.searchsorted(game_id, nxt_id[:flags[3]])
                 path = chosen[src_row].reshape(-1, 1)
             states, game_id = nxt[:flags[3]], nxt_id[:flags[3]]
+            if pcr:
+                full = flags[-1]
     extra = {}
     if resign:
         extra = {"resign_min": resign_min[:num_games], "calibration": calibration[:num_games] != 0}
@@ -157,7 +206,8 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
         z = torch.zeros((0,), dtype=torch.int64, device=dev)
         return {"states": states, "policy": torch.zeros((0, POLICY_OUTPUT_SIZE), dtype=policy_dtype, device=dev),
                 "value": torch.zeros((0,), dtype=torch.float32, device=dev), "game": z, "ply": z, "flags": final_flags[:num_games],
-                "plies": final_plies[:num_games], "sims": 0, "reused": 0, **extra}
+                "plies": final_plies[:num_games], "sims": 0, "reused": 0, "full_searches": 0, "fast_searches": 0, **extra}
+    sum_searches = sum(searched)
     game = torch.cat(rec_game)
     plyv = torch.repeat_interleave(torch.arange(len(sizes), device=dev), torch.tensor(sizes, device=dev))
     final_flags, final_plies = final_flags[:num_games], final_plies[:num_games]
@@ -167,7 +217,8 @@ def play_batch_device(model, num_games, device=None, sims=None, temperature=SP_T
     fpv = torch.where(lost, torch.where(final_plies[game] % 2 == 0, -1.0, 1.0), 0.0)
     value = torch.where(plyv % 2 == 0, fpv, -fpv).to(torch.float32)
     return {"states": torch.cat(rec_state), "policy": torch.cat(rec_policy), "value": value, "game": game, "ply": plyv,
-            "flags": final_flags, "plies": final_plies, "sims": sims_run, "reused": reused, **extra}
+            "flags": final_flags, "plies": final_plies, "sims": sims_run, "reused": reused, "full_searches": full_searches,
+            "fast_searches": sum_searches - full_searches, **extra}
 
 
 def resign_threshold_for(rec, max_false_positive=0.05):
@@ -193,14 +244,15 @@ def resign_threshold_for(rec, max_false_positive=0.05):
 
 def play_batch(model, num_games, device=None, sims=None, temperature=SP_TEMPERATURE, seed=None, max_plies=None, tree_reuse=False,
                dirichlet_alpha=None, noise_fraction=0.25, gumbel_considered=None, gumbel_scale=1.0, resign_threshold=None,
-               resign_calibration=0.1, forced_k=None):
+               resign_calibration=0.1, forced_k=None, fast_sims=None, full_search_prob=0.25):
     """play_batch_device + conversion to the reference's history: a list of [[player, enemy, walls], policy (209 floats), value]
     (self_play.py:51-54, 63-66), games in order, plies in order within a game.  Returns (history, dict with per-game results:
-    flags, plies, and with resign_threshold also resign_min and calibration)."""
+    flags, plies, and with resign_threshold also resign_min and calibration).  With fast_sims the history holds the positions of full
+    searches only."""
     rec = play_batch_device(model, num_games, device, sims, temperature, seed, max_plies, tree_reuse=tree_reuse,
                             dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction, gumbel_considered=gumbel_considered,
                             gumbel_scale=gumbel_scale, resign_threshold=resign_threshold, resign_calibration=resign_calibration,
-                            forced_k=forced_k)
+                            forced_k=forced_k, fast_sims=fast_sims, full_search_prob=full_search_prob)
     rows, _ = gl.unpack_rows(rec["states"])
     rows = rows.cpu().numpy()
     pols = rec["policy"].cpu().numpy()
@@ -225,13 +277,13 @@ def play(model, device=None):
 
 def self_play(game_count=None, model_path=None, data_dir='./data/', rank=0, world_size=1, sims=None, seed=None, tree_reuse=False,
               dirichlet_alpha=None, noise_fraction=0.25, gumbel_considered=None, gumbel_scale=1.0, resign_threshold=None,
-              resign_calibration=0.1, forced_k=None):
+              resign_calibration=0.1, forced_k=None, fast_sims=None, full_search_prob=0.25):
     """Perform self-play games and save the training data (self_play.py:71-98).  With
     world_size > 1 each rank plays its share of the games on its own GPU and rank 0 writes the file.
     tree_reuse=True keeps each game's search tree between moves; dirichlet_alpha adds AlphaZero root noise to every search;
     gumbel_considered searches with the Gumbel AlphaZero root and records its improved policy; resign_threshold lets games resign,
-    resign_calibration of them excepted; forced_k forces root playouts and prunes them from the policy targets (see
-    play_batch_device)."""
+    resign_calibration of them excepted; forced_k forces root playouts and prunes them from the policy targets; fast_sims gives a
+    fraction 1 - full_search_prob of the moves a cheap search and records only the others (see play_batch_device)."""
     game_count = SP_GAME_COUNT if game_count is None else game_count
     model = GNNNetwork()
     model.prep_for_inference(model_path=model_path or (PV_NETWORK_PATH + 'best.pth'))
@@ -239,7 +291,8 @@ def self_play(game_count=None, model_path=None, data_dir='./data/', rank=0, worl
     history, _ = play_batch(model, mine, sims=sims, seed=None if seed is None else seed + rank, tree_reuse=tree_reuse,
                             dirichlet_alpha=dirichlet_alpha, noise_fraction=noise_fraction, gumbel_considered=gumbel_considered,
                             gumbel_scale=gumbel_scale, resign_threshold=resign_threshold,
-                            resign_calibration=resign_calibration, forced_k=forced_k) if mine else ([], None)
+                            resign_calibration=resign_calibration, forced_k=forced_k, fast_sims=fast_sims,
+                            full_search_prob=full_search_prob) if mine else ([], None)
     if world_size > 1:
         import torch.distributed as dist
         gathered = [None] * world_size if rank == 0 else None

@@ -53,7 +53,7 @@ typedef struct AqState {
     uint64_t reserved; /* reserved, 0 */
 } AqState;
 
-#define AQ_VERSION 210 /* bumped with every change of a signature below; the ctypes loader refuses a library of another version */
+#define AQ_VERSION 211 /* bumped with every change of a signature below; the ctypes loader refuses a library of another version */
 int aq_version(void);
 const char *aq_last_error_string(void);
 /* Number of kernels this library has launched in the process so far (monotonic; kernels replayed through a CUDA graph the caller
@@ -348,6 +348,24 @@ int aq_mcts_root_counts_pruned(void *ws, int64_t G, int64_t max_nodes, float c_p
 int aq_mcts_root_noise(void *ws, int64_t G, int64_t max_nodes, const int64_t *game_id, uint64_t seed, int32_t ply,
                        float alpha, float fraction, float *root_priors, void *stream);
 
+/* Prefix entry points (playout cap randomization searches a prefix of the batch): each runs the kernel of its plain entry point over
+ * games [0, rows) of a workspace laid out for G games, 1 <= rows <= G; games [rows, G) are neither read nor written.  Every other
+ * argument, and every per-game array (leaf_states, leaf_kind, priors, values, mask, pawn, game_id, root_priors), is that of the
+ * plain entry point, indexed by the game's row.  AQ_ERR_ARG as the plain entry point, and for rows outside [1, G]. */
+int aq_mcts_select_rows(void *ws, int64_t G, int64_t rows, int64_t max_nodes, float c_puct, AqState *leaf_states, int32_t *leaf_kind,
+                        void *stream);
+int aq_mcts_select_forced_rows(void *ws, int64_t G, int64_t rows, int64_t max_nodes, float c_puct, float forced_k, AqState *leaf_states,
+                               int32_t *leaf_kind, void *stream);
+int aq_mcts_expand_backup_rows(void *ws, int64_t G, int64_t rows, int64_t max_nodes, const float *priors, const float *values,
+                               const uint32_t *mask, const uint8_t *pawn, void *stream);
+int aq_mcts_expand_select_rows(void *ws, int64_t G, int64_t rows, int64_t max_nodes, const float *priors, const float *values,
+                               const uint32_t *mask, const uint8_t *pawn, float c_puct, AqState *leaf_states, int32_t *leaf_kind, void *stream);
+int aq_mcts_expand_select_forced_rows(void *ws, int64_t G, int64_t rows, int64_t max_nodes, const float *priors, const float *values,
+                                      const uint32_t *mask, const uint8_t *pawn, float c_puct, float forced_k, AqState *leaf_states,
+                                      int32_t *leaf_kind, void *stream);
+int aq_mcts_root_noise_rows(void *ws, int64_t G, int64_t rows, int64_t max_nodes, const int64_t *game_id, uint64_t seed, int32_t ply,
+                            float alpha, float fraction, float *root_priors, void *stream);
+
 /* One ply of G lock-step self-play games after their searches (self_play.py:47-60), two launches:
  *   scores = counts ** (1 / temperature) / sum over the root's children (pv_mcts.py:88-95; temperature 0 = one-hot on
  *            the first maximum, np.argmax); policy[g, action] = score, 0 for the other of the 209 actions (self_play.py:51-54),
@@ -394,6 +412,17 @@ int aq_selfplay_advance_resign(const AqState *states, const int32_t *counts, con
                                const double *best_q, double v_resign, double calibration, double *resign_min /*[num_games,2]*/,
                                uint8_t *is_calibration /*[num_games]*/, AqState *next_states, int64_t *next_game_id, uint8_t *final_flags, int64_t *final_plies,
                                int32_t *alive_count, void *workspace, void *stream);
+
+/* Playout cap randomization (KataGo: Wu 2019, section 3.1; the reference has none): which moves get a full search.  One launch, one
+ * CTA.  Rows [0, n) with n = *count (device; NULL: G; clamped to [0, G]) are reordered stably: the full rows first, then the fast
+ * rows, each kind in input order; out_states / out_game_id [n] take the reordered rows, out_row [n] int64 the input row of each
+ * output row, full_count[0] the number of full rows.  Row i is full iff u < full_prob with
+ *   u = (mix64(mix64((seed ^ kPcrDomain) + 0x9E3779B97F4A7C15 * (game_id[i] + 1)) + 0xD1B54A32D192ED03 * (ply + 1)) >> 11) * 2^-53,
+ *   kPcrDomain = 0x082EFA98EC4E6C89 (csrc/mcts.cu)
+ * a function of (seed, game id, ply) alone, independent of the move, noise, Gumbel and calibration draws; full_prob = 1 makes every
+ * row full.  AQ_ERR_ARG for G outside [1, 2^31), full_prob outside [0, 1] or NaN, or a NULL pointer other than count. */
+int aq_selfplay_partition(const AqState *states, const int64_t *game_id, int64_t G, const int32_t *count, uint64_t seed, int32_t ply,
+                          double full_prob, AqState *out_states, int64_t *out_game_id, int64_t *out_row, int32_t *full_count, void *stream);
 
 /* agents.heuristic_eval (agents.py:22-54) for B states: shortest pawn-path lengths to the goal row for the mover
  * and for the enemy (shortest_path_bfs, agents.py:27-41, with the jump rules of legal_actions_pos; -1 = no path).
